@@ -2,6 +2,7 @@
 """bench.py -- throughput of the Sygnals segment->features hot path on B200 (see DESIGN.md "Measurement").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg4|cfg1|cfg2|cfg3|cfg5] [--impl native|reference]
+                    [--dump-outputs DIR]
 
 Default workload = BASELINE.json configs[3] ("cfg4", the config the metric "audio-sec/sec (MFCC+spectral feats)" names):
 ONE 10 h synthetic 44.1 kHz recording, fixed-length 2 s segments with 50 % overlap (36 000 segments), per segment
@@ -21,6 +22,11 @@ collective: round 1's measure) is reported under `weak`.
 float64, incl. its per-frame Python loops; librosa itself is not installable offline) on the host cores.
 
 Other workloads (secondary lines, same contract): cfg3 speech-commands MFCC, cfg2 STFT magnitude sweep, cfg5 Welch PSD.
+
+`--dump-outputs DIR` writes what the timed path computed in its last timed step as DIR/<name>.npy (see `dump_outputs`).  The
+inputs are synthesised from fixed seeds, so two builds run with the same arguments can be compared output for output.  cfg4 and
+cfg1/cfg3 write the output gathered from all ranks; cfg2 and cfg5 have no collective, so under --gpus N > 1 they write rank 0's
+block (its clips / channels, whose inputs are seeded per rank).
 """
 from __future__ import annotations
 
@@ -77,6 +83,30 @@ def emit_json(line: dict) -> None:
         sys.stdout.flush()
     else:
         os.write(_REAL_STDOUT, data)
+
+
+DUMP_BYTES = 60 << 20                                                  # under 64 MB with the .npy headers
+DUMP_SEED = 20240607
+
+
+def dump_outputs(out_dir, arrays: dict, budget: int = DUMP_BYTES) -> None:
+    """Writes each tensor of ``arrays`` (float32 / float64, leading axis = units: segments, clips, channel-seconds) to
+    ``out_dir/<name>.npy``.  When they hold more than ``budget`` bytes in all, each keeps the same fraction of its units, a fixed
+    seeded sample in ascending order, so that the files of two runs with the same arguments hold the same units."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(t.numel() * t.element_size() for t in arrays.values())
+    for name, t in arrays.items():
+        n = t.shape[0]
+        if total > budget:
+            k = max(1, n * budget // total)
+            idx = np.sort(np.random.default_rng(DUMP_SEED).choice(n, k, replace=False))
+            t = t[torch.from_numpy(idx).to(t.device)]
+        a = t.detach().cpu().numpy()
+        if a.dtype not in (np.float32, np.float64):
+            raise TypeError(f"--dump-outputs: {name} is {a.dtype}, expected float32 or float64")
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def env_int(name, default):
@@ -323,6 +353,12 @@ class Ctx:
         self.eng.profile_enable(False)
         return self.max_over_ranks(ms), ms, clk, prof
 
+    def dump(self, arrays: dict) -> None:
+        """--dump-outputs: rank 0 writes the outputs of the last timed step, before any later measurement reuses the device.  The
+        callers pass the gathered output where the step gathers one (cfg4, cfg1/cfg3) and rank 0's own block otherwise (cfg2, cfg5)."""
+        if self.args.dump_outputs and self.rank == 0:
+            dump_outputs(self.args.dump_outputs, arrays)
+
     def time_wall(self, step, steps, warm=1):
         for _ in range(warm):
             step()
@@ -415,9 +451,10 @@ def run_segments(c: Ctx):
         state["full"] = sdist.gather_features(local, plan)             # world 1: returns `local`
 
     ms_max, ms, clk, prof = c.time_device(step, args.steps)
+    full = state["full"]
+    c.dump({"features": full})                                          # float64 [segments, 24]
     audio_total = plan.n_units * unit_seconds(w)                        # unique audio seconds of the whole recording
     value = audio_total * args.steps / (ms_max * 1e-3)
-    full = state["full"]
     checksum = float(torch.nan_to_num(full).sum().item())
     gather_ms = None
     if c.world > 1:                                                     # the collective alone, for the record (it is inside ms_per_step)
@@ -563,6 +600,7 @@ def run_clips(c: Ctx):
         state["full"] = gather_block(c, out, counts)
 
     ms_max, ms, clk, prof = c.time_device(step, args.steps)
+    c.dump({"features": state["full"]})                                 # float32 [clips, rows, frames]
     value = n_all * clip_s * args.steps / (ms_max * 1e-3)
     e2e = None
     if not args.no_e2e and args.workload == "cfg1":
@@ -658,6 +696,7 @@ def run_stft(c: Ctx):
                       "audio_s_per_s": c.world * n * args.steps / (c.max_over_ranks(k_ms) * 1e-3)})
         tot_ms += c.max_over_ranks(k_ms)
         launches += k_n
+    c.dump({f"stft_magnitude_{nf}": outs[nf] for nf in sizes})          # float32 [clips, n_fft / 2 + 1, frames] per size
     value = n_all * len(sizes) * args.steps / (tot_ms * 1e-3)
     e2e = None
     if not args.no_e2e:
@@ -718,6 +757,7 @@ def run_welch(c: Ctx):
         eng.psd_welch_dev(y.data_ptr(), units, float(sr), 0, 1024, 512, 1024, True, 0, psd.data_ptr(), st.data_ptr(), stream)
 
     ms_max, ms, clk, prof = c.time_device(step, args.steps)
+    c.dump({"psd": psd, "stats": st})                                   # float32 [channel-seconds, 513] and [channel-seconds, 3]
     value = n_all * args.steps / (ms_max * 1e-3)
     e2e = None
     if not args.no_e2e:
@@ -768,7 +808,14 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-weak", action="store_true", help="cfg4: skip the weak-scaling side measurement")
     ap.add_argument("--cpu-units", type=int, default=0, help="units per step of the CPU reference arm")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="native arm: write the outputs of the last timed step as DIR/<name>.npy (under 64 MB in all: a seeded sample of a larger "
+                         "output); cfg4/cfg1/cfg3 write the output gathered from all ranks, cfg2/cfg5 rank 0's block"),
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "native":
+        ap.error("--dump-outputs writes the native arm's outputs")
     guard_stdout()
     if args.impl == "reference":
         return run_reference(args)

@@ -87,6 +87,75 @@ def test_secondary_workloads_on_the_gpu(wl, extra):
         assert [s["n_fft"] for s in d["roofline"]["sweep"]] == [512, 2048]
 
 
+def test_bad_step_counts_and_reference_dump_are_refused():
+    for args in (["--steps", "0"], ["--warmup", "-1"], ["--impl", "reference", "--dump-outputs", "out"]):
+        r = run_bench(*args)
+        assert r.returncode == 2 and r.stdout.strip() == "" and "error:" in r.stderr, args
+
+
+def test_dump_outputs_keeps_a_seeded_sample_under_the_budget(tmp_path):
+    import importlib.util
+    import numpy as np
+    import torch
+    spec = importlib.util.spec_from_file_location("bench_module", BENCH)
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    a = torch.arange(1000 * 6, dtype=torch.float64).reshape(1000, 6)
+    b = torch.arange(1000 * 10, dtype=torch.float32).reshape(1000, 10)
+    bench.dump_outputs(str(tmp_path / "all"), {"a": a, "b": b})
+    assert np.array_equal(np.load(tmp_path / "all" / "a.npy"), a.numpy()) and np.load(tmp_path / "all" / "b.npy").dtype == np.float32
+    budget = (a.numel() * 8 + b.numel() * 4) // 4
+    for run in ("s1", "s2"):
+        bench.dump_outputs(str(tmp_path / run), {"a": a, "b": b}, budget=budget)
+    sa, sb = np.load(tmp_path / "s1" / "a.npy"), np.load(tmp_path / "s1" / "b.npy")
+    assert sa.nbytes + sb.nbytes <= budget and sa.shape == (250, 6) and sb.shape == (250, 10)
+    rows = sa[:, 0] / 6
+    assert np.all(np.diff(rows) > 0) and np.array_equal(sb[:, 0] / 10, rows)       # same units in both, ascending
+    assert np.array_equal(np.load(tmp_path / "s2" / "a.npy"), sa)
+    with pytest.raises(TypeError):
+        bench.dump_outputs(str(tmp_path / "i"), {"i": torch.zeros(3, dtype=torch.int32)})
+
+
+@pytest.mark.gpu
+def test_dump_outputs_of_two_runs_agree(tmp_path):
+    """--dump-outputs writes the [segments, 24] float64 vectors of the last timed step; the same arguments give the same inputs, so
+    runs of one build write the same values, whatever the number of steps.  --steps sets the steps actually timed: twice the steps,
+    twice the kernel launches in the timed window."""
+    import numpy as np
+    outs, launches = [], []
+    for run, steps in (("a", 3), ("b", 6)):
+        r = run_bench("--hours", "0.05", "--steps", str(steps), "--warmup", "1", "--no-cpu", "--no-e2e", "--no-weak",
+                      "--dump-outputs", str(tmp_path / run))
+        assert r.returncode == 0, r.stderr[-2000:]
+        d = json.loads(r.stdout.strip().splitlines()[-1])
+        assert d["steps"] == steps
+        launches.append(d["gpu_launches"])
+        assert sorted(os.listdir(tmp_path / run)) == ["features.npy"]
+        outs.append(np.load(tmp_path / run / "features.npy"))
+        assert outs[-1].dtype == np.float64 and outs[-1].shape == (d["config"]["segments"], 24)
+        assert abs(float(np.nansum(outs[-1])) - d["checksum"]) <= 1e-9 * abs(d["checksum"])
+    np.testing.assert_array_equal(outs[0], outs[1])
+    assert launches[0] > 0 and launches[1] == 2 * launches[0], launches
+
+
+@pytest.mark.gpu
+def test_dump_outputs_sample_a_large_output_on_the_device(tmp_path):
+    """cfg3 with 16 000 clips computes [16000, 13, 101] float32 (84 MB): the dump keeps the same seeded sample of clips in every run,
+    under 64 MB."""
+    import numpy as np
+    outs = []
+    for run in ("a", "b"):
+        r = run_bench("--workload", "cfg3", "--units", "16000", "--steps", "2", "--warmup", "1", "--no-cpu", "--no-e2e",
+                      "--dump-outputs", str(tmp_path / run))
+        assert r.returncode == 0, r.stderr[-2000:]
+        f = tmp_path / run / "features.npy"
+        assert sorted(os.listdir(tmp_path / run)) == ["features.npy"] and os.path.getsize(f) < 64_000_000
+        outs.append(np.load(f))
+        assert outs[-1].dtype == np.float32 and 10000 < outs[-1].shape[0] < 16000 and outs[-1].shape[1:] == (13, 101)
+        assert np.isfinite(outs[-1]).all()
+    np.testing.assert_array_equal(outs[0], outs[1])
+
+
 @pytest.mark.parametrize("wl", ["cfg3", "cfg2", "cfg5"])
 def test_reference_arm_secondary_workloads(wl):
     r = run_bench("--impl", "reference", "--workload", wl, "--steps", "1", "--warmup", "0", "--cpu-units", "8")

@@ -35,6 +35,8 @@ def test_cfg2_stft_sweep():
             assert D.dtype == np.complex128
             scale = np.abs(G).max()
             assert np.abs(D - G).max() <= 2e-7 * scale  # golden stored as complex64
+    g = cases.load("cfg2_stft_variants.npz")
+    _close(cases.checksum(clips), g["in_checksum"], 1e-12, 0)
     D = O.compute_stft(clips[0].astype(np.float64), n_fft=1024, hop_length=200, win_length=800, pad_mode="reflect")
     assert np.abs(D - g["D_reflect_1024_800_200"]).max() <= 2e-7 * np.abs(D).max()
     D = O.compute_stft(clips[0].astype(np.float64), n_fft=512, hop_length=128, center=False)

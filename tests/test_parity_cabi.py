@@ -142,7 +142,7 @@ def test_stft_real_outputs_ragged_batches_vs_oracle(eng, n_fft, hop, n, L):
 
 def test_golden_cfg2_reflect_and_nocenter(eng):
     y, sr = cases.cfg2_input()
-    g = cases.load("cfg2_stft_sweep.npz")
+    g = cases.load("cfg2_stft_variants.npz")
     u = eng.units_clips(1, y.shape[1])
     D = eng.stft_host(y[0], u, 1024, 200, 800, pad_mode=_ffi.PAD_IDS["reflect"])
     ref = g["D_reflect_1024_800_200"]
