@@ -176,7 +176,8 @@ __global__ void __launch_bounds__(NT, MINB) frame_warp_kernel(const syg::FrameAr
     float2* const zs = reinterpret_cast<float2*>(wbase + f * RSS);
     float* const pf = wbase + f * RSS;
 
-    // pad / slack words of the spectra are read (with zero weight) by the mel sweep: they must never hold NaN patterns
+    // pad / slack words of the spectra are read (with zero weight) by the mel sweep: they must never hold NaN patterns.  They do
+    // hold FFT data of earlier stages (any sign), which is why the power != 2 sweep raises only weighted taps.
     for (int i = lane; i < WF; i += 32) wbase[i] = 0.0f;
     __syncwarp();
 
@@ -827,13 +828,16 @@ __global__ void __launch_bounds__(NT, MINB) frame_warp_kernel(const syg::FrameAr
                     }
                     acc = (m01.x + m01.y) + (m23.x + m23.y);
                 } else {
+                    // Zero-weight taps also cover the pad words of the spectrum, which still hold FFT data from the transform
+                    // (negative values too): powf of those is NaN, and 0 * NaN would poison the filter.  Only weighted taps
+                    // (always real bins, |X|^2 >= 0) are raised to the power.
                     for (int i = 0; i < d.z; ++i) {
                         const float4 w = TBL ? wv[GS * i] : __ldg(wv + GS * i);
                         const float4 q = pp4[i];
-                        acc = __fmaf_rn(w.x, powf(q.x, a.mel_half_power), acc);
-                        acc = __fmaf_rn(w.y, powf(q.y, a.mel_half_power), acc);
-                        acc = __fmaf_rn(w.z, powf(q.z, a.mel_half_power), acc);
-                        acc = __fmaf_rn(w.w, powf(q.w, a.mel_half_power), acc);
+                        acc = __fmaf_rn(w.x, w.x != 0.0f ? powf(q.x, a.mel_half_power) : 0.0f, acc);
+                        acc = __fmaf_rn(w.y, w.y != 0.0f ? powf(q.y, a.mel_half_power) : 0.0f, acc);
+                        acc = __fmaf_rn(w.z, w.z != 0.0f ? powf(q.z, a.mel_half_power) : 0.0f, acc);
+                        acc = __fmaf_rn(w.w, w.w != 0.0f ? powf(q.w, a.mel_half_power) : 0.0f, acc);
                     }
                 }
                 if (base + sl < a.n_mels && fvalid) {

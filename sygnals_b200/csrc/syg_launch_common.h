@@ -41,6 +41,14 @@ inline int prepare_kernel(K kfn, int threads, size_t smem, KernelCache& kc, int*
     if (dev < 0 || dev >= kMaxDevices) { err = "device index out of range"; return -3; }
     std::lock_guard<std::mutex> lk(kc.mu);
     if (smem > kc.opted[dev] && smem > 48 * 1024) {
+        // checked here rather than left to cudaFuncSetAttribute: its failure would also linger as the thread's last error and
+        // fail the caller's next launch check
+        int optin = 0;
+        LCK(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+        if (smem > (size_t)optin) {
+            err = "the plan needs " + std::to_string(smem) + " bytes of shared memory per block, the device allows " + std::to_string(optin);
+            return -5;                                               // SYG_E_UNSUPPORTED
+        }
         LCK(cudaFuncSetAttribute(kfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         kc.opted[dev] = smem;
     }

@@ -94,7 +94,17 @@ static int frame_warp_dispatch(int n_fft, const syg::FrameArgs& a, int sm_count,
                 if (!nospec && spec_matches<Spec44k>(a)) return frame_warp_spec44k(a, sm_count, st, err);
                 if (!nospec && spec_matches<Spec22k>(a)) return frame_warp_spec22k(a, sm_count, st, err);
             }
-            if (STAGE == 0) return frame_warp_t<FftTile<10, 32>, EXTRA, SYG_NT2048, 1, STAGE>(a, sm_count, st, err);
+            if (STAGE == 0) {
+                // 20 warps leave ~40 KB of shared memory for the plan tables: enough for the interval-form mel and for the tap
+                // tables of the default banks, not for the long taps of a few wide filters (n_mels 40 or fewer without the
+                // interval form, e.g. mel power != 2).  Those plans run 8 warps per CTA.
+                const size_t tbl = WarpTile<FftTile<10, 32>, SYG_NT2048>::table_bytes(a.n_mels, (a.mask & syg::FB_MFCC) ? a.mel_pw_f4 : 0);
+                int dev = 0, optin = 0;
+                LCK(cudaGetDevice(&dev));
+                LCK(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+                if (WarpTile<FftTile<10, 32>, SYG_NT2048>::bytes + tbl <= (size_t)optin)
+                    return frame_warp_t<FftTile<10, 32>, EXTRA, SYG_NT2048, 1, STAGE>(a, sm_count, st, err);
+            }
             return frame_warp_t<FftTile<10, 32>, EXTRA, NT, MINB, STAGE>(a, sm_count, st, err);
     }
     err = "n_fft=" + std::to_string(n_fft) + " has no warp tile";
