@@ -172,6 +172,35 @@ int syg_segment_vectors_host_f32(syg_ctx* ctx, const float* y_host, const syg_un
 int syg_segment_vectors_host_pcm(syg_ctx* ctx, const void* raw_host, int32_t sample_format, int32_t channels,
                                  const syg_units* units, const syg_feature_params* p, const int32_t* agg, double* out_host);
 
+/* Ragged batches: units of their own lengths in one call (a folder of clips, the variable-length segments of one recording).
+ * Unit u is exactly y[starts[u], starts[u] + lengths[u]): no padding to a common length; units may overlap or leave gaps.  It has
+ * T_u = syg_frame_count(lengths[u], ...) frames (0 allowed); F_0 = 0, F_{u+1} = F_u + T_u, F = F_{n_units}.
+ * Features: float32 [n_rows][F], row r of frame t of unit u at out[r * F + F_u + t] -- the reference's features_dict over a
+ * concatenated frame axis with (F_u, F_{u+1}) as segment indices (formatters.py:51-163).  Columns F_u .. F_{u+1}-1 equal, bit for
+ * bit, syg_features_host_f32 on that unit alone (its own power_to_db reference level included).
+ * Segment vectors: float64 [n_units][n_rows], agg[r] in SYG_AGG_* over the unit's T_u frames (T_u = 0: a NaN row).
+ * The tables are HOST memory for the device and the host forms alike; the call stages them before it returns.
+ * Errors: SYG_E_BADARG for a negative start or length, a unit outside the sample buffer or NULL tables (n_units > 0);
+ * SYG_E_UNSUPPORTED for lengths[u] or T_u above 2^31-1; plan errors as syg_features_*.  n_units = 0 or F = 0: nothing to do. */
+typedef struct {
+    int64_t n_units;
+    int64_t total_len;          /* samples in y */
+    const int64_t* starts;      /* [n_units] host memory */
+    const int64_t* lengths;     /* [n_units] host memory */
+} syg_ragged_units;
+
+/* F (>= 0) or a negative SYG_E_*; frame_off (optional, [n_units + 1]) receives F_0 .. F_{n_units} */
+int64_t syg_ragged_frame_offsets(const syg_ragged_units* units, int32_t frame_length, int32_t hop_length, int32_t center,
+                                 int64_t* frame_off);
+int syg_features_ragged_f32(syg_ctx* ctx, const float* y_dev, const syg_ragged_units* units, const syg_feature_params* p,
+                            float* out_dev, void* stream);
+int syg_features_ragged_host_f32(syg_ctx* ctx, const float* y_host, const syg_ragged_units* units, const syg_feature_params* p,
+                                 float* out_host);
+int syg_segment_vectors_ragged_f32(syg_ctx* ctx, const float* y_dev, const syg_ragged_units* units, const syg_feature_params* p,
+                                   const int32_t* agg, double* out_dev, void* stream);
+int syg_segment_vectors_ragged_host_f32(syg_ctx* ctx, const float* y_host, const syg_ragged_units* units,
+                                        const syg_feature_params* p, const int32_t* agg, double* out_host);
+
 /* compute_stft(): out [n_units][1 + n_fft/2][T]; complex64 (interleaved) / float32 magnitude / float32 power */
 int syg_stft_f32(syg_ctx* ctx, const float* y_dev, const syg_units* units, int32_t n_fft, int32_t hop_length,
                  int32_t win_length, int32_t window, int32_t center, int32_t pad_mode, int32_t out_kind,
@@ -223,6 +252,9 @@ int syg_spectral_contrast_from_mag_f32(syg_ctx* ctx, const float* S_dev, int32_t
 int syg_debug_last_stft_path(void);
 /* 1 when the last feature launch kept its (short) units on chip: mel tile + dB + DCT inside the frame kernel, no finalize launch */
 int syg_debug_last_features_resident(void);
+/* frames the feature kernels processed in the last syg_features_* / syg_segment_vectors_* call, all chunks (n_units * T for the
+ * uniform forms, F for the ragged ones) */
+int64_t syg_debug_last_feature_frames(void);
 /* mel projection of the last feature launch with MFCCs: 1 interval form (running sums per mel interval + picks), 0 padded tap sweeps
  * (the form is refused for banks its planner cannot represent; tests pin it for the BASELINE banks so that a refusal is not silent) */
 int syg_debug_last_mel_form(void);

@@ -55,6 +55,11 @@ class SygUnits(C.Structure):
                 ("unit_starts", C.c_void_p), ("unit_valid", C.c_void_p)]
 
 
+class SygRaggedUnits(C.Structure):
+    """Units of their own lengths: unit u is y[starts[u], starts[u] + lengths[u]) (host int64 tables)."""
+    _fields_ = [("n_units", C.c_int64), ("total_len", C.c_int64), ("starts", C.c_void_p), ("lengths", C.c_void_p)]
+
+
 class SygFeatureParams(C.Structure):
     _fields_ = [("sr", C.c_int32), ("frame_length", C.c_int32), ("hop_length", C.c_int32), ("center", C.c_int32),
                 ("window", C.c_int32), ("n_features", C.c_int32), ("features", C.c_int32 * MAX_FEATURES),
@@ -81,7 +86,7 @@ class Library:
         self.dll = C.CDLL(path)
         d = self.dll
         vp, i32, i64, f32, f64, sz = C.c_void_p, C.c_int32, C.c_int64, C.c_float, C.c_double, C.c_size_t
-        PU, PP = C.POINTER(SygUnits), C.POINTER(SygFeatureParams)
+        PU, PP, PR = C.POINTER(SygUnits), C.POINTER(SygFeatureParams), C.POINTER(SygRaggedUnits)
         protos = {
             "syg_version": (C.c_char_p, []),
             "syg_last_error": (C.c_char_p, []),
@@ -103,6 +108,11 @@ class Library:
             "syg_segment_vectors_f32": (C.c_int, [vp, vp, PU, PP, vp, vp, vp]),
             "syg_segment_vectors_host_f32": (C.c_int, [vp, vp, PU, PP, vp, vp]),
             "syg_segment_vectors_host_pcm": (C.c_int, [vp, vp, i32, i32, PU, PP, vp, vp]),
+            "syg_ragged_frame_offsets": (i64, [PR, i32, i32, i32, vp]),
+            "syg_features_ragged_f32": (C.c_int, [vp, vp, PR, PP, vp, vp]),
+            "syg_features_ragged_host_f32": (C.c_int, [vp, vp, PR, PP, vp]),
+            "syg_segment_vectors_ragged_f32": (C.c_int, [vp, vp, PR, PP, vp, vp, vp]),
+            "syg_segment_vectors_ragged_host_f32": (C.c_int, [vp, vp, PR, PP, vp, vp]),
             "syg_stft_f32": (C.c_int, [vp, vp, PU, i32, i32, i32, i32, i32, i32, i32, vp, vp]),
             "syg_stft_host_f32": (C.c_int, [vp, vp, PU, i32, i32, i32, i32, i32, i32, i32, vp]),
             "syg_psd_welch_f32": (C.c_int, [vp, vp, PU, f64, i32, i32, i32, i32, i32, i32, vp, vp, vp]),
@@ -114,6 +124,7 @@ class Library:
             "syg_spectral_contrast_from_mag_f32": (C.c_int, [vp, vp, i32, i64, f64, i32, f64, f64, vp, vp]),
             "syg_debug_last_stft_path": (C.c_int, []),
             "syg_debug_last_features_resident": (C.c_int, []),
+            "syg_debug_last_feature_frames": (i64, []),
             "syg_debug_last_mel_form": (C.c_int, []),
             "syg_debug_set_resident_min_groups": (None, [C.c_int]),
             "syg_debug_window": (C.c_int, [i32, i32, i32, vp]),
@@ -168,6 +179,18 @@ class Library:
                                            int(bool(pad)), mn, starts.ctypes.data, valid.ctypes.data, int(n))
             assert m == n
         return int(seg_len.value), int(seg_hop.value), starts, valid
+
+    def ragged_frame_offsets(self, units: SygRaggedUnits, frame_length: int, hop_length: int, center: bool = True) -> np.ndarray:
+        """int64 ``[n_units + 1]``: F_0 = 0, F_{u+1} = F_u + T_u (T_u = frame_count(lengths[u], ...))."""
+        out = np.zeros(int(units.n_units) + 1, dtype=np.int64)
+        n = self.dll.syg_ragged_frame_offsets(C.byref(units), int(frame_length), int(hop_length), int(bool(center)), out.ctypes.data)
+        if n < 0:
+            self.check(int(n))
+        return out
+
+    def last_feature_frames(self) -> int:
+        """Frames the feature kernels processed in the last features / segment-vectors call of this process."""
+        return int(self.dll.syg_debug_last_feature_frames())
 
     def debug_window(self, window: int, win_length: int, n_fft: int) -> np.ndarray:
         out = np.zeros(n_fft, dtype=np.float32)
@@ -314,6 +337,19 @@ class Engine:
         u.unit_starts, u.unit_valid = starts_ptr, valid_ptr
         return u
 
+    @staticmethod
+    def ragged_units(starts, lengths, total_len: int) -> SygRaggedUnits:
+        """Ragged unit tables (host int64 copies; the returned structure keeps them alive)."""
+        st = np.ascontiguousarray(starts, dtype=np.int64).reshape(-1)
+        ln = np.ascontiguousarray(lengths, dtype=np.int64).reshape(-1)
+        if st.shape != ln.shape:
+            raise ValueError("starts and lengths must have the same length")
+        u = SygRaggedUnits()
+        u.n_units, u.total_len = int(st.shape[0]), int(total_len)
+        u.starts, u.lengths = (st.ctypes.data, ln.ctypes.data) if st.size else (None, None)
+        u._keep = (st, ln)
+        return u
+
     def rows(self, p: SygFeatureParams) -> int:
         n = C.c_int32(0)
         self.lib.check(self.lib.dll.syg_features_rows(C.byref(p), C.byref(n)))
@@ -422,9 +458,43 @@ class Engine:
             int(bool(detrend)), int(scaling), psd.ctypes.data, st.ctypes.data if stats else None))
         return (psd, st) if stats else psd
 
+    def features_ragged_host(self, y: np.ndarray, units: SygRaggedUnits, p: SygFeatureParams, out: Optional[np.ndarray] = None) -> np.ndarray:
+        """float32 ``[n_rows, F]`` for ragged units of the 1-D float32 host buffer ``y`` (row r of frame t of unit u at column F_u + t)."""
+        y = _f32c(y)
+        F = int(self.lib.ragged_frame_offsets(units, p.frame_length, p.hop_length, p.center)[-1])
+        if out is None:
+            out = np.empty((self.rows(p), F), dtype=np.float32)
+        self.lib.check(self.lib.dll.syg_features_ragged_host_f32(self._h, y.ctypes.data, C.byref(units), C.byref(p), out.ctypes.data))
+        return out
+
+    def segment_vectors_ragged_host(self, y: np.ndarray, units: SygRaggedUnits, p: SygFeatureParams, agg_ids: Sequence[int],
+                                    out: Optional[np.ndarray] = None) -> np.ndarray:
+        """float64 ``[n_units, n_rows]``: each ragged unit's frames aggregated per row (a unit without frames gives a NaN row)."""
+        rows = self.rows(p)
+        if len(agg_ids) != rows:
+            raise ValueError("one aggregation id per feature row")
+        y = _f32c(y)
+        if out is None:
+            out = np.empty((int(units.n_units), rows), dtype=np.float64)
+        agg = (C.c_int32 * max(1, rows))(*[int(a) for a in agg_ids])
+        self.lib.check(self.lib.dll.syg_segment_vectors_ragged_host_f32(self._h, y.ctypes.data, C.byref(units), C.byref(p),
+                                                                        C.addressof(agg), out.ctypes.data))
+        return out
+
     # ------------------------------------------------------------------ device-pointer entry points (async)
     def features_dev(self, y_ptr: int, units: SygUnits, p: SygFeatureParams, out_ptr: int, stream: int = 0) -> None:
         self.lib.check(self.lib.dll.syg_features_f32(self._h, y_ptr, C.byref(units), C.byref(p), out_ptr, stream or None))
+
+    def features_ragged_dev(self, y_ptr: int, units: SygRaggedUnits, p: SygFeatureParams, out_ptr: int, stream: int = 0) -> None:
+        """Device form of ``features_ragged_host``: float32 ``[n_rows, F]`` in HBM, asynchronous on ``stream``."""
+        self.lib.check(self.lib.dll.syg_features_ragged_f32(self._h, y_ptr, C.byref(units), C.byref(p), out_ptr, stream or None))
+
+    def segment_vectors_ragged_dev(self, y_ptr: int, units: SygRaggedUnits, p: SygFeatureParams, agg_ids: Sequence[int], out_ptr: int,
+                                   stream: int = 0) -> None:
+        """Device form of ``segment_vectors_ragged_host``: float64 ``[n_units, n_rows]`` in HBM, asynchronous on ``stream``."""
+        agg = (C.c_int32 * max(1, len(agg_ids)))(*[int(a) for a in agg_ids])
+        self.lib.check(self.lib.dll.syg_segment_vectors_ragged_f32(self._h, y_ptr, C.byref(units), C.byref(p), C.addressof(agg), out_ptr,
+                                                                   stream or None))
 
     def stft_dev(self, y_ptr: int, units: SygUnits, n_fft: int, hop: int, win_length: int, window: int, center: bool,
                  pad_mode: int, out_kind: int, out_ptr: int, stream: int = 0) -> None:

@@ -3,6 +3,9 @@
 * :func:`extract_features_batch`  -- many equal-length clips in one launch (BASELINE cfg3 shape)
 * :func:`segment_features`        -- ``segment_fixed_length`` + ``extract_features`` per segment fused into one launch over
                                      the un-segmented recording (BASELINE cfg4 shape); segments are framed by index
+* :func:`extract_features_ragged`, :func:`clip_vectors`
+                                  -- clips of different lengths (a folder of files, variable-length segments) in one launch,
+                                     each clip framed on its own: no padding to the longest
 * :func:`stft_batch`, :func:`psd_welch_batch`
 
 Inputs may be numpy arrays (host path: chunked H2D / kernels / D2H inside the library) or CUDA ``torch`` tensors (device
@@ -10,7 +13,7 @@ path: asynchronous on the current torch stream, result stays in HBM).  Row namin
 """
 from __future__ import annotations
 
-from typing import Dict, List, Optional, Sequence, Tuple
+from typing import Dict, List, NamedTuple, Optional, Sequence, Tuple
 
 import numpy as np
 
@@ -104,6 +107,105 @@ def segment_features(y, sr: int, segment_length_sec: float, features: Sequence[s
     del keep
     return {"names": feature_row_names(features, feature_params), "features": out, "starts": starts, "valid": valid,
             "seg_len": seg_len, "seg_hop": seg_hop}
+
+
+class Windows(NamedTuple):
+    """Windows of ONE sample buffer as ragged clips, without a copy: clip ``u`` is ``y[starts[u] : starts[u] + lengths[u]]``
+    (windows may overlap or leave gaps; e.g. the variable-length segments of one recording).  ``y``: 1-D float32 numpy array or
+    CUDA tensor; ``starts`` / ``lengths``: integer sequences (numpy, lists or torch tensors on any device)."""
+    y: object
+    starts: object
+    lengths: object
+
+
+def _int_table(t) -> np.ndarray:
+    if _is_torch(t):
+        t = t.detach().cpu().numpy()
+    a = np.asarray(t)
+    if a.size and a.dtype.kind not in "iu":
+        raise ValueError("starts and lengths must be integers")
+    return a.astype(np.int64).reshape(-1)
+
+
+def _ragged_input(clips):
+    """``clips`` -> (y, starts, lengths).  A :class:`Windows` is taken as it is; anything else is a sequence of 1-D clips, concatenated
+    once (numpy arrays -> host path, CUDA tensors -> device path)."""
+    if isinstance(clips, Windows):
+        if getattr(clips.y, "ndim", None) != 1:
+            raise ValueError("Windows.y must be a 1-D sample buffer")
+        starts, lengths = _int_table(clips.starts), _int_table(clips.lengths)
+        if starts.shape != lengths.shape:
+            raise ValueError("Windows.starts and Windows.lengths must have the same length")
+        return clips.y, starts, lengths
+    clips = list(clips)
+    for c in clips:
+        if getattr(c, "ndim", None) != 1:
+            raise ValueError("every clip must be a 1-D array (use batch.Windows for windows of one buffer)")
+    lengths = np.array([int(c.shape[0]) for c in clips], dtype=np.int64)
+    starts = np.concatenate([[0], np.cumsum(lengths)[:-1]]).astype(np.int64) if len(clips) else np.zeros(0, dtype=np.int64)
+    if clips and all(_is_torch(c) for c in clips):
+        import torch
+        if not all(c.is_cuda for c in clips):
+            raise ValueError("torch inputs must live on a CUDA device (use numpy arrays for host data)")
+        return torch.cat([c.float() for c in clips]), starts, lengths
+    if any(_is_torch(c) for c in clips):
+        raise ValueError("clips must be all numpy arrays or all CUDA tensors")
+    y = np.concatenate([np.asarray(c, dtype=np.float32) for c in clips]) if clips else np.zeros(0, dtype=np.float32)
+    return y, starts, lengths
+
+
+def _ragged_call(clips, sr, features, frame_length, hop_length, center, window, feature_params, device, agg=None):
+    y, starts, lengths = _ragged_input(clips)
+    if getattr(y, "ndim", None) != 1:
+        raise ValueError("the sample buffer must be 1-D")
+    eng = _engine_for(y, device)
+    p = _ffi.make_params(eng.lib, sr, list(features), frame_length, hop_length, center, window, feature_params)
+    units = eng.ragged_units(starts, lengths, int(y.shape[0]))
+    names = feature_row_names(features, feature_params)
+    ids = None
+    if agg is not None:
+        from .core.ml_utils.formatters import _agg_ids
+        ids = _agg_ids(names, agg)
+    foff = eng.lib.ragged_frame_offsets(units, frame_length, hop_length, center)
+    rows = eng.rows(p)
+    if _is_torch(y):
+        import torch
+        if not y.is_cuda:
+            raise ValueError("torch inputs must live on a CUDA device (use numpy arrays for host data)")
+        if y.dtype != torch.float32 or not y.is_contiguous():
+            y = y.contiguous().float()
+        stream = torch.cuda.current_stream(y.device).cuda_stream
+        if ids is None:
+            out = torch.empty((rows, int(foff[-1])), dtype=torch.float32, device=y.device)
+            eng.features_ragged_dev(y.data_ptr(), units, p, out.data_ptr(), stream)
+        else:
+            out = torch.empty((len(lengths), rows), dtype=torch.float64, device=y.device)
+            eng.segment_vectors_ragged_dev(y.data_ptr(), units, p, ids, out.data_ptr(), stream)
+    else:
+        y = np.ascontiguousarray(y, dtype=np.float32)
+        out = eng.features_ragged_host(y, units, p) if ids is None else eng.segment_vectors_ragged_host(y, units, p, ids)
+    return names, out, foff
+
+
+def extract_features_ragged(clips, sr: int, features: Sequence[str], frame_length: int = 2048, hop_length: int = 512,
+                            center: bool = True, window: str = "hann", feature_params: Optional[dict] = None,
+                            device: Optional[int] = None) -> Dict[str, object]:
+    """Clips of different lengths in one launch.  ``clips``: a sequence of 1-D arrays (numpy: host path; CUDA tensors: device path,
+    asynchronous on the current stream) or a :class:`Windows` ``(y, starts, lengths)`` addressing windows of one buffer without a copy.
+    Returns {'names', 'features': float32 ``[rows, F]``, 'frame_offsets': int64 ``[n_clips + 1]``}: columns
+    ``frame_offsets[c] .. frame_offsets[c + 1] - 1`` are exactly ``extract_features(clip c, ...)`` (the layout of
+    ``format_feature_vectors_per_segment``'s features_dict with those ranges as segment indices)."""
+    names, out, foff = _ragged_call(clips, sr, features, frame_length, hop_length, center, window, feature_params, device)
+    return {"names": names, "features": out, "frame_offsets": foff}
+
+
+def clip_vectors(clips, sr: int, features: Sequence[str], aggregation="mean", frame_length: int = 2048, hop_length: int = 512,
+                 center: bool = True, window: str = "hann", feature_params: Optional[dict] = None, device: Optional[int] = None):
+    """One vector per clip: ``extract_features`` per clip followed by ``format_feature_vectors_per_segment`` with every clip as one
+    segment.  ``clips`` as in :func:`extract_features_ragged`; ``aggregation`` a name or a per-row dict (formatters.py:39-45).
+    Returns (row names, float64 ``[n_clips, rows]``); a clip without frames gives a NaN row."""
+    names, out, _ = _ragged_call(clips, sr, features, frame_length, hop_length, center, window, feature_params, device, agg=aggregation)
+    return names, out
 
 
 def stft_batch(clips, n_fft: int = 2048, hop_length: Optional[int] = None, win_length: Optional[int] = None, window: str = "hann",

@@ -11,7 +11,8 @@ ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libsygb200.so")
 SOURCES = [os.path.join(CSRC, f) for f in ("syg_api.cu", "syg_launch_block.cu", "syg_launch_warp.cu", "syg_launch_warp_stft.cu", "syg_launch_stft_ring.cu", "syg_launch_stft_big.cu",
-                                             "syg_launch_warp_extra.cu", "syg_launch_warp_spec44k.cu", "syg_launch_warp_spec44kl.cu", "syg_launch_warp_spec22k.cu", "syg_launch_welch.cu", "syg_launch_ingest.cu", "syg_launch_agg.cu", "syg_launch_timefeat.cu", "syg_launch_matrix.cu", "syg_launch_mixed.cu", "syg_launch_warp_res.cu")]
+                                             "syg_launch_warp_extra.cu", "syg_launch_warp_spec44k.cu", "syg_launch_warp_spec44kl.cu", "syg_launch_warp_spec22k.cu", "syg_launch_welch.cu", "syg_launch_ingest.cu", "syg_launch_agg.cu", "syg_launch_timefeat.cu", "syg_launch_matrix.cu", "syg_launch_mixed.cu", "syg_launch_warp_res.cu",
+                                             "syg_launch_ragged.cu", "syg_launch_ragged_spec.cu")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC"]
 OBJDIR = os.path.join(ROOT, "build", "obj")
 

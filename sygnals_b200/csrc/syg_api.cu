@@ -287,14 +287,17 @@ int launch_features(int n_fft, const syg::FrameArgs& a_in, int sm_count, cudaStr
     if (variant < 0) { const char* e = std::getenv("SYGB200_VARIANT"); variant = e ? std::atoi(e) : 0; }
     syg::FrameArgs a = a_in;
     a.variant = variant;
+    const bool rag = a.ragged_ut != nullptr;
+    const int mode = rag ? sygdev::MODE_FEATURES_RAGGED : sygdev::MODE_FEATURES;
     if (!native_pow2(n_fft)) {
         syg::MixedPlan mp;
         if (int rc = mixed_plan_of(n_fft, true, mp, "frame_length")) return rc;
-        return launch_rc(syglaunch::frame_mixed(sygdev::MODE_FEATURES, a, mp, sm_count, st, err), err);
+        return launch_rc(syglaunch::frame_mixed(mode, a, mp, sm_count, st, err), err);
     }
-    if (n_fft > 2048) return launch_rc(syglaunch::frame_block(n_fft, sygdev::MODE_FEATURES, a, sm_count, st, err), err);
+    if (n_fft > 2048) return launch_rc(syglaunch::frame_block(n_fft, mode, a, sm_count, st, err), err);
     if (a.res_units > 0) return launch_rc(syglaunch::frame_warp_res(n_fft, a, sm_count, st, err), err);
     constexpr unsigned extra = syg::FB_BANDWIDTH | syg::FB_FLATNESS | syg::FB_DOMINANT | syg::FB_MEAN_AMP | syg::FB_STD_AMP;
+    if (rag) return launch_rc(syglaunch::frame_warp_ragged(n_fft, (a.mask & extra) != 0, a, sm_count, st, err), err);
     return launch_rc(syglaunch::frame_warp(n_fft, (a.mask & extra) != 0, a, sm_count, st, err), err);
 }
 
@@ -306,6 +309,7 @@ int warp_fw(int n_fft) {
 int g_resident_min_groups = -1;     // unit groups a launch needs before the resident kernel is chosen (-1: 4 per SM); tests lower it
 int g_last_mel_form = 0;            // 1: the last feature launch with MFCCs used the interval-form mel projection
 int g_last_features_resident = 0;   // 1: the last feature launch kept its units on chip (frame_warp_kernel STAGE 5)
+long long g_last_feature_frames = 0; // frames the feature kernels processed in the last syg_features_* / syg_segment_vectors_* call
 int g_last_stft_path = 0;   // 5 mixed-radix kernel (lengths that are not powers of two), 1 ring (TMA-staged), 2 warp kernel (register-staged), 3 CTA-cooperative kernels, 4 sub-FFT kernel (n_fft 4096 / 8192): last STFT launch
 
 int launch_stft(int n_fft, const syg::FrameArgs& a, int sm_count, cudaStream_t st) {
@@ -603,6 +607,7 @@ int run_features_chunk(syg_ctx* ctx, const FeaturePlan& pl, const float* y, cons
         }
     }
     g_last_features_resident = a.res_units > 0 ? 1 : 0;
+    g_last_feature_frames += a.n_frames;
     if (a.mask & syg::FB_MFCC) g_last_mel_form = a.mel_iv ? 1 : 0;
     const bool need_fin = (a.mask & (syg::FB_MFCC | syg::FB_CONTRAST)) != 0 && a.res_units == 0;
     if (need_fin) CK(cudaMemsetAsync(a.unit_max, 0, (size_t)g.n_units * 4 * sizeof(unsigned), st));
@@ -864,6 +869,310 @@ int welch_setup(syg_ctx* ctx, const syg_units* u, double fs, int window, int npe
     return mixed ? get_mixed_tables(ctx, nfft, &a.tw, &a.tws) : get_fft_tables(ctx, nfft, &a.tw, &a.tws);
 }
 
+
+// ---------------------------------------------------------------------------------------------- ragged batches
+// Every unit keeps its own length: unit u is y[starts[u], starts[u] + lengths[u]) with T_u frames, the frame axis is the
+// concatenation of the units' frames (frame_off), the feature kernels read a frame's unit, frame index, unit length and start from a
+// per-frame table {u, t, len, start} that ragged_frame_table_kernel writes from frame_off and the unit tables.  Chunks are cut by
+// cumulative frames and samples, never inside a unit.  A chunk may hold only units without frames: no feature kernel runs for it
+// (a launch of zero CTAs is an error), and its segment vectors are the NaN rows of the aggregation.
+
+// validates the tables (host memory) and fills frame_off [n_units + 1]; the plan arguments are checked by build_feature_plan
+int check_ragged(const syg_ragged_units* u, int fl, int hop, int center, std::vector<long long>* frame_off) {
+    if (!u) return fail(SYG_E_BADARG, "units is NULL");
+    if (u->n_units < 0 || u->total_len < 0) return fail(SYG_E_BADARG, "negative unit geometry");
+    if (u->n_units > 0 && (!u->starts || !u->lengths)) return fail(SYG_E_BADARG, "unit tables are NULL");
+    if (frame_off) frame_off->assign((size_t)u->n_units + 1, 0);
+    long long F = 0;
+    for (long long i = 0; i < u->n_units; ++i) {
+        const long long s = u->starts[i], l = u->lengths[i];
+        if (s < 0 || l < 0) return fail(SYG_E_BADARG, "unit %lld: negative start or length", i);
+        if (s > u->total_len || l > u->total_len - s) return fail(SYG_E_BADARG, "unit %lld lies outside the sample buffer", i);
+        if (l > 0x7fffffffLL) return fail(SYG_E_UNSUPPORTED, "unit %lld: length above 2^31-1 samples", i);
+        const long long T = syg_frame_count(l, fl, hop, center);
+        if (T > 0x7fffffffLL) return fail(SYG_E_UNSUPPORTED, "unit %lld: more than 2^31-1 frames", i);
+        F += T;
+        if (frame_off) (*frame_off)[(size_t)i + 1] = F;
+    }
+    return SYG_OK;
+}
+
+size_t al256(size_t b) { return (b + 255) / 256 * 256; }
+
+// device tables of a ragged call, per unit: frame_off (int64, one more entry), starts (int64), lengths (int32), and for the
+// aggregation the unit's first frame relative to its chunk (int64) and its frame count (int32)
+size_t ragged_tbl_bytes(long long n, bool agg) {
+    return al256((size_t)(n + 1) * 8) + al256((size_t)n * 8) + al256((size_t)n * 4) + (agg ? al256((size_t)n * 8) + al256((size_t)n * 4) : 0);
+}
+struct RaggedTbl { long long* foff; long long* starts; int* valid; long long* seg_off; int* seg_len; };
+RaggedTbl ragged_tbl_at(void* base, long long n, bool agg) {
+    char* p = reinterpret_cast<char*>(base);
+    RaggedTbl t;
+    t.foff = reinterpret_cast<long long*>(p); p += al256((size_t)(n + 1) * 8);
+    t.starts = reinterpret_cast<long long*>(p); p += al256((size_t)n * 8);
+    t.valid = reinterpret_cast<int*>(p); p += al256((size_t)n * 4);
+    t.seg_off = agg ? reinterpret_cast<long long*>(p) : nullptr; p += agg ? al256((size_t)n * 8) : 0;
+    t.seg_len = agg ? reinterpret_cast<int*>(p) : nullptr;
+    return t;
+}
+// workspace of a chunk of n units and nf frames: unit maxima, mel energies, contrast peaks / valleys, the frame table, and for
+// the aggregation the chunk's frame features [n_rows][nf]
+size_t ragged_ws_bytes(const FeaturePlan& pl, long long n, long long nf, bool agg) {
+    size_t b = al256((size_t)n * 4 * sizeof(unsigned)) + al256((size_t)nf * pl.fin.n_mels * sizeof(float)) +
+               al256((size_t)nf * 2 * pl.fin.nb * sizeof(float)) + al256((size_t)nf * sizeof(int4));
+    if (agg) b += al256((size_t)nf * pl.n_rows * sizeof(float));
+    return b + 256;
+}
+
+struct RaggedChunk {
+    long long u0, n;               // units
+    long long f0, nf;              // frames
+    long long b, e;                // samples of y the units cover
+};
+
+// host image of the tables of chunk c's units, at entries [at, at + c.n] of t (starts relative to the chunk's first sample, seg_off to
+// its first frame)
+void ragged_tbl_fill(const RaggedTbl& t, long long at, const syg_ragged_units* u, const std::vector<long long>& foff, const RaggedChunk& c) {
+    for (long long i = 0; i <= c.n; ++i) t.foff[at + i] = foff[(size_t)(c.u0 + i)];
+    for (long long i = 0; i < c.n; ++i) {
+        const long long l = u->lengths[c.u0 + i];
+        t.starts[at + i] = l > 0 ? u->starts[c.u0 + i] - c.b : 0;
+        t.valid[at + i] = (int)l;
+        if (t.seg_off) {
+            t.seg_off[at + i] = foff[(size_t)(c.u0 + i)] - c.f0;
+            t.seg_len[at + i] = (int)(foff[(size_t)(c.u0 + i + 1)] - foff[(size_t)(c.u0 + i)]);
+        }
+    }
+}
+
+// greedy cut: a chunk takes units while its workspace stays within ws_limit and its samples / frames within the caps; a unit that
+// exceeds them alone runs alone
+void ragged_chunks(const syg_ragged_units* u, const std::vector<long long>& foff, const FeaturePlan& pl, bool agg, size_t ws_limit,
+                   long long max_samples, long long max_frames, std::vector<RaggedChunk>& out) {
+    out.clear();
+    RaggedChunk c{0, 0, 0, 0, 0, 0};
+    long long b = u->total_len, e = 0;
+    for (long long i = 0; i < u->n_units; ++i) {
+        const long long T = foff[(size_t)i + 1] - foff[(size_t)i];
+        const long long s = u->starts[i], l = u->lengths[i];
+        const long long nb = l > 0 ? std::min(b, s) : b, ne = l > 0 ? std::max(e, s + l) : e;
+        if (c.n > 0 && (ragged_ws_bytes(pl, c.n + 1, c.nf + T, agg) > ws_limit || std::max(ne - nb, 0LL) > max_samples ||
+                        c.nf + T > max_frames || c.n + 1 > 0x7fffffffLL)) {
+            c.b = e > b ? b : 0; c.e = e > b ? e : 0;
+            out.push_back(c);
+            c = RaggedChunk{i, 0, foff[(size_t)i], 0, 0, 0};
+            b = u->total_len; e = 0;
+            if (l > 0) { b = s; e = s + l; }
+        } else {
+            b = nb; e = ne;
+        }
+        c.n += 1;
+        c.nf += T;
+    }
+    if (c.n > 0) { c.b = e > b ? b : 0; c.e = e > b ? e : 0; out.push_back(c); }
+}
+
+// the feature kernels on one chunk: y and the tables are chunk-relative, rows go to out[r * out_stride + f] (f < nf)
+int run_ragged_chunk(syg_ctx* ctx, const FeaturePlan& pl, const float* y, const RaggedTbl& t, long long n, long long nf, float* out,
+                     long long out_stride, void* ws, int n_fft, cudaStream_t st) {
+    syg::FrameArgs a = pl.fa;
+    a.y = y;
+    a.g.n_units = n;
+    a.g.unit_len = 0x7fffffffLL;           // the kernels take a unit's start and length from the frame table
+    a.g.unit_stride = 0;
+    a.g.total_len = 0;
+    a.g.unit_starts = nullptr;
+    a.g.unit_valid = nullptr;
+    a.g.unit0 = 0;
+    a.T = 0;
+    a.n_frames = nf;
+    a.out = out;
+    a.ragged_stride = out_stride;
+    a.res_units = 0;                       // the unit-resident epilogue sizes its tile by units x T: uniform launches only
+    char* w = reinterpret_cast<char*>(ws);
+    a.unit_max = reinterpret_cast<unsigned*>(w);
+    size_t off = al256((size_t)n * 4 * sizeof(unsigned));
+    a.melws = reinterpret_cast<float*>(w + off);
+    off += al256((size_t)nf * pl.fin.n_mels * sizeof(float));
+    a.cws = reinterpret_cast<float*>(w + off);
+    off += al256((size_t)nf * 2 * pl.fin.nb * sizeof(float));
+    int4* ut = reinterpret_cast<int4*>(w + off);
+    a.ragged_ut = ut;
+    g_last_features_resident = 0;
+    g_last_feature_frames += nf;
+    if (a.mask & syg::FB_MFCC) g_last_mel_form = a.mel_iv ? 1 : 0;
+    if (nf == 0) return SYG_OK;            // only units without frames: nothing to compute (and no zero-CTA finalize launch)
+    std::string err;
+    {
+        ProfScope ps(ctx, st, PROF_OTHER);
+        if (int trc = syglaunch::ragged_frame_table(t.foff, t.starts, t.valid, n, nf, ut, ctx->sm_count, st, err)) return fail(trc, "%s", err.c_str());
+    }
+    const bool need_fin = (a.mask & (syg::FB_MFCC | syg::FB_CONTRAST)) != 0;
+    if (need_fin) CK(cudaMemsetAsync(a.unit_max, 0, (size_t)n * 4 * sizeof(unsigned), st));
+    if (a.mask & syg::FB_TIME_EXTRA) {
+        ProfScope ps(ctx, st, PROF_FRAME);
+        if (int trc = syglaunch::time_extra(a, n_fft, pl.entropy_bins, ctx->sm_count, st, err)) return fail(trc, "%s", err.c_str());
+    }
+    if ((a.mask & ~syg::FB_TIME_EXTRA) == 0) return SYG_OK;
+    {
+        ProfScope ps(ctx, st, PROF_FRAME);
+        if (int rc = launch_features(n_fft, a, ctx->sm_count, st)) return rc;
+    }
+    if (!need_fin) return SYG_OK;
+    ProfScope ps(ctx, st, PROF_FINALIZE);
+    syg::FinalizeArgs f = pl.fin;
+    f.n_units = n;
+    f.T = 0;
+    f.melws = a.melws;
+    f.cws = a.cws;
+    f.unit_max = a.unit_max;
+    f.out = out;
+    f.ragged_ut = ut;
+    f.n_frames = nf;
+    f.ragged_stride = out_stride;
+    const int tt = (f.row_mfcc >= 0 && f.n_mels <= 64) ? 64 : 32;     // as run_features_chunk
+    const size_t smem = sygdev::fin_smem_bytes(tt, f.n_mels, f.dct_fold != 0);
+    const unsigned grid = (unsigned)std::min<long long>((nf + tt - 1) / tt, 0x7fffffffLL);
+    if (int frc = syglaunch::finalize(f, tt, grid, 1u, smem, st, err)) return fail(frc, "%s", err.c_str());
+    return SYG_OK;
+}
+
+int check_agg(const FeaturePlan& pl, const int32_t* agg) {
+    if (pl.n_rows > 64) return fail(SYG_E_UNSUPPORTED, "aggregation supports at most 64 rows per call");
+    for (int i = 0; i < pl.n_rows; ++i)
+        if (agg[i] < SYG_AGG_MEAN || agg[i] > SYG_AGG_MAX) return fail(SYG_E_BADARG, "unknown aggregation id %d", agg[i]);
+    return SYG_OK;
+}
+
+// agg == nullptr: out is float32 [n_rows][F]; else float64 [n_units][n_rows]
+int ragged_dev_impl(syg_ctx* ctx, const float* y_dev, const syg_ragged_units* units, const syg_feature_params* p, const int32_t* agg,
+                    void* out_dev, cudaStream_t st) {
+    if (!ctx) return fail(SYG_E_BADARG, "ctx is NULL");
+    if (!p) return fail(SYG_E_BADARG, "params is NULL");
+    std::vector<long long> foff;
+    int rc = check_ragged(units, p->frame_length, p->hop_length, p->center, &foff);
+    if (rc) return rc;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    ENTER_DEVICE(ctx);
+    FeaturePlan pl;
+    syg_units pu{};                                   // the plan's per-unit frame count is not used by ragged launches
+    if ((rc = build_feature_plan(ctx, &pu, p, pl))) return rc;
+    const long long n_units = units->n_units, F = foff.back();
+    if (n_units == 0 || F == 0 || pl.n_rows == 0) return SYG_OK;
+    if (!y_dev && units->total_len > 0) return fail(SYG_E_BADARG, "y_dev is NULL");
+    if (!out_dev) return fail(SYG_E_BADARG, "out_dev is NULL");
+    if (agg && (rc = check_agg(pl, agg))) return rc;
+    const bool ag = agg != nullptr;
+    std::vector<RaggedChunk> chunks;
+    ragged_chunks(units, foff, pl, ag, ctx->ws_limit, 0x7fffffffLL, 1LL << 62, chunks);     // starts < 2^31 in the frame table
+    size_t ws_max = 0;
+    for (const RaggedChunk& c : chunks) ws_max = std::max(ws_max, ragged_ws_bytes(pl, c.n, c.nf, ag));
+    const size_t tbl_bytes = ragged_tbl_bytes(n_units, ag);
+    // the tables of all units go through lane 0's pinned staging block in one copy; the block is rewritten only after the copy that
+    // read it last has completed
+    Lane& L = ctx->lanes[0];
+    if (!L.tbl_done) CK(cudaEventCreateWithFlags(&L.tbl_done, cudaEventDisableTiming));
+    if (L.tbl_used) CK(cudaEventSynchronize(L.tbl_done));
+    if ((rc = L.tbl.ensure(tbl_bytes))) return rc;
+    const RaggedTbl ht = ragged_tbl_at(L.tbl.p, n_units, ag);
+    for (const RaggedChunk& c : chunks) ragged_tbl_fill(ht, c.u0, units, foff, c);
+    if (ctx->ws_done) CK(cudaStreamWaitEvent(st, ctx->ws_done, 0));
+    else CK(cudaEventCreateWithFlags(&ctx->ws_done, cudaEventDisableTiming));
+    if (tbl_bytes + ws_max > ctx->ws.cap) CK(cudaStreamSynchronize(st));   // growing frees the old block: nothing may still use it
+    if ((rc = ctx->ws.ensure(tbl_bytes + ws_max))) return rc;
+    struct Done { syg_ctx* c; cudaStream_t s; ~Done() { cudaEventRecord(c->ws_done, s); } } done_{ctx, st};
+    CK(cudaMemcpyAsync(ctx->ws.p, L.tbl.p, tbl_bytes, cudaMemcpyHostToDevice, st));
+    CK(cudaEventRecord(L.tbl_done, st));
+    L.tbl_used = true;
+    const RaggedTbl dt = ragged_tbl_at(ctx->ws.p, n_units, ag);
+    void* ws = reinterpret_cast<char*>(ctx->ws.p) + tbl_bytes;
+    for (const RaggedChunk& c : chunks) {
+        RaggedTbl ct{dt.foff + c.u0, dt.starts + c.u0, dt.valid + c.u0, ag ? dt.seg_off + c.u0 : nullptr, ag ? dt.seg_len + c.u0 : nullptr};
+        float* feat = ag ? reinterpret_cast<float*>(reinterpret_cast<char*>(ws) + ragged_ws_bytes(pl, c.n, c.nf, true) - 256 -
+                                                    al256((size_t)c.nf * pl.n_rows * sizeof(float)))
+                         : reinterpret_cast<float*>(out_dev) + c.f0;
+        if ((rc = run_ragged_chunk(ctx, pl, y_dev + c.b, ct, c.n, c.nf, feat, ag ? c.nf : F, ws, p->frame_length, st))) return rc;
+        if (!ag) continue;
+        std::string err;
+        ProfScope ps(ctx, st, PROF_OTHER);
+        const int arc = syglaunch::aggregate(feat, c.n, pl.n_rows, c.nf, ct.seg_off, ct.seg_len, 0, agg,
+                                             reinterpret_cast<double*>(out_dev) + (size_t)c.u0 * pl.n_rows, ctx->sm_count, st, err);
+        if (arc) return fail(arc, "%s", err.c_str());
+    }
+    return SYG_OK;
+}
+
+// host forms: chunks alternate between the two lanes (H2D of the chunk's samples and tables, kernels, D2H overlapped)
+int ragged_host_impl(syg_ctx* ctx, const float* y_host, const syg_ragged_units* units, const syg_feature_params* p, const int32_t* agg,
+                     void* out_host) {
+    if (!ctx) return fail(SYG_E_BADARG, "ctx is NULL");
+    if (!p) return fail(SYG_E_BADARG, "params is NULL");
+    std::vector<long long> foff;
+    int rc = check_ragged(units, p->frame_length, p->hop_length, p->center, &foff);
+    if (rc) return rc;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    ENTER_DEVICE(ctx);
+    FeaturePlan pl;
+    syg_units pu{};
+    if ((rc = build_feature_plan(ctx, &pu, p, pl))) return rc;
+    const long long n_units = units->n_units, F = foff.back();
+    if (n_units == 0 || F == 0 || pl.n_rows == 0) return SYG_OK;
+    if (!y_host && units->total_len > 0) return fail(SYG_E_BADARG, "y_host is NULL");
+    if (!out_host) return fail(SYG_E_BADARG, "out_host is NULL");
+    if (agg && (rc = check_agg(pl, agg))) return rc;
+    const bool ag = agg != nullptr;
+    // 128 MiB of samples and 256 MiB of frame features per chunk (host_pipeline's targets); at least two chunks keep both lanes busy
+    long long max_frames = std::max<long long>(1, (long long)(((size_t)256 << 20) / ((size_t)pl.n_rows * sizeof(float))));
+    if (n_units > 1) max_frames = std::min<long long>(max_frames, std::max<long long>(1, (F + 1) / 2));
+    std::vector<RaggedChunk> chunks;
+    ragged_chunks(units, foff, pl, ag, ctx->ws_limit, (long long)(((size_t)128 << 20) / sizeof(float)), max_frames, chunks);
+    for (int l = 0; l < 2; ++l) {
+        if (!ctx->lanes[l].stream) CK(cudaStreamCreateWithFlags(&ctx->lanes[l].stream, cudaStreamNonBlocking));
+        if (!ctx->lanes[l].tbl_done) CK(cudaEventCreateWithFlags(&ctx->lanes[l].tbl_done, cudaEventDisableTiming));
+    }
+    int li = 0;
+    for (const RaggedChunk& c : chunks) {
+        Lane& L = ctx->lanes[li];
+        li ^= 1;
+        const size_t tbl_bytes = ragged_tbl_bytes(c.n, ag);
+        const size_t out_bytes = ag ? (size_t)c.n * pl.n_rows * sizeof(double) : (size_t)c.nf * pl.n_rows * sizeof(float);
+        if ((rc = L.in.ensure(std::max<size_t>((size_t)(c.e - c.b) * sizeof(float), 256)))) return rc;
+        if ((rc = L.out0.ensure(std::max<size_t>(out_bytes, 256)))) return rc;
+        if ((rc = L.ws.ensure(tbl_bytes + ragged_ws_bytes(pl, c.n, c.nf, ag)))) return rc;
+        // the lane's previous chunk has left its device buffers when this chunk's work reaches them (same stream => ordered)
+        if (c.e > c.b) CK(cudaMemcpyAsync(L.in.p, y_host + c.b, (size_t)(c.e - c.b) * sizeof(float), cudaMemcpyHostToDevice, L.stream));
+        if (L.tbl_used) CK(cudaEventSynchronize(L.tbl_done));
+        if ((rc = L.tbl.ensure(tbl_bytes))) return rc;
+        ragged_tbl_fill(ragged_tbl_at(L.tbl.p, c.n, ag), 0, units, foff, c);
+        CK(cudaMemcpyAsync(L.ws.p, L.tbl.p, tbl_bytes, cudaMemcpyHostToDevice, L.stream));
+        CK(cudaEventRecord(L.tbl_done, L.stream));
+        L.tbl_used = true;
+        const RaggedTbl ct = ragged_tbl_at(L.ws.p, c.n, ag);
+        void* ws = reinterpret_cast<char*>(L.ws.p) + tbl_bytes;
+        float* feat = ag ? reinterpret_cast<float*>(reinterpret_cast<char*>(ws) + ragged_ws_bytes(pl, c.n, c.nf, true) - 256 -
+                                                    al256((size_t)c.nf * pl.n_rows * sizeof(float)))
+                         : reinterpret_cast<float*>(L.out0.p);
+        if ((rc = run_ragged_chunk(ctx, pl, reinterpret_cast<const float*>(L.in.p), ct, c.n, c.nf, feat, c.nf, ws, p->frame_length,
+                                   L.stream)))
+            return rc;
+        if (ag) {
+            std::string err;
+            ProfScope ps(ctx, L.stream, PROF_OTHER);
+            const int arc = syglaunch::aggregate(feat, c.n, pl.n_rows, c.nf, ct.seg_off, ct.seg_len, 0, agg,
+                                                 reinterpret_cast<double*>(L.out0.p), ctx->sm_count, L.stream, err);
+            if (arc) return fail(arc, "%s", err.c_str());
+            CK(cudaMemcpyAsync(reinterpret_cast<double*>(out_host) + (size_t)c.u0 * pl.n_rows, L.out0.p, out_bytes, cudaMemcpyDeviceToHost,
+                               L.stream));
+        } else {
+            for (int r = 0; r < pl.n_rows; ++r)          // row r of the chunk lands at columns [f0, f0 + nf) of output row r
+                CK(cudaMemcpyAsync(reinterpret_cast<float*>(out_host) + (size_t)r * F + c.f0, reinterpret_cast<float*>(L.out0.p) + (size_t)r * c.nf,
+                                   (size_t)c.nf * sizeof(float), cudaMemcpyDeviceToHost, L.stream));
+        }
+    }
+    for (int l = 0; l < 2; ++l) CK(cudaStreamSynchronize(ctx->lanes[l].stream));
+    return SYG_OK;
+}
+
 }  // namespace
 
 // ================================================================================================ C ABI
@@ -989,6 +1298,7 @@ int64_t syg_frame_count(int64_t n_samples, int32_t frame_length, int32_t hop_len
 int syg_features_f32(syg_ctx* ctx, const float* y_dev, const syg_units* units, const syg_feature_params* p,
                      float* out_dev, void* stream) {
     SYG_TRACE();
+    g_last_feature_frames = 0;
     if (!ctx) return fail(SYG_E_BADARG, "ctx is NULL");
     int rc = check_units(units);
     if (rc) return rc;
@@ -1022,6 +1332,7 @@ int syg_features_f32(syg_ctx* ctx, const float* y_dev, const syg_units* units, c
 static int features_host_impl(syg_ctx* ctx, const void* y_host, InFmt inf, const syg_units* units, const syg_feature_params* p,
                               const int32_t* agg, void* out_host) {
     NvtxRange nvtx_range_(agg ? "syg_segment_vectors_host" : "syg_features_host");
+    g_last_feature_frames = 0;
     if (!ctx) return fail(SYG_E_BADARG, "ctx is NULL");
     if (inf.fmt >= 0 && (inf.fmt > SYG_PCM_F32 || inf.channels < 1 || inf.channels > 64))
         return fail(SYG_E_BADARG, "bad PCM layout (format %d, %d channels)", inf.fmt, inf.channels);
@@ -1094,6 +1405,7 @@ int syg_segment_vectors_host_pcm(syg_ctx* ctx, const void* raw_host, int32_t sam
 int syg_segment_vectors_f32(syg_ctx* ctx, const float* y_dev, const syg_units* units, const syg_feature_params* p,
                             const int32_t* agg, double* out_dev, void* stream) {
     SYG_TRACE();
+    g_last_feature_frames = 0;
     if (!ctx) return fail(SYG_E_BADARG, "ctx is NULL");
     if (!agg) return fail(SYG_E_BADARG, "agg is NULL");
     int rc = check_units(units);
@@ -1131,6 +1443,46 @@ int syg_segment_vectors_f32(syg_ctx* ctx, const float* y_dev, const syg_units* u
         if (arc) return fail(arc, "%s", err.c_str());
     }
     return SYG_OK;
+}
+
+int64_t syg_ragged_frame_offsets(const syg_ragged_units* units, int32_t frame_length, int32_t hop_length, int32_t center,
+                                 int64_t* frame_off) {
+    if (frame_length < 1 || hop_length < 1) return fail(SYG_E_BADARG, "frame_length and hop_length must be >= 1");
+    std::vector<long long> foff;
+    const int rc = check_ragged(units, frame_length, hop_length, center, &foff);
+    if (rc) return rc;
+    if (frame_off) for (size_t i = 0; i < foff.size(); ++i) frame_off[i] = foff[i];
+    return foff.back();
+}
+
+int syg_features_ragged_f32(syg_ctx* ctx, const float* y_dev, const syg_ragged_units* units, const syg_feature_params* p,
+                            float* out_dev, void* stream) {
+    SYG_TRACE();
+    g_last_feature_frames = 0;
+    return ragged_dev_impl(ctx, y_dev, units, p, nullptr, out_dev, reinterpret_cast<cudaStream_t>(stream));
+}
+
+int syg_features_ragged_host_f32(syg_ctx* ctx, const float* y_host, const syg_ragged_units* units, const syg_feature_params* p,
+                                 float* out_host) {
+    SYG_TRACE();
+    g_last_feature_frames = 0;
+    return ragged_host_impl(ctx, y_host, units, p, nullptr, out_host);
+}
+
+int syg_segment_vectors_ragged_f32(syg_ctx* ctx, const float* y_dev, const syg_ragged_units* units, const syg_feature_params* p,
+                                   const int32_t* agg, double* out_dev, void* stream) {
+    SYG_TRACE();
+    g_last_feature_frames = 0;
+    if (!agg) return fail(SYG_E_BADARG, "agg is NULL");
+    return ragged_dev_impl(ctx, y_dev, units, p, agg, out_dev, reinterpret_cast<cudaStream_t>(stream));
+}
+
+int syg_segment_vectors_ragged_host_f32(syg_ctx* ctx, const float* y_host, const syg_ragged_units* units,
+                                        const syg_feature_params* p, const int32_t* agg, double* out_host) {
+    SYG_TRACE();
+    g_last_feature_frames = 0;
+    if (!agg) return fail(SYG_E_BADARG, "agg is NULL");
+    return ragged_host_impl(ctx, y_host, units, p, agg, out_host);
 }
 
 int syg_ingest_pcm(syg_ctx* ctx, const void* raw_dev, int32_t sample_format, int32_t channels, int64_t n_frames, float* mono_dev,
@@ -1357,6 +1709,7 @@ int syg_spectral_contrast_from_mag_f32(syg_ctx* ctx, const float* S_dev, int32_t
 
 int syg_debug_last_stft_path(void) { return g_last_stft_path; }
 int syg_debug_last_features_resident(void) { return g_last_features_resident; }
+int64_t syg_debug_last_feature_frames(void) { return g_last_feature_frames; }
 int syg_debug_last_mel_form(void) { return g_last_mel_form; }
 void syg_debug_set_resident_min_groups(int n) { g_resident_min_groups = n; }
 

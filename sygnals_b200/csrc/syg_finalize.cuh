@@ -18,13 +18,18 @@ namespace sygdev {
 // Persistent: the chunk's frames are one flat sequence cut into tiles of kFinTT consecutive frames (a tile may straddle units:
 // every slot carries its own unit, reference level and clamps), CTAs stride over the tiles.  Short units (T = 101 in the
 // speech-commands shape) no longer leave partial tiles or one tiny CTA per 32 frames.
-template <int kFinTT>
+// KT = kFinTT | kFinRagged: ragged launch (a.ragged_ut), the chunk's a.n_frames frames, row r of frame gf at
+// out[r * ragged_stride + gf]
+constexpr int kFinRagged = 1 << 16;
+template <int KT>
 __global__ void __launch_bounds__(kThreads) finalize_kernel_t(const syg::FinalizeArgs a) {
+    constexpr int kFinTT = KT & (kFinRagged - 1);
+    constexpr bool RAG = (KT & kFinRagged) != 0;
     SYG_DYN_SMEM(smem_raw);
     __shared__ long long s_out[kFinTT];         // offset of (unit, row 0, frame t) in `out`
     __shared__ float s_ref[kFinTT], s_floor[kFinTT], s_pfloor[kFinTT], s_vfloor[kFinTT];
     const int tid = threadIdx.x;
-    const long long total = a.n_units * (long long)a.T;
+    const long long total = RAG ? a.n_frames : a.n_units * (long long)a.T;
     const long long n_tiles = (total + kFinTT - 1) / kFinTT;
     const int N = a.n_mels;
     const int H = a.dct_fold ? (N + 1) / 2 : N;
@@ -43,10 +48,10 @@ __global__ void __launch_bounds__(kThreads) finalize_kernel_t(const syg::Finaliz
         const int nt = (int)min((long long)kFinTT, total - gf0);
         if (tid < nt) {
             const long long gf = gf0 + tid;
-            const long long u = gf / a.T;
-            const int t = (int)(gf - u * a.T);
+            const long long u = RAG ? (long long)__ldg(a.ragged_ut + gf).x : gf / a.T;
+            const int t = RAG ? 0 : (int)(gf - u * a.T);
             const unsigned* um = a.unit_max + u * 4;
-            s_out[tid] = u * (long long)a.n_rows * a.T + t;
+            s_out[tid] = RAG ? gf : u * (long long)a.n_rows * a.T + t;
             // power_to_db(ref=np.max): the maximum of S_db over the unit is attained at the maximum energy -> 0 dB
             const float ref_db = db10(fmaxf(a.amin, __uint_as_float(um[0])));
             s_ref[tid] = ref_db;
@@ -132,8 +137,8 @@ __global__ void __launch_bounds__(kThreads) finalize_kernel_t(const syg::Finaliz
                     // lane holds D[row g][cols 2q, 2q+1] = coefficient par + 2 (m0 + g) of frames nt8 + 2q, nt8 + 2q + 1
                     if (a_ok) {
                         const int t0 = nt8 + 2 * q;
-                        if (t0 < nt) a.out[s_out[t0] + (long long)(a.row_mfcc + c_a) * a.T] = (float)d0;
-                        if (t0 + 1 < nt) a.out[s_out[t0 + 1] + (long long)(a.row_mfcc + c_a) * a.T] = (float)d1;
+                        if (t0 < nt) a.out[s_out[t0] + (long long)(a.row_mfcc + c_a) * (RAG ? a.ragged_stride : a.T)] = (float)d0;
+                        if (t0 + 1 < nt) a.out[s_out[t0 + 1] + (long long)(a.row_mfcc + c_a) * (RAG ? a.ragged_stride : a.T)] = (float)d1;
                     }
                 }
             }
@@ -145,7 +150,7 @@ __global__ void __launch_bounds__(kThreads) finalize_kernel_t(const syg::Finaliz
                     const float* c = a.cws + (gf0 + tt) * (2 * a.nb);
                     const float pdb = fmaxf(db10(fmaxf(a.amin, c[bd])), s_pfloor[tt]);
                     const float vdb = fmaxf(db10(fmaxf(a.amin, c[a.nb + bd])), s_vfloor[tt]);
-                    a.out[s_out[tt] + (long long)(a.row_contrast + bd) * a.T] = pdb - vdb;
+                    a.out[s_out[tt] + (long long)(a.row_contrast + bd) * (RAG ? a.ragged_stride : a.T)] = pdb - vdb;
                 }
             }
         }

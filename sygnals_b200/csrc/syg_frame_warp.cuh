@@ -138,6 +138,9 @@ SYG_DEVICE SYG_INLINE double lanes_scan_incl(double v, int gl) {
 //          in shared words, and after the group's last frame the CTA applies power_to_db(ref = unit max, top_db) and the DCT (FP64
 //          DMMA, the code of finalize_kernel) in place and writes the MFCC rows: no mel workspace round trip through HBM, no
 //          finalize launch.  Two CTAs per SM alternate between their transform and their epilogue phases.
+// STAGE 6: STAGE 0 for ragged units (FrameArgs::ragged_ut): every frame looks its unit and frame index up in the per-frame table,
+//          rows go to out[r * ragged_stride + gf].  The row stores spell the stride out at every site: a hoisted
+//          64-bit stride changes the register allocation of the uniform instantiations.
 // (A two-launch variant -- FFT kernel + 64-register epilogue kernel with the spectra handed over through a workspace -- was
 // measured and removed: +4 % at best, see DESIGN.md 4.1 and profiles/r01_t_two_stage_ncu_summary.txt.  CTA barriers between
 // the phases of the fused kernel were measured too: +8 % time.)
@@ -154,7 +157,8 @@ __global__ void __launch_bounds__(NT, MINB) frame_warp_kernel(const syg::FrameAr
     const int row_rms = kLay ? SP::row_rms : a.row_rms, row_crest = kLay ? SP::row_crest : a.row_crest, row_peak = kLay ? SP::row_peak : a.row_peak;
     const int row_centroid = kLay ? SP::row_centroid : a.row_centroid, row_rolloff = kLay ? SP::row_rolloff : a.row_rolloff;
     // feature stages: pass 2 produces Z/2 (halved twiddle table, element 0 entering with the pending scale 0.5) and the split runs in tangent form (split_power_h)
-    constexpr bool kHalfZ = (STAGE == 0 || STAGE == 5) && (SYG_SPLIT_HALF != 0);
+    constexpr bool kHalfZ = (STAGE == 0 || STAGE == 5 || STAGE == 6) && (SYG_SPLIT_HALF != 0);
+    constexpr bool RAG = (STAGE == 6);
     SYG_DYN_SMEM(smem_raw);
     const int tid = threadIdx.x;
     const int warp = tid >> 5, lane = tid & 31;
@@ -185,7 +189,7 @@ __global__ void __launch_bounds__(NT, MINB) frame_warp_kernel(const syg::FrameAr
     // warps' regions -- 116 table loads per lane and frame become LDS with no L1 tag traffic and no misses
     // STAGE 4 keeps window / twiddles / (full-scale) split twiddles there too, behind the per-warp tile blocks: its L1 pipe is the
     // busiest unit (95 %) and 40 of its 56 loads per lane and task were table reads through the L1 tag stage
-    constexpr bool TBL = (STAGE == 0 || STAGE == 4 || STAGE == 5);
+    constexpr bool TBL = (STAGE == 0 || STAGE == 4 || STAGE == 5 || STAGE == 6);
     unsigned char* const tb = smem_raw + ((size_t)WT::kWarps * WF + (STAGE == 4 ? (size_t)WT::kWarps * WB4 : 0)) * sizeof(float);
     const float2* const t_win = TBL ? reinterpret_cast<const float2*>(tb) : reinterpret_cast<const float2*>(a.window);
     const float2* const t_tw = TBL ? reinterpret_cast<const float2*>(tb + WT::kWinB) : a.tw;
@@ -208,7 +212,7 @@ __global__ void __launch_bounds__(NT, MINB) frame_warp_kernel(const syg::FrameAr
             if (kHalfZ) d_twsh[i] = split_twiddle_h(__ldg(a.tws + i), 4 * i < M);
             else d_twsh[i] = __ldg((STAGE == 4 ? a.tws : a.twsh) + i);
         }
-        if ((STAGE == 0 || STAGE == 5) && (mask & syg::FB_MFCC)) {
+        if ((STAGE == 0 || STAGE == 5 || STAGE == 6) && (mask & syg::FB_MFCC)) {
             int4* d_sl = const_cast<int4*>(t_slots);
             for (int i = tid; i < a.n_mels; i += NT) d_sl[i] = __ldg(a.mel_slots + i);
             float4* d_mw = const_cast<float4*>(t_melw);
@@ -232,8 +236,8 @@ __global__ void __launch_bounds__(NT, MINB) frame_warp_kernel(const syg::FrameAr
     // STAGE 4 walks "super tasks" of 8 consecutive frames (SUBS tasks each) per warp: small steps of FW frames inside one, a
     // large step to the warp's next super task
     const long long stride_frames = (STAGE == 4) ? (stride_tasks - 1) * TT4 + FW : stride_tasks * FW;
-    const long long du = stride_frames / a.T;
-    const int dt = (int)(stride_frames - du * a.T);
+    const long long du = RAG ? 0 : stride_frames / a.T;
+    const int dt = RAG ? 0 : (int)(stride_frames - du * a.T);
     // STAGE 5: outer loop over this CTA's unit groups (every other stage: one pass)
     const long long n_groups = RES ? (a.g.n_units + a.res_units - 1) / a.res_units : 1;
     for (long long grp = RES ? blockIdx.x : 0; grp < n_groups; grp += RES ? gridDim.x : 1) {
@@ -246,8 +250,10 @@ __global__ void __launch_bounds__(NT, MINB) frame_warp_kernel(const syg::FrameAr
     }
     long long gf_run = RES ? grp_f0 + (long long)warp * FW + f
                            : ((long long)blockIdx.x * WT::kWarps + warp) * ((STAGE == 4) ? TT4 : FW) + f;
-    long long u_run = gf_run / a.T;
-    int t_run = (int)(gf_run - u_run * a.T);
+    long long u_run = RAG ? 0 : gf_run / a.T;
+    int t_run = RAG ? 0 : (int)(gf_run - u_run * a.T);
+    // STAGE 6: the table entry of this lane's next frame is loaded one task ahead (its latency hides behind the current task)
+    int4 rnext = (RAG && gf_run < frame_end) ? __ldg(a.ragged_ut + gf_run) : make_int4(0, 0, 0, 0);
     const long long task_begin = (STAGE == 4) ? ((long long)blockIdx.x * WT::kWarps + warp) * SUBS : (RES ? 0 : (long long)blockIdx.x * WT::kWarps);
     const long long task_end = (STAGE == 4) ? ((a.n_frames + TT4 - 1) / TT4) * SUBS : (RES ? (frame_end - grp_f0 + FW - 1) / FW : n_tasks);
     // STAGE 0 / 3 / 5: all warps of the CTA run the same number of iterations (tasks past the end are processed as empty frames)
@@ -260,11 +266,12 @@ __global__ void __launch_bounds__(NT, MINB) frame_warp_kernel(const syg::FrameAr
         const long long gf = gf_run;
         // one frame per warp and no barrier inside the task (feature stage): a task past the end is simply skipped, and `valid` is a
         // compile-time true for everything below (no predicates on the feature stores, no branches around the workspace rows)
-        constexpr bool kSkipInvalid = (STAGE == 0 && FW == 1);
+        constexpr bool kSkipInvalid = ((STAGE == 0 || STAGE == 6) && FW == 1);
         const bool valid_rt = gf < frame_end;
         const bool valid = kSkipInvalid ? true : valid_rt;
-        const long long u = (kSkipInvalid || valid) ? u_run : 0;
-        const int t = (kSkipInvalid || valid) ? t_run : 0;
+        const int4 rut = rnext;
+        const long long u = RAG ? (long long)rut.x : ((kSkipInvalid || valid) ? u_run : 0);
+        const int t = RAG ? rut.y : ((kSkipInvalid || valid) ? t_run : 0);
         if (STAGE == 4 && ((task0 + 1) & (SUBS - 1)) != 0) {          // next task of the same super task: FW frames on
             gf_run += FW;
             t_run += FW;
@@ -273,13 +280,14 @@ __global__ void __launch_bounds__(NT, MINB) frame_warp_kernel(const syg::FrameAr
             u_run += du;
             t_run += dt;
         }
-        while (t_run >= a.T) { t_run -= a.T; ++u_run; }
+        if (!RAG) while (t_run >= a.T) { t_run -= a.T; ++u_run; }
+        if (RAG) rnext = gf_run < frame_end ? __ldg(a.ragged_ut + gf_run) : make_int4(0, 0, 0, 0);
         if (kSkipInvalid && !valid_rt) continue;
-        UnitRef ur = unit_ref(a.g, u);
+        UnitRef ur = RAG ? UnitRef{(long long)rut.w, (long long)rut.z} : unit_ref(a.g, u);
         if (!valid) ur.valid = 0;
         const long long p0 = (long long)t * a.hop - a.cpad;
 
-        float* const orow = a.out + (long long)u * a.n_rows * a.T + t;
+        float* const orow = RAG ? a.out + gf : a.out + (long long)u * a.n_rows * a.T + t;
         // ---------------- framing + window + time-domain partial statistics ----------------
         float2 z[E];
         float2 sq2 = make_float2(0.0f, 0.0f);
@@ -507,22 +515,22 @@ __global__ void __launch_bounds__(NT, MINB) frame_warp_kernel(const syg::FrameAr
             const float tpk = lanes_max<G>(pk);
             if (j == 0 && valid) {
                 const float rms = sqrt_approx(tsq * (1.0f / (float)TL::NFFT));     // MUFU.SQRT (1 ulp) instead of the IEEE sequence; bar: rel 1e-5
-                if (row_rms >= 0) orow[(long long)row_rms * a.T] = rms;
+                if (row_rms >= 0) orow[(long long)row_rms * (RAG ? a.ragged_stride : a.T)] = rms;
                 // eps(float64) = 2^-52 is a float too: the reference's `rms < eps` on the widened value is this float comparison
-                if (row_crest >= 0) orow[(long long)row_crest * a.T] = (rms < 2.220446049250313e-16f) ? 0.0f : __fdividef(tpk, rms);
-                if (row_peak >= 0) orow[(long long)row_peak * a.T] = tpk;
+                if (row_crest >= 0) orow[(long long)row_crest * (RAG ? a.ragged_stride : a.T)] = (rms < 2.220446049250313e-16f) ? 0.0f : __fdividef(tpk, rms);
+                if (row_peak >= 0) orow[(long long)row_peak * (RAG ? a.ragged_stride : a.T)] = tpk;
             }
             if (EXTRA) {
                 if (mask & (syg::FB_STD_AMP | syg::FB_MEAN_AMP)) {
                     const double tsum = lanes_sum<G>(s_sum), tabs = lanes_sum<G>(s_abs), tsqd = lanes_sum<G>(s_sqd);
                     if (j == 0 && valid) {
                         const double n = (double)TL::NFFT;
-                        if (a.row_mean_amp >= 0) orow[(long long)a.row_mean_amp * a.T] = (float)(tabs / n);
+                        if (a.row_mean_amp >= 0) orow[(long long)a.row_mean_amp * (RAG ? a.ragged_stride : a.T)] = (float)(tabs / n);
                         if (a.row_std_amp >= 0) {
                             const double mu = tsum / n;
                             double var = tsqd / n - mu * mu;
                             if (var < 0.0) var = 0.0;
-                            orow[(long long)a.row_std_amp * a.T] = (float)sqrt(var);
+                            orow[(long long)a.row_std_amp * (RAG ? a.ragged_stride : a.T)] = (float)sqrt(var);
                         }
                     }
                 }
@@ -584,11 +592,11 @@ __global__ void __launch_bounds__(NT, MINB) frame_warp_kernel(const syg::FrameAr
             double centroid_hz = 0.0;
             if constexpr (EXTRA) {                                       // spectral_bandwidth needs the float64 centroid
                 if ((double)tm >= kEps64) centroid_hz = a.bin_hz * ((double)tkm / (double)tm);
-                if (row_centroid >= 0 && j == 0 && valid) orow[(long long)row_centroid * a.T] = (float)centroid_hz;
+                if (row_centroid >= 0 && j == 0 && valid) orow[(long long)row_centroid * (RAG ? a.ragged_stride : a.T)] = (float)centroid_hz;
             } else {
                 // the sums are FP32 already; one FP32 division (2^-23 relative against a 1e-5 parity bar) instead of a float64 one
                 const float c = (tm >= 2.220446049250313e-16f) ? (float)a.bin_hz * __fdividef(tkm, tm) : 0.0f;
-                if (row_centroid >= 0 && j == 0 && valid) orow[(long long)row_centroid * a.T] = c;
+                if (row_centroid >= 0 && j == 0 && valid) orow[(long long)row_centroid * (RAG ? a.ragged_stride : a.T)] = c;
             }
             if (row_rolloff >= 0) {
                 // first bin whose cumulative power reaches roll_percent * total (frequency_domain.py:334-346)
@@ -629,7 +637,7 @@ __global__ void __launch_bounds__(NT, MINB) frame_warp_kernel(const syg::FrameAr
                     if (total_p < kEps64) bin = M;                                      // silent frame -> freqs[-1]
                     else if (found) bin = kL + posw;
                     else bin = (L == G - 1) ? M : kL + E - 1;                           // only the lane's last element is left
-                    orow[(long long)row_rolloff * a.T] = (float)(a.bin_hz * (double)bin);
+                    orow[(long long)row_rolloff * (RAG ? a.ragged_stride : a.T)] = (float)(a.bin_hz * (double)bin);
                 }
             }
             if (EXTRA) {
@@ -642,7 +650,7 @@ __global__ void __launch_bounds__(NT, MINB) frame_warp_kernel(const syg::FrameAr
                             fl = exp((double)tl / (double)B) / am;
                             fl = fl < 0.0 ? 0.0 : (fl > 1.0 ? 1.0 : fl);
                         }
-                        orow[(long long)a.row_flatness * a.T] = (float)fl;
+                        orow[(long long)a.row_flatness * (RAG ? a.ragged_stride : a.T)] = (float)fl;
                     }
                 }
                 if (a.row_bandwidth >= 0) {
@@ -658,13 +666,13 @@ __global__ void __launch_bounds__(NT, MINB) frame_warp_kernel(const syg::FrameAr
                         sb += (double)sqrtf(p_ny) * d * d;
                     }
                     const double tb = lanes_sum<G>(sb);
-                    if (j == 0 && valid) orow[(long long)a.row_bandwidth * a.T] = ((double)tm < kEps64) ? 0.0f : (float)sqrt(tb / (double)tm);
+                    if (j == 0 && valid) orow[(long long)a.row_bandwidth * (RAG ? a.ragged_stride : a.T)] = ((double)tm < kEps64) ? 0.0f : (float)sqrt(tb / (double)tm);
                 }
                 if (a.row_dominant >= 0) {
                     const float gmax = lanes_max<G>(vmax);
                     float mi = (vmax == gmax) ? -(float)imax : -1.0e9f;
                     mi = lanes_max<G>(mi);
-                    if (j == 0 && valid) orow[(long long)a.row_dominant * a.T] = (float)(a.bin_hz * (double)(-mi));
+                    if (j == 0 && valid) orow[(long long)a.row_dominant * (RAG ? a.ragged_stride : a.T)] = (float)(a.bin_hz * (double)(-mi));
                 }
             }
         }

@@ -97,17 +97,19 @@ __global__ void __launch_bounds__(kThreads) frame_kernel(const syg::FrameArgs a)
     const int warp = tid >> 5, lane = tid & 31;
     const long long n_rounds = (a.n_frames + F - 1) / F;
     const int B = M + 1;
+    constexpr bool RAG = (MODE == MODE_FEATURES_RAGGED);
 
     for (long long round = blockIdx.x; round < n_rounds; round += gridDim.x) {
         const long long gf = round * F + f;
         const bool valid = gf < a.n_frames;
-        const long long u = valid ? gf / a.T : 0;
-        const int t = valid ? (int)(gf - u * a.T) : 0;
-        UnitRef ur = unit_ref(a.g, u);
+        const int4 rut = (RAG && valid) ? __ldg(a.ragged_ut + gf) : make_int4(0, 0, 0, 0);
+        const long long u = RAG ? (long long)rut.x : (valid ? gf / a.T : 0);
+        const int t = RAG ? rut.y : (valid ? (int)(gf - u * a.T) : 0);
+        UnitRef ur = RAG ? UnitRef{(long long)rut.w, (long long)rut.z} : unit_ref(a.g, u);
         if (!valid) ur.valid = 0;
         const long long p0 = (long long)t * a.hop - a.cpad;
 
-        if (MODE == MODE_FEATURES) {
+        if (MODE != MODE_STFT) {
             for (int i = tid; i < F * 4; i += kThreads) smax[i] = 0u;
         }
 
@@ -120,7 +122,7 @@ __global__ void __launch_bounds__(kThreads) frame_kernel(const syg::FrameArgs a)
             const int c = j + r * G;
             const float2 v = load_pair(a.y, ur, p0 + 2 * c, a.pad_mode);
             const float2 w = __ldg(reinterpret_cast<const float2*>(a.window) + c);
-            if (MODE == MODE_FEATURES) {
+            if (MODE != MODE_STFT) {
                 s_sq += (double)v.x * (double)v.x + (double)v.y * (double)v.y;
                 s_sum += (double)v.x + (double)v.y;
                 s_abs += (double)fabsf(v.x) + (double)fabsf(v.y);
@@ -148,7 +150,7 @@ __global__ void __launch_bounds__(kThreads) frame_kernel(const syg::FrameArgs a)
                 float xkr, xki, xmr, xmi;
                 real_split(zkr, zki, zmr, zmi, w.x, w.y, xkr, xki, xmr, xmi);
                 const int k2 = M - k;                      // k = 0 -> bin M (Nyquist); k = M/2 -> itself
-                if (MODE == MODE_FEATURES) {
+                if (MODE != MODE_STFT) {
                     SST(&pw[f * PW + padi(k)], __fmaf_rn(xkr, xkr, xki * xki));
                     if (k2 != k) SST(&pw[f * PW + padi(k2)], __fmaf_rn(xmr, xmr, xmi * xmi));
                 } else if (valid) {
@@ -172,7 +174,7 @@ __global__ void __launch_bounds__(kThreads) frame_kernel(const syg::FrameArgs a)
         }
         __syncthreads();
 
-        float* const orow = a.out + (long long)u * a.n_rows * a.T + t;
+        float* const orow = RAG ? a.out + gf : a.out + (long long)u * a.n_rows * a.T + t;
 
         // ---------------- time-domain features (unwindowed, zero-padded frame) ----------------
         if (a.mask & syg::FB_TIME_ANY) {
@@ -186,15 +188,15 @@ __global__ void __launch_bounds__(kThreads) frame_kernel(const syg::FrameArgs a)
             if (j == 0 && valid) {
                 const double n = (double)TL::NFFT;
                 const double rms = sqrt(tsq / n);
-                if (a.row_rms >= 0) orow[(long long)a.row_rms * a.T] = (float)rms;
-                if (a.row_crest >= 0) orow[(long long)a.row_crest * a.T] = (rms < kEps64) ? 0.0f : (float)((double)tpk / rms);
-                if (a.row_peak >= 0) orow[(long long)a.row_peak * a.T] = tpk;
-                if (a.row_mean_amp >= 0) orow[(long long)a.row_mean_amp * a.T] = (float)(tabs / n);
+                if (a.row_rms >= 0) orow[(long long)a.row_rms * (RAG ? a.ragged_stride : a.T)] = (float)rms;
+                if (a.row_crest >= 0) orow[(long long)a.row_crest * (RAG ? a.ragged_stride : a.T)] = (rms < kEps64) ? 0.0f : (float)((double)tpk / rms);
+                if (a.row_peak >= 0) orow[(long long)a.row_peak * (RAG ? a.ragged_stride : a.T)] = tpk;
+                if (a.row_mean_amp >= 0) orow[(long long)a.row_mean_amp * (RAG ? a.ragged_stride : a.T)] = (float)(tabs / n);
                 if (a.row_std_amp >= 0) {
                     const double mu = tsum / n;
                     double var = tsq / n - mu * mu;
                     if (var < 0.0) var = 0.0;
-                    orow[(long long)a.row_std_amp * a.T] = (float)sqrt(var);
+                    orow[(long long)a.row_std_amp * (RAG ? a.ragged_stride : a.T)] = (float)sqrt(var);
                 }
             }
         }
@@ -227,10 +229,10 @@ __global__ void __launch_bounds__(kThreads) frame_kernel(const syg::FrameArgs a)
             const double tkm = group_sum<G>(skm, dsc);
             double centroid_hz = 0.0;
             if (tm >= kEps64) centroid_hz = a.bin_hz * (tkm / tm);
-            if (a.row_centroid >= 0 && j == 0 && valid) orow[(long long)a.row_centroid * a.T] = (float)centroid_hz;
+            if (a.row_centroid >= 0 && j == 0 && valid) orow[(long long)a.row_centroid * (RAG ? a.ragged_stride : a.T)] = (float)centroid_hz;
             if (a.row_rolloff >= 0) {
                 if (total_p < kEps64) {
-                    if (j == 0 && valid) orow[(long long)a.row_rolloff * a.T] = (float)(a.bin_hz * (double)M);
+                    if (j == 0 && valid) orow[(long long)a.row_rolloff * (RAG ? a.ragged_stride : a.T)] = (float)(a.bin_hz * (double)M);
                 } else {
                     const double thr = a.roll_percent * total_p;
                     if (incl >= thr && prev < thr) {           // exactly one thread of the group
@@ -240,7 +242,7 @@ __global__ void __launch_bounds__(kThreads) frame_kernel(const syg::FrameArgs a)
                             c += (double)SLD(&pf[padi(k0 + i)]);
                             if (c >= thr) { bin = k0 + i; break; }
                         }
-                        if (valid) orow[(long long)a.row_rolloff * a.T] = (float)(a.bin_hz * (double)bin);
+                        if (valid) orow[(long long)a.row_rolloff * (RAG ? a.ragged_stride : a.T)] = (float)(a.bin_hz * (double)bin);
                     }
                 }
             }
@@ -253,7 +255,7 @@ __global__ void __launch_bounds__(kThreads) frame_kernel(const syg::FrameArgs a)
                         fl = exp(tl / (double)B) / am;
                         fl = fl < 0.0 ? 0.0 : (fl > 1.0 ? 1.0 : fl);
                     }
-                    orow[(long long)a.row_flatness * a.T] = (float)fl;
+                    orow[(long long)a.row_flatness * (RAG ? a.ragged_stride : a.T)] = (float)fl;
                 }
             }
             if (a.row_bandwidth >= 0) {
@@ -264,14 +266,14 @@ __global__ void __launch_bounds__(kThreads) frame_kernel(const syg::FrameArgs a)
                     sb += mg * d * d;
                 }
                 const double tb = group_sum<G>(sb, dsc);
-                if (j == 0 && valid) orow[(long long)a.row_bandwidth * a.T] = (tm < kEps64) ? 0.0f : (float)sqrt(tb / tm);
+                if (j == 0 && valid) orow[(long long)a.row_bandwidth * (RAG ? a.ragged_stride : a.T)] = (tm < kEps64) ? 0.0f : (float)sqrt(tb / tm);
             }
             if (a.row_dominant >= 0) {
                 // np.argmax: first bin attaining the maximum = smallest index among the threads holding it
                 const float gmax = group_max<G>(vmax, dsc);
                 float mi = (vmax == gmax) ? -(float)imax : -1.0e9f;
                 mi = group_max<G>(mi, dsc);
-                if (j == 0 && valid) orow[(long long)a.row_dominant * a.T] = (float)(a.bin_hz * (double)(-mi));
+                if (j == 0 && valid) orow[(long long)a.row_dominant * (RAG ? a.ragged_stride : a.T)] = (float)(a.bin_hz * (double)(-mi));
             }
         }
 
@@ -336,7 +338,7 @@ __global__ void __launch_bounds__(kThreads) frame_kernel(const syg::FrameArgs a)
                 const long long gff = round * F + ff;
                 if (slot < 3 && gff < a.n_frames) {
                     const unsigned v = smax[i];
-                    if (v) atomicMax(&a.unit_max[(gff / a.T) * 4 + slot], v);
+                    if (v) atomicMax(&a.unit_max[(RAG ? (long long)__ldg(a.ragged_ut + gff).x : gff / a.T) * 4 + slot], v);
                 }
             }
         }

@@ -16,6 +16,12 @@ int stft_big(int n_fft, const syg::FrameArgs& a, int sm_count, cudaStream_t st, 
 // unit-resident feature kernel (short units, MFCC epilogue on chip): units per CTA group for this plan (0 = not eligible), launch
 int frame_warp_res_units(int n_fft, const syg::FrameArgs& a);
 int frame_warp_res(int n_fft, const syg::FrameArgs& a, int sm_count, cudaStream_t st, std::string& err);
+// ragged launches (FrameArgs::ragged_ut, syg_launch_ragged.cu): the per-frame table {unit, frame in unit, length, start} from frame
+// offsets frame_off[n_units + 1] and the unit tables (starts < 2^31: relative to the chunk's samples), and the warp feature kernel
+// (STAGE 6).  frame_block / frame_mixed / time_extra / finalize take MODE_FEATURES_RAGGED / ragged_ut themselves.
+int ragged_frame_table(const long long* frame_off, const long long* starts, const int* valid, long long n_units, long long n_frames,
+                       int4* ut, int sm_count, cudaStream_t st, std::string& err);
+int frame_warp_ragged(int n_fft, bool extra, const syg::FrameArgs& a, int sm_count, cudaStream_t st, std::string& err);
 int frame_warp_stft(int n_fft, const syg::FrameArgs& a, int sm_count, cudaStream_t st, std::string& err);
 int finalize(const syg::FinalizeArgs& a, int tt, unsigned grid_x, unsigned grid_y, size_t smem, cudaStream_t st, std::string& err);
 int aggregate(const float* feats, long long n_seg, int n_rows, long long row_stride, const long long* seg_off, const int* seg_len,

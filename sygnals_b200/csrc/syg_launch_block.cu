@@ -58,6 +58,11 @@ int frame_block(int n_fft, int mode, const syg::FrameArgs& a, int sm_count, cuda
             case 11: return frame_block_t<FftTile<11, 16>, MODE_STFT>(a, sm_count, st, err);
             case 12: return frame_block_t<FftTile<12, 16>, MODE_STFT>(a, sm_count, st, err);
         }
+    } else if (mode == MODE_FEATURES_RAGGED) {
+        switch (l) {
+            case 11: return frame_block_t<FftTile<11, 16>, MODE_FEATURES_RAGGED>(a, sm_count, st, err);
+            case 12: return frame_block_t<FftTile<12, 16>, MODE_FEATURES_RAGGED>(a, sm_count, st, err);
+        }
     } else {
         switch (l) {
             case 11: return frame_block_t<FftTile<11, 16>, MODE_FEATURES>(a, sm_count, st, err);
@@ -68,9 +73,9 @@ int frame_block(int n_fft, int mode, const syg::FrameArgs& a, int sm_count, cuda
     return -5;
 }
 
-template <int TT>
+template <int TT, bool RAG>
 static int finalize_t(const syg::FinalizeArgs& a, unsigned grid_x, unsigned grid_y, size_t smem, cudaStream_t st, std::string& err) {
-    auto kfn = sygdev::finalize_kernel_t<TT>;
+    auto kfn = sygdev::finalize_kernel_t<RAG ? (TT | sygdev::kFinRagged) : TT>;
     if (smem > 48 * 1024) {                         // the S_db tile exceeds the default 48 KB for wide mel banks
         static KernelCache kc;
         int nb = 0;
@@ -83,7 +88,10 @@ static int finalize_t(const syg::FinalizeArgs& a, unsigned grid_x, unsigned grid
 
 // tt = frames per CTA tile: 32 (default) or 64 (narrow mel banks: the CTA is latency bound, twice the frames amortise it)
 int finalize(const syg::FinalizeArgs& a, int tt, unsigned grid_x, unsigned grid_y, size_t smem, cudaStream_t st, std::string& err) {
-    return tt == 64 ? finalize_t<64>(a, grid_x, grid_y, smem, st, err) : finalize_t<32>(a, grid_x, grid_y, smem, st, err);
+    if (grid_x == 0 || grid_y == 0) return 0;        // no frames: a launch of zero CTAs would fail with an invalid configuration
+    if (a.ragged_ut)
+        return tt == 64 ? finalize_t<64, true>(a, grid_x, grid_y, smem, st, err) : finalize_t<32, true>(a, grid_x, grid_y, smem, st, err);
+    return tt == 64 ? finalize_t<64, false>(a, grid_x, grid_y, smem, st, err) : finalize_t<32, false>(a, grid_x, grid_y, smem, st, err);
 }
 
 }  // namespace syglaunch

@@ -10,7 +10,7 @@ static int mixed_threads(int L) { return L <= 256 ? 64 : (L <= 1024 ? 128 : 256)
 template <int MODE, int NT>
 static int frame_mixed_t(const syg::FrameArgs& a, const syg::MixedPlan& mp, int sm_count, cudaStream_t st, std::string& err) {
     auto kfn = sygdev::frame_mixed_kernel<MODE, NT>;
-    const size_t smem = sygdev::mixed_layout(mp.L, mp.B, MODE == sygdev::MODE_FEATURES, NT).bytes;
+    const size_t smem = sygdev::mixed_layout(mp.L, mp.B, MODE != sygdev::MODE_STFT, NT).bytes;
     static KernelCache kc;
     int blocks_per_sm = 0;
     if (int rc = prepare_kernel(kfn, NT, smem, kc, &blocks_per_sm, err)) return rc;
@@ -31,6 +31,7 @@ static int frame_mixed_m(const syg::FrameArgs& a, const syg::MixedPlan& mp, int 
 }
 
 int frame_mixed(int mode, const syg::FrameArgs& a, const syg::MixedPlan& mp, int sm_count, cudaStream_t st, std::string& err) {
+    if (mode == sygdev::MODE_FEATURES_RAGGED) return frame_mixed_m<sygdev::MODE_FEATURES_RAGGED>(a, mp, sm_count, st, err);
     return mode == sygdev::MODE_STFT ? frame_mixed_m<sygdev::MODE_STFT>(a, mp, sm_count, st, err)
                                      : frame_mixed_m<sygdev::MODE_FEATURES>(a, mp, sm_count, st, err);
 }

@@ -17,22 +17,26 @@ SYG_DEVICE SYG_INLINE double wsum_d(double v) {
     return v;
 }
 
-__global__ void __launch_bounds__(kThreads) time_extra_kernel(const syg::FrameArgs a, const int fl, const int entropy_bins) {
+// RAG: ragged launch (a.ragged_ut): the unit and frame index come from the per-frame table, a unit is its own valid samples, rows go
+// to [n_rows][n_frames]
+template <bool RAG>
+SYG_DEVICE SYG_INLINE void time_extra_body(const syg::FrameArgs& a, const int fl, const int entropy_bins) {
     const int lane = threadIdx.x & 31;
     const long long warps = (long long)gridDim.x * (kThreads / 32);
     const double n = (double)fl;
     for (long long gf = (long long)blockIdx.x * (kThreads / 32) + (threadIdx.x >> 5); gf < a.n_frames; gf += warps) {
-        const long long u = gf / a.T;
-        const int t = (int)(gf - u * a.T);
-        const UnitRef ur = unit_ref(a.g, u);
+        const int4 rut = RAG ? __ldg(a.ragged_ut + gf) : make_int4(0, 0, 0, 0);
+        const long long u = RAG ? (long long)rut.x : gf / a.T;
+        const int t = RAG ? rut.y : (int)(gf - u * a.T);
+        const UnitRef ur = RAG ? UnitRef{(long long)rut.w, (long long)rut.z} : unit_ref(a.g, u);
         const float* yb = a.y + ur.start;
         const long long p0 = (long long)t * a.hop - a.cpad;
-        float* const orow = a.out + (long long)u * a.n_rows * a.T + t;
+        float* const orow = RAG ? a.out + gf : a.out + (long long)u * a.n_rows * a.T + t;
         // ---- pass 1: sum, extremes of the zero-padded frame; zero crossings of the edge-padded frame
         double s1 = 0.0;
         float mn = __uint_as_float(0x7f800000u), mx = __uint_as_float(0xff800000u);
         int zc = 0;
-        const long long L = a.g.unit_len;
+        const long long L = RAG ? ur.valid : a.g.unit_len;
         for (int i = lane; i < fl; i += 32) {
             const long long pos = p0 + i;
             const float x = (pos >= 0 && pos < ur.valid) ? __ldg(yb + pos) : 0.0f;
@@ -55,7 +59,7 @@ __global__ void __launch_bounds__(kThreads) time_extra_kernel(const syg::FrameAr
             mn = fminf(mn, __shfl_xor_sync(kFull, mn, o));
             mx = fmaxf(mx, __shfl_xor_sync(kFull, mx, o));
         }
-        if (lane == 0 && a.row_zcr >= 0) orow[(long long)a.row_zcr * a.T] = (float)((double)zc / n);
+        if (lane == 0 && a.row_zcr >= 0) orow[(long long)a.row_zcr * (RAG ? a.ragged_stride : a.T)] = (float)((double)zc / n);
         const bool need_mom = a.row_skew >= 0 || a.row_kurt >= 0;
         const bool need_ent = a.row_entropy >= 0;
         if (!need_mom && !need_ent) continue;
@@ -96,12 +100,12 @@ __global__ void __launch_bounds__(kThreads) time_extra_kernel(const syg::FrameAr
                 if (a.row_skew >= 0) {
                     double v = 0.0;
                     if (!flat && fl >= 3) v = sqrt((n - 1.0) * n) / (n - 2.0) * m3 / pow(m2, 1.5);
-                    orow[(long long)a.row_skew * a.T] = (float)v;
+                    orow[(long long)a.row_skew * (RAG ? a.ragged_stride : a.T)] = (float)v;
                 }
                 if (a.row_kurt >= 0) {
                     double v = 0.0;
                     if (!flat && fl >= 4) v = 1.0 / (n - 2.0) / (n - 3.0) * ((n * n - 1.0) * m4 / (m2 * m2) - 3.0 * (n - 1.0) * (n - 1.0));
-                    orow[(long long)a.row_kurt * a.T] = (float)v;
+                    orow[(long long)a.row_kurt * (RAG ? a.ragged_stride : a.T)] = (float)v;
                 }
             }
         }
@@ -120,9 +124,16 @@ __global__ void __launch_bounds__(kThreads) time_extra_kernel(const syg::FrameAr
                 }
                 ent = wsum_d(ent);
             }
-            if (lane == 0) orow[(long long)a.row_entropy * a.T] = (float)ent;
+            if (lane == 0) orow[(long long)a.row_entropy * (RAG ? a.ragged_stride : a.T)] = (float)ent;
         }
     }
+}
+
+__global__ void __launch_bounds__(kThreads) time_extra_kernel(const syg::FrameArgs a, const int fl, const int entropy_bins) {
+    time_extra_body<false>(a, fl, entropy_bins);
+}
+__global__ void __launch_bounds__(kThreads) time_extra_ragged_kernel(const syg::FrameArgs a, const int fl, const int entropy_bins) {
+    time_extra_body<true>(a, fl, entropy_bins);
 }
 
 }  // namespace sygdev
@@ -132,7 +143,8 @@ int time_extra(const syg::FrameArgs& a, int frame_length, int entropy_bins, int 
     if (a.n_frames <= 0) return 0;
     const long long want = (a.n_frames + sygdev::kThreads / 32 - 1) / (sygdev::kThreads / 32);
     const int grid = (int)std::min<long long>(want, (long long)sm_count * 8);
-    SYG_LAUNCH(sygdev::time_extra_kernel, grid, sygdev::kThreads, 0, st, a, frame_length, entropy_bins);
+    if (a.ragged_ut) SYG_LAUNCH(sygdev::time_extra_ragged_kernel, grid, sygdev::kThreads, 0, st, a, frame_length, entropy_bins);
+    else SYG_LAUNCH(sygdev::time_extra_kernel, grid, sygdev::kThreads, 0, st, a, frame_length, entropy_bins);
     LCK(cudaGetLastError());
     return 0;
 }

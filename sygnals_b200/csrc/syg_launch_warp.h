@@ -16,15 +16,19 @@ namespace syglaunch {
 int frame_warp_spec44k(const syg::FrameArgs& a, int sm_count, cudaStream_t st, std::string& err);
 int frame_warp_spec22k(const syg::FrameArgs& a, int sm_count, cudaStream_t st, std::string& err);
 int frame_warp_spec44kl(const syg::FrameArgs& a, int sm_count, cudaStream_t st, std::string& err);
+// the same three for ragged launches (STAGE 6; syg_launch_ragged_spec.cu)
+int frame_warp_spec44k_ragged(const syg::FrameArgs& a, int sm_count, cudaStream_t st, std::string& err);
+int frame_warp_spec22k_ragged(const syg::FrameArgs& a, int sm_count, cudaStream_t st, std::string& err);
+int frame_warp_spec44kl_ragged(const syg::FrameArgs& a, int sm_count, cudaStream_t st, std::string& err);
 
-// STAGE 0: features; 3: STFT output through a CTA tile; 4: STFT magnitude / power through warp-private tiles (see syg_frame_warp.cuh)
+// STAGE 0: features; 6: features of ragged units; 3: STFT output through a CTA tile; 4: STFT magnitude / power through warp-private tiles (see syg_frame_warp.cuh)
 template <class TL, bool EXTRA, int NT, int MINB, int STAGE, class SP = sygdev::SpecNone>
 static int frame_warp_t(const syg::FrameArgs& a, int sm_count, cudaStream_t st, std::string& err) {
     using WT = sygdev::WarpTile<TL, NT>;
     auto kfn = sygdev::frame_warp_kernel<TL, EXTRA, NT, MINB, STAGE, SP>;
     size_t smem = (size_t)WT::kWarps * WT::FW * WT::RS * sizeof(float);
     const int wide = (STAGE == 3 && a.out_kind == 0) ? 1 : 0;        // complex64 tile
-    if (STAGE == 0) smem += WT::table_bytes(a.n_mels, (a.mask & syg::FB_MFCC) ? a.mel_pw_f4 : 0);
+    if (STAGE == 0 || STAGE == 6) smem += WT::table_bytes(a.n_mels, (a.mask & syg::FB_MFCC) ? a.mel_pw_f4 : 0);
     if (STAGE == 3) {
         const int TT = WT::kWarps * WT::FW;
         smem += (size_t)TT * sizeof(long long) + (size_t)(WT::M + 1) * (TT + 1) * (wide ? 8 : 4);
@@ -85,16 +89,20 @@ static int frame_warp_dispatch(int n_fft, const syg::FrameArgs& a, int sm_count,
         case 10:
             if constexpr (STAGE == 4) break;
             // features: one CTA of 16 warps per SM so that the 38 KB of plan tables are held once (leaves ~50 KB of L1)
-            if constexpr (STAGE == 0 && !EXTRA) {
+            if constexpr ((STAGE == 0 || STAGE == 6) && !EXTRA) {
                 static int nospec = -1;                               // SYGB200_NO_SPEC=1: always the generic loops (A/B measurements)
                 if (nospec < 0) { const char* e = std::getenv("SYGB200_NO_SPEC"); nospec = e ? std::atoi(e) : 0; }
                 static int nolay = -1;                                // SYGB200_NO_SPECL=1: skip the layout-specialised instantiation (A/B)
                 if (nolay < 0) { const char* e = std::getenv("SYGB200_NO_SPECL"); nolay = e ? std::atoi(e) : 0; }
-                if (!nospec && !nolay && spec_matches<Spec44kL>(a)) return frame_warp_spec44kl(a, sm_count, st, err);
-                if (!nospec && spec_matches<Spec44k>(a)) return frame_warp_spec44k(a, sm_count, st, err);
-                if (!nospec && spec_matches<Spec22k>(a)) return frame_warp_spec22k(a, sm_count, st, err);
+                constexpr bool rag = (STAGE == 6);
+                if (!nospec && !nolay && spec_matches<Spec44kL>(a))
+                    return rag ? frame_warp_spec44kl_ragged(a, sm_count, st, err) : frame_warp_spec44kl(a, sm_count, st, err);
+                if (!nospec && spec_matches<Spec44k>(a))
+                    return rag ? frame_warp_spec44k_ragged(a, sm_count, st, err) : frame_warp_spec44k(a, sm_count, st, err);
+                if (!nospec && spec_matches<Spec22k>(a))
+                    return rag ? frame_warp_spec22k_ragged(a, sm_count, st, err) : frame_warp_spec22k(a, sm_count, st, err);
             }
-            if (STAGE == 0) {
+            if (STAGE == 0 || STAGE == 6) {
                 // 20 warps leave ~40 KB of shared memory for the plan tables: enough for the interval-form mel and for the tap
                 // tables of the default banks, not for the long taps of a few wide filters (n_mels 40 or fewer without the
                 // interval form, e.g. mel power != 2).  Those plans run 8 warps per CTA.

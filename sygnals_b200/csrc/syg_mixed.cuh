@@ -161,7 +161,8 @@ template <int MODE, int NT>
 __global__ void __launch_bounds__(NT) frame_mixed_kernel(const syg::FrameArgs a, const syg::MixedPlan mp) {
     SYG_DYN_SMEM(smem_raw);
     const int L = mp.L, B = mp.B, N = mp.n;
-    const MixedLayout lay = mixed_layout(L, B, MODE == MODE_FEATURES, NT);
+    const MixedLayout lay = mixed_layout(L, B, MODE != MODE_STFT, NT);
+    constexpr bool RAG = (MODE == MODE_FEATURES_RAGGED);
     float* const smf = reinterpret_cast<float*>(smem_raw);
     float2* const bufa = reinterpret_cast<float2*>(smf + lay.off_a);
     float2* const bufb = reinterpret_cast<float2*>(smf + lay.off_b);
@@ -174,11 +175,12 @@ __global__ void __launch_bounds__(NT) frame_mixed_kernel(const syg::FrameArgs a,
     const int warp = tid >> 5, lane = tid & 31;
 
     for (long long gf = blockIdx.x; gf < a.n_frames; gf += gridDim.x) {
-        const long long u = gf / a.T;
-        const int t = (int)(gf - u * a.T);
-        const UnitRef ur = unit_ref(a.g, u);
+        const int4 rut = RAG ? __ldg(a.ragged_ut + gf) : make_int4(0, 0, 0, 0);
+        const long long u = RAG ? (long long)rut.x : gf / a.T;
+        const int t = RAG ? rut.y : (int)(gf - u * a.T);
+        const UnitRef ur = RAG ? UnitRef{(long long)rut.w, (long long)rut.z} : unit_ref(a.g, u);
         const long long p0 = (long long)t * a.hop - a.cpad;
-        if (MODE == MODE_FEATURES && tid < 4) smax[tid] = 0u;
+        if (MODE != MODE_STFT && tid < 4) smax[tid] = 0u;
 
         // ---------------- framing + window + time-domain partial statistics ----------------
         double s_sq = 0.0, s_sum = 0.0, s_abs = 0.0;
@@ -187,7 +189,7 @@ __global__ void __launch_bounds__(NT) frame_mixed_kernel(const syg::FrameArgs a,
             for (int c = tid; c < L; c += NT) {
                 const float2 v = load_pair(a.y, ur, p0 + 2 * c, a.pad_mode);
                 const float2 w = __ldg(reinterpret_cast<const float2*>(a.window) + c);
-                if (MODE == MODE_FEATURES) {
+                if (MODE != MODE_STFT) {
                     s_sq += (double)v.x * (double)v.x + (double)v.y * (double)v.y;
                     s_sum += (double)v.x + (double)v.y;
                     s_abs += (double)fabsf(v.x) + (double)fabsf(v.y);
@@ -199,7 +201,7 @@ __global__ void __launch_bounds__(NT) frame_mixed_kernel(const syg::FrameArgs a,
             for (int c = tid; c < L; c += NT) {
                 const float v = load_one(a.y, ur, p0 + c, a.pad_mode);
                 const float w = __ldg(a.window + c);
-                if (MODE == MODE_FEATURES) {
+                if (MODE != MODE_STFT) {
                     s_sq += (double)v * (double)v;
                     s_sum += (double)v;
                     s_abs += (double)fabsf(v);
@@ -230,7 +232,7 @@ __global__ void __launch_bounds__(NT) frame_mixed_kernel(const syg::FrameArgs a,
         mixed_bins<NT>(z, mp, a.tws, tid, [&](int k, float re, float im) { SST(&pw[padi(k)], __fmaf_rn(re, re, im * im)); });
         __syncthreads();
 
-        float* const orow = a.out + (long long)u * a.n_rows * a.T + t;
+        float* const orow = RAG ? a.out + gf : a.out + (long long)u * a.n_rows * a.T + t;
         // ---------------- time-domain features (unwindowed, zero-padded frame) ----------------
         if (a.mask & syg::FB_TIME_ANY) {
             const double tsq = group_sum<NT>(s_sq, dsc);
@@ -243,15 +245,15 @@ __global__ void __launch_bounds__(NT) frame_mixed_kernel(const syg::FrameArgs a,
             if (tid == 0) {
                 const double n = (double)N;
                 const double rms = sqrt(tsq / n);
-                if (a.row_rms >= 0) orow[(long long)a.row_rms * a.T] = (float)rms;
-                if (a.row_crest >= 0) orow[(long long)a.row_crest * a.T] = (rms < kEps64) ? 0.0f : (float)((double)tpk / rms);
-                if (a.row_peak >= 0) orow[(long long)a.row_peak * a.T] = tpk;
-                if (a.row_mean_amp >= 0) orow[(long long)a.row_mean_amp * a.T] = (float)(tabs / n);
+                if (a.row_rms >= 0) orow[(long long)a.row_rms * (RAG ? a.ragged_stride : a.T)] = (float)rms;
+                if (a.row_crest >= 0) orow[(long long)a.row_crest * (RAG ? a.ragged_stride : a.T)] = (rms < kEps64) ? 0.0f : (float)((double)tpk / rms);
+                if (a.row_peak >= 0) orow[(long long)a.row_peak * (RAG ? a.ragged_stride : a.T)] = tpk;
+                if (a.row_mean_amp >= 0) orow[(long long)a.row_mean_amp * (RAG ? a.ragged_stride : a.T)] = (float)(tabs / n);
                 if (a.row_std_amp >= 0) {
                     const double mu = tsum / n;
                     double var = tsq / n - mu * mu;
                     if (var < 0.0) var = 0.0;
-                    orow[(long long)a.row_std_amp * a.T] = (float)sqrt(var);
+                    orow[(long long)a.row_std_amp * (RAG ? a.ragged_stride : a.T)] = (float)sqrt(var);
                 }
             }
         }
@@ -282,10 +284,10 @@ __global__ void __launch_bounds__(NT) frame_mixed_kernel(const syg::FrameArgs a,
             const double tkm = group_sum<NT>(skm, dsc);
             double centroid_hz = 0.0;
             if (tm >= kEps64) centroid_hz = a.bin_hz * (tkm / tm);
-            if (a.row_centroid >= 0 && tid == 0) orow[(long long)a.row_centroid * a.T] = (float)centroid_hz;
+            if (a.row_centroid >= 0 && tid == 0) orow[(long long)a.row_centroid * (RAG ? a.ragged_stride : a.T)] = (float)centroid_hz;
             if (a.row_rolloff >= 0) {
                 if (total_p < kEps64) {
-                    if (tid == 0) orow[(long long)a.row_rolloff * a.T] = (float)(a.bin_hz * (double)(B - 1));
+                    if (tid == 0) orow[(long long)a.row_rolloff * (RAG ? a.ragged_stride : a.T)] = (float)(a.bin_hz * (double)(B - 1));
                 } else {
                     const double thr = a.roll_percent * total_p;
                     if (incl >= thr && prev < thr) {                    // exactly one thread
@@ -295,7 +297,7 @@ __global__ void __launch_bounds__(NT) frame_mixed_kernel(const syg::FrameArgs a,
                             c += (double)SLD(&pw[padi(k)]);
                             if (c >= thr) { bin = k; break; }
                         }
-                        orow[(long long)a.row_rolloff * a.T] = (float)(a.bin_hz * (double)bin);
+                        orow[(long long)a.row_rolloff * (RAG ? a.ragged_stride : a.T)] = (float)(a.bin_hz * (double)bin);
                     }
                 }
             }
@@ -308,7 +310,7 @@ __global__ void __launch_bounds__(NT) frame_mixed_kernel(const syg::FrameArgs a,
                         fl = exp(tl / (double)B) / am;
                         fl = fl < 0.0 ? 0.0 : (fl > 1.0 ? 1.0 : fl);
                     }
-                    orow[(long long)a.row_flatness * a.T] = (float)fl;
+                    orow[(long long)a.row_flatness * (RAG ? a.ragged_stride : a.T)] = (float)fl;
                 }
             }
             if (a.row_bandwidth >= 0) {
@@ -319,14 +321,14 @@ __global__ void __launch_bounds__(NT) frame_mixed_kernel(const syg::FrameArgs a,
                     sb += mg * d * d;
                 }
                 const double tb = group_sum<NT>(sb, dsc);
-                if (tid == 0) orow[(long long)a.row_bandwidth * a.T] = (tm < kEps64) ? 0.0f : (float)sqrt(tb / tm);
+                if (tid == 0) orow[(long long)a.row_bandwidth * (RAG ? a.ragged_stride : a.T)] = (tm < kEps64) ? 0.0f : (float)sqrt(tb / tm);
             }
             if (a.row_dominant >= 0) {
                 // np.argmax: first bin attaining the maximum = smallest index among the threads holding it
                 const float gmax = group_max<NT>(vmax, dsc);
                 float mi = (vmax == gmax) ? -(float)imax : -1.0e9f;
                 mi = group_max<NT>(mi, dsc);
-                if (tid == 0) orow[(long long)a.row_dominant * a.T] = (float)(a.bin_hz * (double)(-mi));
+                if (tid == 0) orow[(long long)a.row_dominant * (RAG ? a.ragged_stride : a.T)] = (float)(a.bin_hz * (double)(-mi));
             }
         }
 

@@ -7,6 +7,7 @@ namespace sygdev {
 constexpr int kThreads = 256;               // threads per CTA of every kernel
 constexpr int MODE_FEATURES = 0;            // frame kernel modes
 constexpr int MODE_STFT = 1;
+constexpr int MODE_FEATURES_RAGGED = 2;     // features of units with their own lengths (FrameArgs::ragged_ut)
 constexpr int kFinTT = 32;                  // frames per finalize CTA
 // row pitch (floats) of the finalize kernel's S_db tile for N mel bands: >= N and 4 mod 8, so that rows start 16-byte aligned
 // and the 8 frames x 4 columns of a DMMA B fragment (and its mirrored columns) fall on 32 distinct banks
@@ -124,6 +125,11 @@ struct FrameArgs {
     // ---- stft
     int out_kind;               // 0 complex64, 1 magnitude, 2 power
     void* stft_out;             // [n_units][B][T]
+    // ---- ragged launches (MODE_FEATURES_RAGGED, frame_warp_kernel STAGE 6): units of their own lengths.  ragged_ut[gf] =
+    // {unit, frame in unit, unit length, unit start in y} of frame gf (one load, nothing that depends on another load; the chunk's
+    // samples span less than 2^31); row r of frame gf goes to out[r * ragged_stride + gf].  T and the tables of g are unused.
+    const int4* ragged_ut;      // [n_frames]
+    long long ragged_stride;    // >= n_frames
 };
 
 // run-time plan of the mixed-radix kernels (syg_mixed.cuh): n real samples per transform, L complex points in shared memory
@@ -145,6 +151,9 @@ struct FinalizeArgs {
     const float* cws;
     const unsigned* unit_max;
     float* out;
+    const int4* ragged_ut;              // ragged launches: [n_frames] {unit, frame in unit, ...} (T unused)
+    long long n_frames;                 // ragged launches: frames of the chunk
+    long long ragged_stride;            // ragged launches: row r of frame gf at out[r * ragged_stride + gf]
 };
 
 struct WelchArgs {
