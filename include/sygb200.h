@@ -248,8 +248,29 @@ int syg_spectral_contrast_from_mag_f32(syg_ctx* ctx, const float* S_dev, int32_t
                                        double fmin, double quantile, float* out_dev, void* stream);
 
 /* which kernel family the last syg_stft_* call of this process launched: 1 TMA-staged ring kernel, 2 register-staged warp
- * kernel, 3 CTA-cooperative kernels, 4 sub-FFT kernel for n_fft 4096 / 8192 (tests and bench.py report it) */
+ * kernel, 3 CTA-cooperative kernels, 4 sub-FFT kernel for n_fft 4096 / 8192, 5 mixed-radix kernel (tests and bench.py report it).
+ * Two values only the SYGB200_* comparison switches reach (DESIGN.md 6): 6 the per-frame CTA kernel frame_kernel<MODE_STFT> in
+ * place of the default kernel (SYGB200_STFT_BLOCK=1), 7 the warp kernel's CTA tile for magnitude / power output at n_fft <= 512
+ * (SYGB200_STFT_CTA_TILE=1). */
 int syg_debug_last_stft_path(void);
+/* frame-kernel instantiation of the last syg_features_* / syg_segment_vectors_* launch (uniform and ragged forms alike) */
+enum {
+    SYG_FK_WARP_WIDE = 1,    /* generic warp kernel, 640 threads (n_fft 2048)                                            */
+    SYG_FK_WARP = 2,         /* generic warp kernel, 256 threads (n_fft <= 1024; 2048 when the plan tables need the room)  */
+    SYG_FK_SPEC44K = 3,      /* n_fft 2048 kernels with plan constants: 44.1 kHz contrast bands / mel sweeps                */
+    SYG_FK_SPEC22K = 4,      /*   22.05 kHz contrast bands / mel sweeps                                                       */
+    SYG_FK_SPEC44KL = 5,     /*   Spec44k plus the feature set and row layout of the reference's default request             */
+    SYG_FK_RESIDENT = 6,     /* unit-resident warp kernel (mel tile, dB and DCT on chip, no finalize launch)                */
+    SYG_FK_BLOCK = 7,        /* CTA-cooperative frame kernel (n_fft 4096 / 8192)                                           */
+    SYG_FK_MIXED = 8         /* mixed-radix kernel (lengths that are not powers of two)                                    */
+};
+int syg_debug_last_feature_kernel(void);
+/* the last finalize launch of a feature call (mel dB + DCT + contrast): frames per CTA tile, CTAs, tiles (a grid-stride loop
+ * covers tiles > ctas); all three 0 before the first one */
+void syg_debug_last_finalize(int32_t* tile_frames, int64_t* ctas, int64_t* tiles);
+/* kernel of the last syg_psd_welch_* call */
+enum { SYG_WELCH_WARP = 1, SYG_WELCH_BLOCK = 2, SYG_WELCH_MIXED = 3 };
+int syg_debug_last_welch_path(void);
 /* 1 when the last feature launch kept its (short) units on chip: mel tile + dB + DCT inside the frame kernel, no finalize launch */
 int syg_debug_last_features_resident(void);
 /* frames the feature kernels processed in the last syg_features_* / syg_segment_vectors_* call, all chunks (n_units * T for the

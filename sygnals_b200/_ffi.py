@@ -44,6 +44,9 @@ AGG_IDS = {"mean": 0, "std": 1, "median": 2, "min": 3, "max": 4}      # formatte
 PCM_U8, PCM_S16, PCM_S24, PCM_S32, PCM_F32 = 0, 1, 2, 3, 4              # sample formats of a WAV 'data' payload
 PCM_BYTES = {PCM_U8: 1, PCM_S16: 2, PCM_S24: 3, PCM_S32: 4, PCM_F32: 4}
 MAX_FEATURES = 16
+# syg_debug_last_feature_kernel / syg_debug_last_welch_path values (include/sygb200.h)
+FK_WARP_WIDE, FK_WARP, FK_SPEC44K, FK_SPEC22K, FK_SPEC44KL, FK_RESIDENT, FK_BLOCK, FK_MIXED = 1, 2, 3, 4, 5, 6, 7, 8
+WELCH_WARP, WELCH_BLOCK, WELCH_MIXED = 1, 2, 3
 
 
 class EngineError(RuntimeError):
@@ -126,6 +129,9 @@ class Library:
             "syg_debug_last_features_resident": (C.c_int, []),
             "syg_debug_last_feature_frames": (i64, []),
             "syg_debug_last_mel_form": (C.c_int, []),
+            "syg_debug_last_feature_kernel": (C.c_int, []),
+            "syg_debug_last_finalize": (None, [C.POINTER(i32), C.POINTER(i64), C.POINTER(i64)]),
+            "syg_debug_last_welch_path": (C.c_int, []),
             "syg_debug_set_resident_min_groups": (None, [C.c_int]),
             "syg_debug_window": (C.c_int, [i32, i32, i32, vp]),
             "syg_debug_mel_basis": (C.c_int, [i32, i32, i32, f64, f64, vp]),
@@ -191,6 +197,12 @@ class Library:
     def last_feature_frames(self) -> int:
         """Frames the feature kernels processed in the last features / segment-vectors call of this process."""
         return int(self.dll.syg_debug_last_feature_frames())
+
+    def last_finalize(self) -> tuple:
+        """(frames per tile, CTAs, tiles) of the last finalize launch of a feature call."""
+        tt, ctas, tiles = C.c_int32(0), C.c_int64(0), C.c_int64(0)
+        self.dll.syg_debug_last_finalize(C.byref(tt), C.byref(ctas), C.byref(tiles))
+        return int(tt.value), int(ctas.value), int(tiles.value)
 
     def debug_window(self, window: int, win_length: int, n_fft: int) -> np.ndarray:
         out = np.zeros(n_fft, dtype=np.float32)

@@ -281,12 +281,8 @@ int get_window(syg_ctx* ctx, int window, int win_length, int n_fft, bool centred
 // failures as a negative SYG_E_* code plus a message.
 int launch_rc(int rc, const std::string& err) { return rc == SYG_OK ? SYG_OK : fail(rc, "%s", err.c_str()); }
 
-int launch_features(int n_fft, const syg::FrameArgs& a_in, int sm_count, cudaStream_t st) {
+int launch_features(int n_fft, const syg::FrameArgs& a, int sm_count, cudaStream_t st) {
     std::string err;
-    static int variant = -1;
-    if (variant < 0) { const char* e = std::getenv("SYGB200_VARIANT"); variant = e ? std::atoi(e) : 0; }
-    syg::FrameArgs a = a_in;
-    a.variant = variant;
     const bool rag = a.ragged_ut != nullptr;
     const int mode = rag ? sygdev::MODE_FEATURES_RAGGED : sygdev::MODE_FEATURES;
     if (!native_pow2(n_fft)) {
@@ -306,11 +302,14 @@ int warp_fw(int n_fft) {
     switch (ilog2i(n_fft / 2)) { case 4: return 8; case 5: return 8; case 6: return 4; case 7: return 4; case 8: return 2; case 9: return 2; default: return 1; }
 }
 
+}  // namespace
+namespace syglaunch { LastLaunch g_last; }
+namespace {
+
 int g_resident_min_groups = -1;     // unit groups a launch needs before the resident kernel is chosen (-1: 4 per SM); tests lower it
 int g_last_mel_form = 0;            // 1: the last feature launch with MFCCs used the interval-form mel projection
 int g_last_features_resident = 0;   // 1: the last feature launch kept its units on chip (frame_warp_kernel STAGE 5)
 long long g_last_feature_frames = 0; // frames the feature kernels processed in the last syg_features_* / syg_segment_vectors_* call
-int g_last_stft_path = 0;   // 5 mixed-radix kernel (lengths that are not powers of two), 1 ring (TMA-staged), 2 warp kernel (register-staged), 3 CTA-cooperative kernels, 4 sub-FFT kernel (n_fft 4096 / 8192): last STFT launch
 
 int launch_stft(int n_fft, const syg::FrameArgs& a, int sm_count, cudaStream_t st) {
     std::string err;
@@ -319,20 +318,20 @@ int launch_stft(int n_fft, const syg::FrameArgs& a, int sm_count, cudaStream_t s
     if (!native_pow2(n_fft)) {
         syg::MixedPlan mp;
         if (int rc = mixed_plan_of(n_fft, false, mp, "n_fft")) return rc;
-        g_last_stft_path = 5;
+        syglaunch::g_last.stft_path = 5;
         return launch_rc(syglaunch::frame_mixed(sygdev::MODE_STFT, a, mp, sm_count, st, err), err);
     }
     if (n_fft >= 4096 && !env && a.out_kind != 0) {
-        g_last_stft_path = 4;
+        syglaunch::g_last.stft_path = 4;
         return launch_rc(syglaunch::stft_big(n_fft, a, sm_count, st, err), err);
     }
     if (n_fft <= 2048 && !env) {
         const int rrc = syglaunch::stft_ring(n_fft, a, sm_count, st, err);      // samples staged by the TMA engine where the layout allows it
-        g_last_stft_path = rrc <= 0 ? 1 : 2;
+        syglaunch::g_last.stft_path = rrc <= 0 ? 1 : 2;
         if (rrc <= 0) return launch_rc(rrc, err);
         return launch_rc(syglaunch::frame_warp_stft(n_fft, a, sm_count, st, err), err);
     }
-    g_last_stft_path = 3;
+    syglaunch::g_last.stft_path = env ? 6 : 3;                          // 6: frame_kernel in place of the default kernel
     return launch_rc(syglaunch::frame_block(n_fft, sygdev::MODE_STFT, a, sm_count, st, err), err);
 }
 
@@ -571,6 +570,27 @@ int build_feature_plan(syg_ctx* ctx, const syg_units* u, const syg_feature_param
     return SYG_OK;
 }
 
+// The finalize launch of a feature chunk of n_frames frames (uniform and ragged).  Tile height: 64 frames for narrow mel banks (the
+// CTA is latency bound, twice the frames amortise it), else 32; one CTA per tile.  SYGB200_FIN_TT=32|64 overrides the tile height and
+// SYGB200_FIN_CTAS=k caps the grid at k CTAs per SM, the kernel's grid-stride loop then covers the remaining tiles (A/B measurements).
+int launch_finalize(syg_ctx* ctx, const syg::FinalizeArgs& f, long long n_frames, cudaStream_t st) {
+    static int fin_tt = -1;
+    if (fin_tt < 0) { const char* e = std::getenv("SYGB200_FIN_TT"); fin_tt = e ? std::atoi(e) : 0; }
+    static int fin_cap = -1;
+    if (fin_cap < 0) { const char* e = std::getenv("SYGB200_FIN_CTAS"); fin_cap = e ? std::atoi(e) : 0; }
+    const int tt = fin_tt == 32 || fin_tt == 64 ? fin_tt : ((f.row_mfcc >= 0 && f.n_mels <= 64) ? 64 : 32);
+    const size_t smem = sygdev::fin_smem_bytes(tt, f.n_mels, f.dct_fold != 0);         // folded FP64 S_db rows
+    const long long n_tiles = (n_frames + tt - 1) / tt;
+    const long long cap = fin_cap > 0 ? (long long)ctx->sm_count * fin_cap : 0x7fffffffLL;
+    const unsigned grid = (unsigned)std::min<long long>(n_tiles, cap);
+    syglaunch::g_last.fin_tt = tt;
+    syglaunch::g_last.fin_ctas = grid;
+    syglaunch::g_last.fin_tiles = n_tiles;
+    std::string err;
+    const int frc = syglaunch::finalize(f, tt, grid, 1u, smem, st, err);
+    return frc ? fail(frc, "%s", err.c_str()) : SYG_OK;
+}
+
 // run the two kernels for units [0, n) of geometry g, writing out rows for those units
 int run_features_chunk(syg_ctx* ctx, const FeaturePlan& pl, const float* y, const syg::UnitGeom& g, float* out,
                        void* ws, int n_fft, cudaStream_t st) {
@@ -632,18 +652,7 @@ int run_features_chunk(syg_ctx* ctx, const FeaturePlan& pl, const float* y, cons
         f.cws = a.cws;
         f.unit_max = a.unit_max;
         f.out = out;
-        static int fin_tt = -1;                                       // SYGB200_FIN_TT=32|64 overrides the tile height (A/B)
-        if (fin_tt < 0) { const char* e = std::getenv("SYGB200_FIN_TT"); fin_tt = e ? std::atoi(e) : 0; }
-        const int tt = fin_tt == 32 || fin_tt == 64 ? fin_tt : ((f.row_mfcc >= 0 && f.n_mels <= 64) ? 64 : 32);
-        const size_t smem = sygdev::fin_smem_bytes(tt, f.n_mels, f.dct_fold != 0);         // folded FP64 S_db rows
-        const long long n_tiles = (g.n_units * (long long)pl.T + tt - 1) / tt;
-        static int fin_cap = -1;                                      // SYGB200_FIN_CTAS: CTAs per SM of the finalize grid (0 = one CTA per tile)
-        if (fin_cap < 0) { const char* e = std::getenv("SYGB200_FIN_CTAS"); fin_cap = e ? std::atoi(e) : 0; }
-        const long long cap = fin_cap > 0 ? (long long)ctx->sm_count * fin_cap : 0x7fffffffLL;
-        const unsigned grid = (unsigned)std::min<long long>(n_tiles, cap);
-        std::string err;
-        const int frc = syglaunch::finalize(f, tt, grid, 1u, smem, st, err);
-        if (frc) return fail(frc, "%s", err.c_str());
+        if (int frc = launch_finalize(ctx, f, g.n_units * (long long)pl.T, st)) return frc;
     }
     return SYG_OK;
 }
@@ -1030,11 +1039,7 @@ int run_ragged_chunk(syg_ctx* ctx, const FeaturePlan& pl, const float* y, const 
     f.ragged_ut = ut;
     f.n_frames = nf;
     f.ragged_stride = out_stride;
-    const int tt = (f.row_mfcc >= 0 && f.n_mels <= 64) ? 64 : 32;     // as run_features_chunk
-    const size_t smem = sygdev::fin_smem_bytes(tt, f.n_mels, f.dct_fold != 0);
-    const unsigned grid = (unsigned)std::min<long long>((nf + tt - 1) / tt, 0x7fffffffLL);
-    if (int frc = syglaunch::finalize(f, tt, grid, 1u, smem, st, err)) return fail(frc, "%s", err.c_str());
-    return SYG_OK;
+    return launch_finalize(ctx, f, nf, st);
 }
 
 int check_agg(const FeaturePlan& pl, const int32_t* agg) {
@@ -1707,7 +1712,14 @@ int syg_spectral_contrast_from_mag_f32(syg_ctx* ctx, const float* S_dev, int32_t
     return rc ? fail(rc, "%s", err.c_str()) : SYG_OK;
 }
 
-int syg_debug_last_stft_path(void) { return g_last_stft_path; }
+int syg_debug_last_stft_path(void) { return syglaunch::g_last.stft_path; }
+int syg_debug_last_feature_kernel(void) { return syglaunch::g_last.feature_kernel; }
+void syg_debug_last_finalize(int32_t* tile_frames, int64_t* ctas, int64_t* tiles) {
+    if (tile_frames) *tile_frames = syglaunch::g_last.fin_tt;
+    if (ctas) *ctas = syglaunch::g_last.fin_ctas;
+    if (tiles) *tiles = syglaunch::g_last.fin_tiles;
+}
+int syg_debug_last_welch_path(void) { return syglaunch::g_last.welch_path; }
 int syg_debug_last_features_resident(void) { return g_last_features_resident; }
 int64_t syg_debug_last_feature_frames(void) { return g_last_feature_frames; }
 int syg_debug_last_mel_form(void) { return g_last_mel_form; }

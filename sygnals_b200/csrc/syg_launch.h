@@ -3,9 +3,20 @@
 
 #include <string>
 
+#include "../../include/sygb200.h"
 #include "syg_params.h"
 
 namespace syglaunch {
+// what the last launch of each kernel family ran, for the syg_debug_last_* getters: one host store per launch
+struct LastLaunch {
+    int feature_kernel = 0;        // SYG_FK_*
+    int stft_path = 0;             // syg_debug_last_stft_path
+    int welch_path = 0;            // SYG_WELCH_*
+    int fin_tt = 0;                // finalize: frames per tile, CTAs, tiles
+    long long fin_ctas = 0, fin_tiles = 0;
+};
+extern LastLaunch g_last;
+
 // all return 0 or a negative SYG_E_* code (-3 CUDA, -5 unsupported) with a message in err
 int frame_block(int n_fft, int mode, const syg::FrameArgs& a, int sm_count, cudaStream_t st, std::string& err);
 int frame_warp(int n_fft, bool extra, const syg::FrameArgs& a, int sm_count, cudaStream_t st, std::string& err);

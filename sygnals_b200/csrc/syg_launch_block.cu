@@ -17,6 +17,7 @@ static int frame_block_t(const syg::FrameArgs& a, int sm_count, cudaStream_t st,
     const long long n_rounds = (a.n_frames + TL::F - 1) / TL::F;
     if (n_rounds <= 0) return 0;
     const int grid = (int)std::min<long long>(n_rounds, (long long)sm_count * blocks_per_sm);
+    if constexpr (MODE != sygdev::MODE_STFT) g_last.feature_kernel = SYG_FK_BLOCK;
     SYG_LAUNCH(kfn, grid, sygdev::kThreads, SM::bytes, st, a);
     LCK(cudaGetLastError());
     return 0;

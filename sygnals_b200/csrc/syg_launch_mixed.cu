@@ -16,6 +16,7 @@ static int frame_mixed_t(const syg::FrameArgs& a, const syg::MixedPlan& mp, int 
     if (int rc = prepare_kernel(kfn, NT, smem, kc, &blocks_per_sm, err)) return rc;
     if (a.n_frames <= 0) return 0;
     const int grid = (int)std::min<long long>(a.n_frames, (long long)sm_count * blocks_per_sm);
+    if constexpr (MODE != sygdev::MODE_STFT) g_last.feature_kernel = SYG_FK_MIXED;
     SYG_LAUNCH(kfn, grid, NT, smem, st, a, mp);
     LCK(cudaGetLastError());
     return 0;
@@ -45,6 +46,7 @@ static int welch_mixed_t(const syg::WelchArgs& a, const syg::MixedPlan& mp, int 
     if (int rc = prepare_kernel(kfn, NT, smem, kc, &blocks_per_sm, err)) return rc;
     if (a.g.n_units <= 0) return 0;
     const int grid = (int)std::min<long long>(a.g.n_units, (long long)sm_count * blocks_per_sm);
+    g_last.welch_path = SYG_WELCH_MIXED;
     SYG_LAUNCH(kfn, grid, NT, smem, st, a, mp);
     LCK(cudaGetLastError());
     return 0;

@@ -2,6 +2,7 @@
 #pragma once
 
 #include <cstdlib>
+#include <type_traits>
 
 #include "syg_launch_common.h"
 #include "syg_frame_warp.cuh"
@@ -43,6 +44,11 @@ static int frame_warp_t(const syg::FrameArgs& a, int sm_count, cudaStream_t st, 
     const long long n_rounds = (a.n_frames + per_cta - 1) / per_cta;
     if (n_rounds <= 0) return 0;
     const int grid = (int)std::min<long long>(n_rounds, (long long)sm_count * blocks_per_sm_w);
+    if constexpr (STAGE == 0 || STAGE == 6)
+        g_last.feature_kernel = std::is_same<SP, sygdev::Spec44kL>::value ? SYG_FK_SPEC44KL
+                                : std::is_same<SP, sygdev::Spec44k>::value ? SYG_FK_SPEC44K
+                                : std::is_same<SP, sygdev::Spec22k>::value ? SYG_FK_SPEC22K
+                                : NT == SYG_NT2048 ? SYG_FK_WARP_WIDE : SYG_FK_WARP;
     SYG_LAUNCH(kfn, grid, NT, smem, st, a);
     LCK(cudaGetLastError());
     return 0;

@@ -48,6 +48,7 @@ int res_t(const syg::FrameArgs& a_in, int sm_count, cudaStream_t st, std::string
     const long long n_groups = (a.g.n_units + a.res_units - 1) / a.res_units;
     if (n_groups <= 0) return 0;
     const int grid = (int)std::min<long long>(n_groups, (long long)sm_count * bps);
+    g_last.feature_kernel = SYG_FK_RESIDENT;
     SYG_LAUNCH(kfn, grid, NT, smem, st, a);
     LCK(cudaGetLastError());
     return 0;

@@ -9,7 +9,10 @@ int frame_warp_stft(int n_fft, const syg::FrameArgs& a, int sm_count, cudaStream
     // real-valued output of the small transforms: warp-private tiles (no CTA barrier); SYGB200_STFT_CTA_TILE=1 keeps the CTA tile
     static int env = -1;
     if (env < 0) { const char* e = std::getenv("SYGB200_STFT_CTA_TILE"); env = e ? std::atoi(e) : 0; }
-    if (!env && a.out_kind != 0 && n_fft <= 512) return frame_warp_dispatch<false, 4>(n_fft, a, sm_count, st, err);
+    if (a.out_kind != 0 && n_fft <= 512) {
+        if (!env) return frame_warp_dispatch<false, 4>(n_fft, a, sm_count, st, err);
+        g_last.stft_path = 7;                                           // reached only through the switch
+    }
     return frame_warp_dispatch<false, 3>(n_fft, a, sm_count, st, err);
 }
 }  // namespace syglaunch

@@ -16,6 +16,7 @@ static int welch_t(const syg::WelchArgs& a, int sm_count, cudaStream_t st, std::
     if (int rc = prepare_kernel(kfn, sygdev::kThreads, SM::bytes, kc, &blocks_per_sm, err)) return rc;
     if (a.g.n_units <= 0) return 0;
     const int grid = (int)std::min<long long>(a.g.n_units, (long long)sm_count * blocks_per_sm);
+    g_last.welch_path = SYG_WELCH_BLOCK;
     SYG_LAUNCH(kfn, grid, sygdev::kThreads, SM::bytes, st, a);
     LCK(cudaGetLastError());
     return 0;
@@ -31,6 +32,7 @@ static int welch_warp_t(const syg::WelchArgs& a, int sm_count, cudaStream_t st, 
     if (a.g.n_units <= 0) return 0;
     const long long want = (a.g.n_units + NT / 32 - 1) / (NT / 32);
     const int grid = (int)std::min<long long>(want, (long long)sm_count * blocks_per_sm);
+    g_last.welch_path = SYG_WELCH_WARP;
     SYG_LAUNCH(kfn, grid, NT, WW::bytes, st, a);
     LCK(cudaGetLastError());
     return 0;

@@ -116,7 +116,6 @@ struct FrameArgs {
     int mel_iv;                 // 1: mel_pw holds the interval-form blob (sygplan::MelIntervals) instead of sweep taps
     int mel_nsweeps;            // sweeps of the warp kernel's mel plan and their float4 step counts (host side: lets the launcher
     int mel_steps[8];           // pick a plan-specialised kernel); 0 sweeps = not recorded
-    int variant;                // measurement switch (SYGB200_VARIANT, default 0): bit 0 = per-scheduler lock step (see frame_warp_kernel)
     // ---- unit-resident MFCC epilogue (frame_warp_kernel STAGE 5): the finalize arguments + units per CTA group
     int res_units;
     const double* fin_dct;

@@ -58,7 +58,9 @@ def test_layout_specialised_kernel_equals_the_plan_specialised_one(eng):
     from sygnals_b200.batch import feature_row_names
     u = eng.units_clips(y.shape[0], y.shape[1])
     out_l = eng.features_host(y.ravel(), u, _ffi.make_params(eng.lib, sr, order_l, n_fft, hop))
+    assert eng.lib.dll.syg_debug_last_feature_kernel() == _ffi.FK_SPEC44KL
     out_p = eng.features_host(y.ravel(), u, _ffi.make_params(eng.lib, sr, order_p, n_fft, hop))
+    assert eng.lib.dll.syg_debug_last_feature_kernel() == _ffi.FK_SPEC44K
     names_l, names_p = feature_row_names(order_l, None), feature_row_names(order_p, None)
     assert sorted(names_l) == sorted(names_p) and len(names_l) == 24
     for i, n in enumerate(names_l):
