@@ -103,8 +103,8 @@ struct PinnedBuf {                 // page-locked host staging owned by a lane (
 
 struct Lane {                      // one in-flight chunk of a *_host_* call
     cudaStream_t stream = nullptr;
-    DevBuf in, raw, out0, out1, starts, valid, ws, feat;
-    PinnedBuf tbl;                 // explicit unit tables of the chunk (starts | valid), reused once tbl_done has passed
+    DevBuf in, raw, out0, out1, units, ws;   // units: the chunk's explicit unit tables (starts | valid)
+    PinnedBuf tbl;                 // host image of the chunk's unit tables, reused once tbl_done has passed
     cudaEvent_t tbl_done = nullptr;
     bool tbl_used = false;
 };
@@ -150,6 +150,24 @@ struct ProfScope {
     ~ProfScope() {
         if (a && b) { cudaEventRecord(b, st); c->prof_pairs.push_back({a, b, kind}); }
     }
+};
+
+// The workspace of the device-pointer entry points is shared by every call on the context: a claim orders the kernels the call
+// enqueues on st behind the previous user's, whatever stream that was (calls on ONE stream are ordered anyway; two streams would
+// otherwise overwrite each other's mel energies), and the next user behind them (ws_done, recorded when the claim leaves scope).
+struct WsClaim {
+    syg_ctx* ctx;
+    cudaStream_t st;
+    bool held = false;
+    int claim(size_t bytes) {
+        if (ctx->ws_done) CK(cudaStreamWaitEvent(st, ctx->ws_done, 0));
+        else CK(cudaEventCreateWithFlags(&ctx->ws_done, cudaEventDisableTiming));
+        if (bytes > ctx->ws.cap) CK(cudaStreamSynchronize(st));   // growing frees the old block: nothing may still use it
+        if (int rc = ctx->ws.ensure(bytes)) return rc;
+        held = true;
+        return SYG_OK;
+    }
+    ~WsClaim() { if (held) cudaEventRecord(ctx->ws_done, st); }
 };
 }  // namespace
 
@@ -587,32 +605,77 @@ int launch_finalize(syg_ctx* ctx, const syg::FinalizeArgs& f, long long n_frames
     syglaunch::g_last.fin_ctas = grid;
     syglaunch::g_last.fin_tiles = n_tiles;
     std::string err;
-    const int frc = syglaunch::finalize(f, tt, grid, 1u, smem, st, err);
-    return frc ? fail(frc, "%s", err.c_str()) : SYG_OK;
+    return launch_rc(syglaunch::finalize(f, tt, grid, 1u, smem, st, err), err);
 }
 
-// run the two kernels for units [0, n) of geometry g, writing out rows for those units
-int run_features_chunk(syg_ctx* ctx, const FeaturePlan& pl, const float* y, const syg::UnitGeom& g, float* out,
-                       void* ws, int n_fft, cudaStream_t st) {
+size_t al256(size_t b) { return (b + 255) / 256 * 256; }
+
+// consecutive 256-byte aligned parts of a block at base; with a null base it only counts the bytes
+struct Carve {
+    char* base;
+    size_t bytes = 0;
+    template <class T> T* take(size_t count) {
+        T* p = base ? reinterpret_cast<T*>(base + bytes) : nullptr;
+        bytes += al256(count * sizeof(T));
+        return p;
+    }
+};
+
+// The workspace of a feature chunk of n units and nf frames, each part 256-byte aligned: unit maxima, mel energies, contrast peaks /
+// valleys, the frame table of a ragged chunk, the frame features [n_rows][nf] of an aggregated chunk, then 256 spare bytes.  With a
+// null base it only sizes the block.
+struct FeatWs {
+    unsigned* unit_max = nullptr;
+    float* melws = nullptr;
+    float* cws = nullptr;
+    int4* ut = nullptr;
+    float* feat = nullptr;
+    size_t bytes = 0;
+};
+FeatWs feat_ws(const FeaturePlan& pl, long long n, long long nf, bool ragged, bool agg, void* base = nullptr) {
+    Carve c{static_cast<char*>(base)};
+    FeatWs w;
+    w.unit_max = c.take<unsigned>((size_t)n * 4);
+    w.melws = c.take<float>((size_t)nf * pl.fin.n_mels);
+    w.cws = c.take<float>((size_t)nf * 2 * pl.fin.nb);
+    if (ragged) w.ut = c.take<int4>(nf);
+    if (agg) w.feat = c.take<float>((size_t)nf * pl.n_rows);
+    w.bytes = c.bytes + 256;
+    return w;
+}
+
+// device tables of a ragged chunk, per unit: frame_off (one more entry), starts, lengths, and for the aggregation the unit's first
+// frame relative to its chunk and its frame count
+struct RaggedTbl { long long* foff; long long* starts; int* valid; long long* seg_off; int* seg_len; size_t bytes; };
+
+// The feature kernels on one chunk of the units g, nf frames, in the workspace w (feat_ws).  Uniform chunks (rt == nullptr) write
+// rows [unit][row][T] to out; ragged ones build their frame table from the device tables rt (y and the tables chunk-relative) and
+// write row r of frame f to out[r * out_stride + f].
+int run_features_chunk(syg_ctx* ctx, const FeaturePlan& pl, const float* y, const syg::UnitGeom& g, const RaggedTbl* rt, long long nf,
+                       long long out_stride, float* out, const FeatWs& w, cudaStream_t st) {
+    const int n_fft = pl.n_fft;
     syg::FrameArgs a = pl.fa;
     a.y = y;
     a.g = g;
-    a.n_frames = g.n_units * (long long)pl.T;
+    a.n_frames = nf;
     a.out = out;
-    char* w = reinterpret_cast<char*>(ws);
-    a.unit_max = reinterpret_cast<unsigned*>(w);
-    size_t off = ((size_t)g.n_units * 4 * sizeof(unsigned) + 255) / 256 * 256;
-    a.melws = reinterpret_cast<float*>(w + off);
-    off += ((size_t)a.n_frames * pl.fin.n_mels * sizeof(float) + 255) / 256 * 256;
-    a.cws = reinterpret_cast<float*>(w + off);
+    a.unit_max = w.unit_max;
+    a.melws = w.melws;
+    a.cws = w.cws;
+    if (rt) {
+        a.T = 0;
+        a.ragged_stride = out_stride;
+        a.ragged_ut = w.ut;
+    }
     // Short units with an MFCC-only epilogue stay on chip (frame_warp_kernel STAGE 5): no mel workspace, no finalize launch.  Needs
-    // enough unit groups to fill the GPU; SYGB200_NO_RES=1 keeps the two-kernel path (A/B measurements).
+    // enough unit groups to fill the GPU; SYGB200_NO_RES=1 keeps the two-kernel path (A/B measurements).  The epilogue sizes its
+    // tile by units x T: uniform chunks only.
     {
         static int no_res = -1;
         if (no_res < 0) { const char* e = std::getenv("SYGB200_NO_RES"); no_res = e ? std::atoi(e) : 0; }
         constexpr unsigned other = syg::FB_CONTRAST | syg::FB_BANDWIDTH | syg::FB_FLATNESS | syg::FB_DOMINANT | syg::FB_MEAN_AMP | syg::FB_STD_AMP;
         a.res_units = 0;
-        if (!no_res && (a.mask & syg::FB_MFCC) && !(a.mask & other) && native_pow2(n_fft) && n_fft <= 1024) {
+        if (!rt && !no_res && (a.mask & syg::FB_MFCC) && !(a.mask & other) && native_pow2(n_fft) && n_fft <= 1024) {
             const int ku = syglaunch::frame_warp_res_units(n_fft, a);
             const long long min_groups = g_resident_min_groups >= 0 ? g_resident_min_groups : 4LL * ctx->sm_count;
             if (ku > 0 && (g.n_units + ku - 1) / ku >= min_groups) {
@@ -627,48 +690,66 @@ int run_features_chunk(syg_ctx* ctx, const FeaturePlan& pl, const float* y, cons
         }
     }
     g_last_features_resident = a.res_units > 0 ? 1 : 0;
-    g_last_feature_frames += a.n_frames;
+    g_last_feature_frames += nf;
     if (a.mask & syg::FB_MFCC) g_last_mel_form = a.mel_iv ? 1 : 0;
+    if (nf == 0) return SYG_OK;            // only ragged units without frames: nothing to compute (and no zero-CTA finalize launch)
+    std::string err;
+    int rc = SYG_OK;
+    if (rt) {
+        ProfScope ps(ctx, st, PROF_OTHER);
+        rc = launch_rc(syglaunch::ragged_frame_table(rt->foff, rt->starts, rt->valid, g.n_units, nf, w.ut, ctx->sm_count, st, err), err);
+        if (rc) return rc;
+    }
     const bool need_fin = (a.mask & (syg::FB_MFCC | syg::FB_CONTRAST)) != 0 && a.res_units == 0;
     if (need_fin) CK(cudaMemsetAsync(a.unit_max, 0, (size_t)g.n_units * 4 * sizeof(unsigned), st));
-    int rc = SYG_OK;
     if (a.mask & syg::FB_TIME_EXTRA) {                                  // zcr / skewness / kurtosis / entropy: their own streaming kernel
-        std::string err;
         ProfScope ps(ctx, st, PROF_FRAME);
-        const int trc = syglaunch::time_extra(a, n_fft, pl.entropy_bins, ctx->sm_count, st, err);
-        if (trc) return fail(trc, "%s", err.c_str());
+        rc = launch_rc(syglaunch::time_extra(a, n_fft, pl.entropy_bins, ctx->sm_count, st, err), err);
+        if (rc) return rc;
     }
     if ((a.mask & ~syg::FB_TIME_EXTRA) == 0) return SYG_OK;             // nothing for the frame kernels
     {
         ProfScope ps(ctx, st, PROF_FRAME);
         rc = launch_features(n_fft, a, ctx->sm_count, st);
     }
-    if (rc) return rc;
-    if (need_fin) {
-        ProfScope ps(ctx, st, PROF_FINALIZE);
-        syg::FinalizeArgs f = pl.fin;
-        f.n_units = g.n_units;
-        f.melws = a.melws;
-        f.cws = a.cws;
-        f.unit_max = a.unit_max;
-        f.out = out;
-        if (int frc = launch_finalize(ctx, f, g.n_units * (long long)pl.T, st)) return frc;
+    if (rc || !need_fin) return rc;
+    ProfScope ps(ctx, st, PROF_FINALIZE);
+    syg::FinalizeArgs f = pl.fin;
+    f.n_units = g.n_units;
+    f.melws = a.melws;
+    f.cws = a.cws;
+    f.unit_max = a.unit_max;
+    f.out = out;
+    if (rt) {
+        f.T = 0;
+        f.ragged_ut = w.ut;
+        f.n_frames = nf;
+        f.ragged_stride = out_stride;
     }
+    return launch_finalize(ctx, f, nf, st);
+}
+
+int check_agg(const FeaturePlan& pl, const int32_t* agg) {
+    if (pl.n_rows > 64) return fail(SYG_E_UNSUPPORTED, "aggregation supports at most 64 rows per call");
+    for (int i = 0; i < pl.n_rows; ++i)
+        if (agg[i] < SYG_AGG_MEAN || agg[i] > SYG_AGG_MAX) return fail(SYG_E_BADARG, "unknown aggregation id %d", agg[i]);
     return SYG_OK;
 }
 
-size_t features_ws_bytes(const FeaturePlan& pl, long long n) {
-    size_t b = ((size_t)n * 4 * sizeof(unsigned) + 255) / 256 * 256;
-    b += ((size_t)n * pl.T * pl.fin.n_mels * sizeof(float) + 255) / 256 * 256;
-    b += ((size_t)n * pl.T * 2 * pl.fin.nb * sizeof(float) + 255) / 256 * 256;
-    return b + 256;
+// segment vectors of n units from their frame features feat [n_rows][row_stride]: float64 [n][n_rows] to out
+int launch_aggregate(syg_ctx* ctx, const FeaturePlan& pl, const float* feat, long long n, long long row_stride, const long long* seg_off,
+                     const int* seg_len, int fixed_len, const int32_t* agg, double* out, cudaStream_t st) {
+    std::string err;
+    ProfScope ps(ctx, st, PROF_OTHER);
+    return launch_rc(syglaunch::aggregate(feat, n, pl.n_rows, row_stride, seg_off, seg_len, fixed_len, agg, out, ctx->sm_count, st, err), err);
 }
 
 // ---------------------------------------------------------------------------------------------- host pipelines
-struct HostChunk {
-    long long u0, n;               // units of the chunk
-    long long begin, end;          // sample range of y_host covered by the chunk
-};
+// samples of table unit i that its frames read: unit_valid[i] (else the rest of the buffer) clamped to [0, unit_len]
+long long table_valid(const syg_units* u, long long i) {
+    const long long v = u->unit_valid ? u->unit_valid[i] : u->total_len - u->unit_starts[i];
+    return std::min<long long>(std::max<long long>(v, 0), u->unit_len);
+}
 
 // sample range needed by units [u0, u0 + n)
 void chunk_range(const syg_units* u, long long u0, long long n, long long* begin, long long* end) {
@@ -682,9 +763,7 @@ void chunk_range(const syg_units* u, long long u0, long long n, long long* begin
     }
     long long b = u->total_len, e = 0;
     for (long long i = u0; i < u0 + n; ++i) {
-        const long long s = u->unit_starts[i];
-        long long v = u->unit_valid ? u->unit_valid[i] : u->total_len - s;
-        v = std::min<long long>(std::max<long long>(v, 0), u->unit_len);
+        const long long s = u->unit_starts[i], v = table_valid(u, i);
         if (v > 0) { b = std::min(b, s); e = std::max(e, s + v); }
     }
     if (e < b) { b = 0; e = 0; }
@@ -697,20 +776,60 @@ int check_host_units(const syg_units* u) {
     if (u->unit_starts) {
         for (long long i = 0; i < u->n_units; ++i) {
             const long long s = u->unit_starts[i];
-            long long v = u->unit_valid ? u->unit_valid[i] : u->total_len - s;
-            v = std::min<long long>(std::max<long long>(v, 0), u->unit_len);
-            if (s < 0 || s + v > u->total_len) return fail(SYG_E_BADARG, "unit %lld lies outside the sample buffer", i);
+            if (s < 0 || s + table_valid(u, i) > u->total_len) return fail(SYG_E_BADARG, "unit %lld lies outside the sample buffer", i);
         }
     }
     return SYG_OK;
 }
 
-// Generic chunked host pipeline: H2D of the chunk's samples, `run` on the lane's stream, D2H of up to two outputs.
-template <class Run>
-int host_pipeline(syg_ctx* ctx, const void* y_host_any, InFmt inf, const syg_units* u, size_t out0_per_unit, void* out0_host,
-                  size_t out1_per_unit, void* out1_host, size_t ws_per_unit, long long max_chunk_units, Run run) {
-    const unsigned char* y_bytes = reinterpret_cast<const unsigned char*>(y_host_any);
+// the two lanes of the *_host_* calls: chunks alternate between their streams (H2D, kernels and D2H of neighbours overlap)
+int open_lanes(syg_ctx* ctx) {
+    for (Lane& L : ctx->lanes)
+        if (!L.stream) CK(cudaStreamCreateWithFlags(&L.stream, cudaStreamNonBlocking));
+    return SYG_OK;
+}
+
+// H2D of samples [b, e) of a host payload to L.in as float32 mono.  A PCM payload crosses PCIe as it is (fewer bytes) and is
+// de-interleaved, averaged and widened on the device.  The lane's previous chunk has left its device buffers when this chunk's work
+// reaches them (same stream => ordered).
+int upload_samples(syg_ctx* ctx, Lane& L, const void* y_host, InFmt inf, long long b, long long e) {
     const size_t fb = inf.frame_bytes();
+    if (int rc = L.in.ensure(std::max<size_t>((size_t)(e - b) * sizeof(float), 256))) return rc;
+    if (e <= b) return SYG_OK;
+    const unsigned char* src = reinterpret_cast<const unsigned char*>(y_host) + (size_t)b * fb;
+    if (inf.fmt < 0) {
+        CK(cudaMemcpyAsync(L.in.p, src, (size_t)(e - b) * fb, cudaMemcpyHostToDevice, L.stream));
+        return SYG_OK;
+    }
+    if (int rc = L.raw.ensure((size_t)(e - b) * fb)) return rc;
+    CK(cudaMemcpyAsync(L.raw.p, src, (size_t)(e - b) * fb, cudaMemcpyHostToDevice, L.stream));
+    std::string err;
+    ProfScope ps(ctx, L.stream, PROF_OTHER);
+    return launch_rc(syglaunch::pcm_to_f32(L.raw.p, inf.fmt, inf.channels, e - b, reinterpret_cast<float*>(L.in.p), ctx->sm_count,
+                                           L.stream, err), err);
+}
+
+// Unit tables of `bytes` to dev on st through the lane's pinned staging block, after `fill` has written their host image there.  The
+// block is rewritten only after the copy that read it last has completed (an event wait that has practically always passed), so the
+// streams never stall.
+template <class Fill>
+int stage_tables(Lane& L, size_t bytes, void* dev, cudaStream_t st, Fill fill) {
+    if (!L.tbl_done) CK(cudaEventCreateWithFlags(&L.tbl_done, cudaEventDisableTiming));
+    if (L.tbl_used) CK(cudaEventSynchronize(L.tbl_done));
+    if (int rc = L.tbl.ensure(bytes)) return rc;
+    fill(L.tbl.p);
+    CK(cudaMemcpyAsync(dev, L.tbl.p, bytes, cudaMemcpyHostToDevice, st));
+    CK(cudaEventRecord(L.tbl_done, st));
+    L.tbl_used = true;
+    return SYG_OK;
+}
+
+// Generic chunked host pipeline: H2D of the chunk's samples, `run(lane, y, g)` on the lane's stream with the chunk's samples on the
+// device and its geometry there, D2H of up to two outputs.  ws_per_unit bounds the chunk by the workspace limit; `run` sizes the
+// lane's workspace.
+template <class Run>
+int host_pipeline(syg_ctx* ctx, const void* y_host, InFmt inf, const syg_units* u, size_t out0_per_unit, void* out0_host,
+                  size_t out1_per_unit, void* out1_host, size_t ws_per_unit, long long max_chunk_units, Run run) {
     if (u->n_units == 0) return SYG_OK;
     const size_t in_target = (size_t)128 << 20, out_target = (size_t)256 << 20;
     long long span = u->unit_starts ? u->unit_len : std::max<long long>(1, std::min(u->unit_stride, u->unit_len));
@@ -720,72 +839,46 @@ int host_pipeline(syg_ctx* ctx, const void* y_host_any, InFmt inf, const syg_uni
     chunk = std::min(chunk, max_chunk_units);
     if (u->n_units > 1) chunk = std::min<long long>(chunk, (u->n_units + 1) / 2);           // keep both lanes busy
     chunk = std::max<long long>(chunk, 1);
-    for (int l = 0; l < 2; ++l) {
-        if (!ctx->lanes[l].stream) CK(cudaStreamCreateWithFlags(&ctx->lanes[l].stream, cudaStreamNonBlocking));
-        if (!ctx->lanes[l].tbl_done) CK(cudaEventCreateWithFlags(&ctx->lanes[l].tbl_done, cudaEventDisableTiming));
-    }
+    int rc = open_lanes(ctx);
+    if (rc) return rc;
     int li = 0;
     for (long long u0 = 0; u0 < u->n_units; u0 += chunk, li ^= 1) {
         const long long n = std::min(chunk, u->n_units - u0);
         Lane& L = ctx->lanes[li];
         long long b, e;
         chunk_range(u, u0, n, &b, &e);
-        int rc;
-        if ((rc = L.in.ensure(std::max<size_t>((size_t)(e - b) * sizeof(float), 256)))) return rc;
+        if ((rc = upload_samples(ctx, L, y_host, inf, b, e))) return rc;
         if ((rc = L.out0.ensure(std::max<size_t>(out0_per_unit * n, 256)))) return rc;
         if (out1_per_unit && (rc = L.out1.ensure(out1_per_unit * n))) return rc;
-        if (ws_per_unit && (rc = L.ws.ensure(ws_per_unit * n + 4096))) return rc;
-        // the lane's previous chunk has left its device buffers when this chunk's work reaches them (same stream => ordered)
-        if (e > b && inf.fmt < 0) CK(cudaMemcpyAsync(L.in.p, y_bytes + (size_t)b * fb, (size_t)(e - b) * fb, cudaMemcpyHostToDevice, L.stream));
-        if (e > b && inf.fmt >= 0) {                                    // PCM payload: fewer PCIe bytes; de-interleaved, averaged and widened on the device
-            if ((rc = L.raw.ensure((size_t)(e - b) * fb))) return rc;
-            CK(cudaMemcpyAsync(L.raw.p, y_bytes + (size_t)b * fb, (size_t)(e - b) * fb, cudaMemcpyHostToDevice, L.stream));
-            std::string err;
-            ProfScope ps(ctx, L.stream, PROF_OTHER);
-            const int crc = syglaunch::pcm_to_f32(L.raw.p, inf.fmt, inf.channels, e - b, reinterpret_cast<float*>(L.in.p), ctx->sm_count, L.stream, err);
-            if (crc) return fail(crc, "%s", err.c_str());
-        }
-        syg_units cu;
-        cu.n_units = n;
-        cu.unit_len = u->unit_len;
-        cu.unit_starts = nullptr;
-        cu.unit_valid = nullptr;
-        if (!u->unit_starts) {
-            // analytic starts continue inside the chunk: unit i of the chunk starts at (u0+i)*stride - b
-            cu.unit_stride = u->unit_stride;
-            cu.total_len = e - b;
-        } else {
-            // the chunk's table goes through the lane's own pinned staging block; it is rewritten only after the copy that read it
-            // two chunks ago has completed (an event wait that has practically always passed), so the streams never stall
-            const size_t off_valid = ((size_t)n * sizeof(long long) + 15) / 16 * 16;
-            if (L.tbl_used) CK(cudaEventSynchronize(L.tbl_done));
-            if ((rc = L.tbl.ensure(off_valid + (size_t)n * sizeof(int)))) return rc;
-            long long* rel = reinterpret_cast<long long*>(L.tbl.p);
-            int* val = reinterpret_cast<int*>(reinterpret_cast<char*>(L.tbl.p) + off_valid);
-            for (long long i = 0; i < n; ++i) {
-                const long long s = u->unit_starts[u0 + i];
-                long long v = u->unit_valid ? u->unit_valid[u0 + i] : u->total_len - s;
-                v = std::min<long long>(std::max<long long>(v, 0), u->unit_len);
-                rel[i] = v > 0 ? s - b : 0;
-                val[i] = (int)v;
-            }
-            if ((rc = L.starts.ensure(n * sizeof(long long)))) return rc;
-            if ((rc = L.valid.ensure(n * sizeof(int)))) return rc;
-            CK(cudaMemcpyAsync(L.starts.p, rel, n * sizeof(long long), cudaMemcpyHostToDevice, L.stream));
-            CK(cudaMemcpyAsync(L.valid.p, val, n * sizeof(int), cudaMemcpyHostToDevice, L.stream));
-            CK(cudaEventRecord(L.tbl_done, L.stream));
-            L.tbl_used = true;
-            cu.unit_stride = 0;
-            cu.total_len = e - b;
-            cu.unit_starts = reinterpret_cast<const int64_t*>(L.starts.p);
-            cu.unit_valid = reinterpret_cast<const int32_t*>(L.valid.p);
-        }
-        // analytic chunks: the kernel computes start = (u + unit0) * stride; shift the base pointer instead
-        const float* y_dev = reinterpret_cast<const float*>(L.in.p);
+        syg::UnitGeom g{};
+        g.n_units = n;
+        g.unit_len = u->unit_len;
         long long shift = 0;
-        if (!u->unit_starts) shift = u0 * u->unit_stride - b;        // >= 0: first unit's start relative to the chunk
-        rc = run(L, y_dev, cu, shift, u0, n);
-        if (rc) return rc;
+        if (!u->unit_starts) {
+            // analytic starts continue inside the chunk: the kernel computes start = u * stride (unit0 = 0), so the base pointer moves
+            // to the chunk's first unit, shift >= 0 samples past b
+            shift = u0 * u->unit_stride - b;
+            g.unit_stride = u->unit_stride;
+            g.total_len = e - b - shift;
+        } else {
+            // the chunk's own table, starts relative to b: int64 starts, then int32 valid lengths at a 16-byte boundary
+            const size_t off_valid = ((size_t)n * sizeof(long long) + 15) / 16 * 16, bytes = off_valid + (size_t)n * sizeof(int);
+            if ((rc = L.units.ensure(bytes))) return rc;
+            rc = stage_tables(L, bytes, L.units.p, L.stream, [&](void* h) {
+                long long* rel = reinterpret_cast<long long*>(h);
+                int* val = reinterpret_cast<int*>(reinterpret_cast<char*>(h) + off_valid);
+                for (long long i = 0; i < n; ++i) {
+                    const long long v = table_valid(u, u0 + i);
+                    rel[i] = v > 0 ? u->unit_starts[u0 + i] - b : 0;
+                    val[i] = (int)v;
+                }
+            });
+            if (rc) return rc;
+            g.total_len = e - b;
+            g.unit_starts = reinterpret_cast<const long long*>(L.units.p);
+            g.unit_valid = reinterpret_cast<const int*>(reinterpret_cast<char*>(L.units.p) + off_valid);
+        }
+        if ((rc = run(L, reinterpret_cast<const float*>(L.in.p) + shift, g))) return rc;
         CK(cudaMemcpyAsync(reinterpret_cast<char*>(out0_host) + (size_t)u0 * out0_per_unit, L.out0.p, out0_per_unit * n,
                            cudaMemcpyDeviceToHost, L.stream));
         if (out1_per_unit && out1_host)
@@ -794,19 +887,6 @@ int host_pipeline(syg_ctx* ctx, const void* y_host_any, InFmt inf, const syg_uni
     }
     for (int l = 0; l < 2; ++l) CK(cudaStreamSynchronize(ctx->lanes[l].stream));
     return SYG_OK;
-}
-
-// geometry of a host chunk on the device: analytic chunks keep (unit0 = 0) and fold the offset into the pointer
-syg::UnitGeom chunk_geom(const syg_units& cu, long long shift) {
-    syg::UnitGeom g;
-    g.n_units = cu.n_units;
-    g.unit_len = cu.unit_len;
-    g.unit_stride = cu.unit_stride;
-    g.total_len = cu.total_len - shift;     // samples available from the (shifted) base
-    g.unit_starts = reinterpret_cast<const long long*>(cu.unit_starts);
-    g.unit_valid = cu.unit_valid;
-    g.unit0 = 0;
-    return g;
 }
 
 int stft_setup(syg_ctx* ctx, const syg_units* u, int n_fft, int hop, int win_length, int window, int center, int pad_mode,
@@ -906,31 +986,27 @@ int check_ragged(const syg_ragged_units* u, int fl, int hop, int center, std::ve
     return SYG_OK;
 }
 
-size_t al256(size_t b) { return (b + 255) / 256 * 256; }
-
-// device tables of a ragged call, per unit: frame_off (int64, one more entry), starts (int64), lengths (int32), and for the
-// aggregation the unit's first frame relative to its chunk (int64) and its frame count (int32)
-size_t ragged_tbl_bytes(long long n, bool agg) {
-    return al256((size_t)(n + 1) * 8) + al256((size_t)n * 8) + al256((size_t)n * 4) + (agg ? al256((size_t)n * 8) + al256((size_t)n * 4) : 0);
-}
-struct RaggedTbl { long long* foff; long long* starts; int* valid; long long* seg_off; int* seg_len; };
-RaggedTbl ragged_tbl_at(void* base, long long n, bool agg) {
-    char* p = reinterpret_cast<char*>(base);
-    RaggedTbl t;
-    t.foff = reinterpret_cast<long long*>(p); p += al256((size_t)(n + 1) * 8);
-    t.starts = reinterpret_cast<long long*>(p); p += al256((size_t)n * 8);
-    t.valid = reinterpret_cast<int*>(p); p += al256((size_t)n * 4);
-    t.seg_off = agg ? reinterpret_cast<long long*>(p) : nullptr; p += agg ? al256((size_t)n * 8) : 0;
-    t.seg_len = agg ? reinterpret_cast<int*>(p) : nullptr;
+// the RaggedTbl of n units at base (with a null base only its size)
+RaggedTbl ragged_tbl(void* base, long long n, bool agg) {
+    Carve c{static_cast<char*>(base)};
+    RaggedTbl t{};
+    t.foff = c.take<long long>(n + 1);
+    t.starts = c.take<long long>(n);
+    t.valid = c.take<int>(n);
+    if (agg) {
+        t.seg_off = c.take<long long>(n);
+        t.seg_len = c.take<int>(n);
+    }
+    t.bytes = c.bytes;
     return t;
 }
-// workspace of a chunk of n units and nf frames: unit maxima, mel energies, contrast peaks / valleys, the frame table, and for
-// the aggregation the chunk's frame features [n_rows][nf]
-size_t ragged_ws_bytes(const FeaturePlan& pl, long long n, long long nf, bool agg) {
-    size_t b = al256((size_t)n * 4 * sizeof(unsigned)) + al256((size_t)nf * pl.fin.n_mels * sizeof(float)) +
-               al256((size_t)nf * 2 * pl.fin.nb * sizeof(float)) + al256((size_t)nf * sizeof(int4));
-    if (agg) b += al256((size_t)nf * pl.n_rows * sizeof(float));
-    return b + 256;
+
+// geometry of a ragged chunk of n units: the kernels take a unit's start and length from the frame table
+syg::UnitGeom ragged_geom(long long n) {
+    syg::UnitGeom g{};
+    g.n_units = n;
+    g.unit_len = 0x7fffffffLL;
+    return g;
 }
 
 struct RaggedChunk {
@@ -965,7 +1041,7 @@ void ragged_chunks(const syg_ragged_units* u, const std::vector<long long>& foff
         const long long T = foff[(size_t)i + 1] - foff[(size_t)i];
         const long long s = u->starts[i], l = u->lengths[i];
         const long long nb = l > 0 ? std::min(b, s) : b, ne = l > 0 ? std::max(e, s + l) : e;
-        if (c.n > 0 && (ragged_ws_bytes(pl, c.n + 1, c.nf + T, agg) > ws_limit || std::max(ne - nb, 0LL) > max_samples ||
+        if (c.n > 0 && (feat_ws(pl, c.n + 1, c.nf + T, true, agg).bytes > ws_limit || std::max(ne - nb, 0LL) > max_samples ||
                         c.nf + T > max_frames || c.n + 1 > 0x7fffffffLL)) {
             c.b = e > b ? b : 0; c.e = e > b ? e : 0;
             out.push_back(c);
@@ -979,74 +1055,6 @@ void ragged_chunks(const syg_ragged_units* u, const std::vector<long long>& foff
         c.nf += T;
     }
     if (c.n > 0) { c.b = e > b ? b : 0; c.e = e > b ? e : 0; out.push_back(c); }
-}
-
-// the feature kernels on one chunk: y and the tables are chunk-relative, rows go to out[r * out_stride + f] (f < nf)
-int run_ragged_chunk(syg_ctx* ctx, const FeaturePlan& pl, const float* y, const RaggedTbl& t, long long n, long long nf, float* out,
-                     long long out_stride, void* ws, int n_fft, cudaStream_t st) {
-    syg::FrameArgs a = pl.fa;
-    a.y = y;
-    a.g.n_units = n;
-    a.g.unit_len = 0x7fffffffLL;           // the kernels take a unit's start and length from the frame table
-    a.g.unit_stride = 0;
-    a.g.total_len = 0;
-    a.g.unit_starts = nullptr;
-    a.g.unit_valid = nullptr;
-    a.g.unit0 = 0;
-    a.T = 0;
-    a.n_frames = nf;
-    a.out = out;
-    a.ragged_stride = out_stride;
-    a.res_units = 0;                       // the unit-resident epilogue sizes its tile by units x T: uniform launches only
-    char* w = reinterpret_cast<char*>(ws);
-    a.unit_max = reinterpret_cast<unsigned*>(w);
-    size_t off = al256((size_t)n * 4 * sizeof(unsigned));
-    a.melws = reinterpret_cast<float*>(w + off);
-    off += al256((size_t)nf * pl.fin.n_mels * sizeof(float));
-    a.cws = reinterpret_cast<float*>(w + off);
-    off += al256((size_t)nf * 2 * pl.fin.nb * sizeof(float));
-    int4* ut = reinterpret_cast<int4*>(w + off);
-    a.ragged_ut = ut;
-    g_last_features_resident = 0;
-    g_last_feature_frames += nf;
-    if (a.mask & syg::FB_MFCC) g_last_mel_form = a.mel_iv ? 1 : 0;
-    if (nf == 0) return SYG_OK;            // only units without frames: nothing to compute (and no zero-CTA finalize launch)
-    std::string err;
-    {
-        ProfScope ps(ctx, st, PROF_OTHER);
-        if (int trc = syglaunch::ragged_frame_table(t.foff, t.starts, t.valid, n, nf, ut, ctx->sm_count, st, err)) return fail(trc, "%s", err.c_str());
-    }
-    const bool need_fin = (a.mask & (syg::FB_MFCC | syg::FB_CONTRAST)) != 0;
-    if (need_fin) CK(cudaMemsetAsync(a.unit_max, 0, (size_t)n * 4 * sizeof(unsigned), st));
-    if (a.mask & syg::FB_TIME_EXTRA) {
-        ProfScope ps(ctx, st, PROF_FRAME);
-        if (int trc = syglaunch::time_extra(a, n_fft, pl.entropy_bins, ctx->sm_count, st, err)) return fail(trc, "%s", err.c_str());
-    }
-    if ((a.mask & ~syg::FB_TIME_EXTRA) == 0) return SYG_OK;
-    {
-        ProfScope ps(ctx, st, PROF_FRAME);
-        if (int rc = launch_features(n_fft, a, ctx->sm_count, st)) return rc;
-    }
-    if (!need_fin) return SYG_OK;
-    ProfScope ps(ctx, st, PROF_FINALIZE);
-    syg::FinalizeArgs f = pl.fin;
-    f.n_units = n;
-    f.T = 0;
-    f.melws = a.melws;
-    f.cws = a.cws;
-    f.unit_max = a.unit_max;
-    f.out = out;
-    f.ragged_ut = ut;
-    f.n_frames = nf;
-    f.ragged_stride = out_stride;
-    return launch_finalize(ctx, f, nf, st);
-}
-
-int check_agg(const FeaturePlan& pl, const int32_t* agg) {
-    if (pl.n_rows > 64) return fail(SYG_E_UNSUPPORTED, "aggregation supports at most 64 rows per call");
-    for (int i = 0; i < pl.n_rows; ++i)
-        if (agg[i] < SYG_AGG_MEAN || agg[i] > SYG_AGG_MAX) return fail(SYG_E_BADARG, "unknown aggregation id %d", agg[i]);
-    return SYG_OK;
 }
 
 // agg == nullptr: out is float32 [n_rows][F]; else float64 [n_units][n_rows]
@@ -1071,38 +1079,25 @@ int ragged_dev_impl(syg_ctx* ctx, const float* y_dev, const syg_ragged_units* un
     std::vector<RaggedChunk> chunks;
     ragged_chunks(units, foff, pl, ag, ctx->ws_limit, 0x7fffffffLL, 1LL << 62, chunks);     // starts < 2^31 in the frame table
     size_t ws_max = 0;
-    for (const RaggedChunk& c : chunks) ws_max = std::max(ws_max, ragged_ws_bytes(pl, c.n, c.nf, ag));
-    const size_t tbl_bytes = ragged_tbl_bytes(n_units, ag);
-    // the tables of all units go through lane 0's pinned staging block in one copy; the block is rewritten only after the copy that
-    // read it last has completed
-    Lane& L = ctx->lanes[0];
-    if (!L.tbl_done) CK(cudaEventCreateWithFlags(&L.tbl_done, cudaEventDisableTiming));
-    if (L.tbl_used) CK(cudaEventSynchronize(L.tbl_done));
-    if ((rc = L.tbl.ensure(tbl_bytes))) return rc;
-    const RaggedTbl ht = ragged_tbl_at(L.tbl.p, n_units, ag);
-    for (const RaggedChunk& c : chunks) ragged_tbl_fill(ht, c.u0, units, foff, c);
-    if (ctx->ws_done) CK(cudaStreamWaitEvent(st, ctx->ws_done, 0));
-    else CK(cudaEventCreateWithFlags(&ctx->ws_done, cudaEventDisableTiming));
-    if (tbl_bytes + ws_max > ctx->ws.cap) CK(cudaStreamSynchronize(st));   // growing frees the old block: nothing may still use it
-    if ((rc = ctx->ws.ensure(tbl_bytes + ws_max))) return rc;
-    struct Done { syg_ctx* c; cudaStream_t s; ~Done() { cudaEventRecord(c->ws_done, s); } } done_{ctx, st};
-    CK(cudaMemcpyAsync(ctx->ws.p, L.tbl.p, tbl_bytes, cudaMemcpyHostToDevice, st));
-    CK(cudaEventRecord(L.tbl_done, st));
-    L.tbl_used = true;
-    const RaggedTbl dt = ragged_tbl_at(ctx->ws.p, n_units, ag);
-    void* ws = reinterpret_cast<char*>(ctx->ws.p) + tbl_bytes;
+    for (const RaggedChunk& c : chunks) ws_max = std::max(ws_max, feat_ws(pl, c.n, c.nf, true, ag).bytes);
+    // the workspace holds the tables of all units, then the workspace of the chunk in flight
+    const size_t tbl_bytes = ragged_tbl(nullptr, n_units, ag).bytes;
+    WsClaim ws{ctx, st};
+    if ((rc = ws.claim(tbl_bytes + ws_max))) return rc;
+    rc = stage_tables(ctx->lanes[0], tbl_bytes, ctx->ws.p, st, [&](void* h) {          // one copy through lane 0's staging block
+        const RaggedTbl ht = ragged_tbl(h, n_units, ag);
+        for (const RaggedChunk& c : chunks) ragged_tbl_fill(ht, c.u0, units, foff, c);
+    });
+    if (rc) return rc;
+    const RaggedTbl dt = ragged_tbl(ctx->ws.p, n_units, ag);
     for (const RaggedChunk& c : chunks) {
-        RaggedTbl ct{dt.foff + c.u0, dt.starts + c.u0, dt.valid + c.u0, ag ? dt.seg_off + c.u0 : nullptr, ag ? dt.seg_len + c.u0 : nullptr};
-        float* feat = ag ? reinterpret_cast<float*>(reinterpret_cast<char*>(ws) + ragged_ws_bytes(pl, c.n, c.nf, true) - 256 -
-                                                    al256((size_t)c.nf * pl.n_rows * sizeof(float)))
-                         : reinterpret_cast<float*>(out_dev) + c.f0;
-        if ((rc = run_ragged_chunk(ctx, pl, y_dev + c.b, ct, c.n, c.nf, feat, ag ? c.nf : F, ws, p->frame_length, st))) return rc;
-        if (!ag) continue;
-        std::string err;
-        ProfScope ps(ctx, st, PROF_OTHER);
-        const int arc = syglaunch::aggregate(feat, c.n, pl.n_rows, c.nf, ct.seg_off, ct.seg_len, 0, agg,
-                                             reinterpret_cast<double*>(out_dev) + (size_t)c.u0 * pl.n_rows, ctx->sm_count, st, err);
-        if (arc) return fail(arc, "%s", err.c_str());
+        RaggedTbl ct{dt.foff + c.u0, dt.starts + c.u0, dt.valid + c.u0, ag ? dt.seg_off + c.u0 : nullptr, ag ? dt.seg_len + c.u0 : nullptr, 0};
+        const FeatWs w = feat_ws(pl, c.n, c.nf, true, ag, reinterpret_cast<char*>(ctx->ws.p) + tbl_bytes);
+        float* feat = ag ? w.feat : reinterpret_cast<float*>(out_dev) + c.f0;
+        if ((rc = run_features_chunk(ctx, pl, y_dev + c.b, ragged_geom(c.n), &ct, c.nf, ag ? c.nf : F, feat, w, st))) return rc;
+        if (ag && (rc = launch_aggregate(ctx, pl, feat, c.n, c.nf, ct.seg_off, ct.seg_len, 0, agg,
+                                         reinterpret_cast<double*>(out_dev) + (size_t)c.u0 * pl.n_rows, st)))
+            return rc;
     }
     return SYG_OK;
 }
@@ -1131,41 +1126,27 @@ int ragged_host_impl(syg_ctx* ctx, const float* y_host, const syg_ragged_units* 
     if (n_units > 1) max_frames = std::min<long long>(max_frames, std::max<long long>(1, (F + 1) / 2));
     std::vector<RaggedChunk> chunks;
     ragged_chunks(units, foff, pl, ag, ctx->ws_limit, (long long)(((size_t)128 << 20) / sizeof(float)), max_frames, chunks);
-    for (int l = 0; l < 2; ++l) {
-        if (!ctx->lanes[l].stream) CK(cudaStreamCreateWithFlags(&ctx->lanes[l].stream, cudaStreamNonBlocking));
-        if (!ctx->lanes[l].tbl_done) CK(cudaEventCreateWithFlags(&ctx->lanes[l].tbl_done, cudaEventDisableTiming));
-    }
+    if ((rc = open_lanes(ctx))) return rc;
     int li = 0;
     for (const RaggedChunk& c : chunks) {
         Lane& L = ctx->lanes[li];
         li ^= 1;
-        const size_t tbl_bytes = ragged_tbl_bytes(c.n, ag);
+        // the lane's workspace holds the chunk's tables, then the chunk's feature workspace
+        const size_t tbl_bytes = ragged_tbl(nullptr, c.n, ag).bytes;
         const size_t out_bytes = ag ? (size_t)c.n * pl.n_rows * sizeof(double) : (size_t)c.nf * pl.n_rows * sizeof(float);
-        if ((rc = L.in.ensure(std::max<size_t>((size_t)(c.e - c.b) * sizeof(float), 256)))) return rc;
+        if ((rc = upload_samples(ctx, L, y_host, InFmt{}, c.b, c.e))) return rc;
         if ((rc = L.out0.ensure(std::max<size_t>(out_bytes, 256)))) return rc;
-        if ((rc = L.ws.ensure(tbl_bytes + ragged_ws_bytes(pl, c.n, c.nf, ag)))) return rc;
-        // the lane's previous chunk has left its device buffers when this chunk's work reaches them (same stream => ordered)
-        if (c.e > c.b) CK(cudaMemcpyAsync(L.in.p, y_host + c.b, (size_t)(c.e - c.b) * sizeof(float), cudaMemcpyHostToDevice, L.stream));
-        if (L.tbl_used) CK(cudaEventSynchronize(L.tbl_done));
-        if ((rc = L.tbl.ensure(tbl_bytes))) return rc;
-        ragged_tbl_fill(ragged_tbl_at(L.tbl.p, c.n, ag), 0, units, foff, c);
-        CK(cudaMemcpyAsync(L.ws.p, L.tbl.p, tbl_bytes, cudaMemcpyHostToDevice, L.stream));
-        CK(cudaEventRecord(L.tbl_done, L.stream));
-        L.tbl_used = true;
-        const RaggedTbl ct = ragged_tbl_at(L.ws.p, c.n, ag);
-        void* ws = reinterpret_cast<char*>(L.ws.p) + tbl_bytes;
-        float* feat = ag ? reinterpret_cast<float*>(reinterpret_cast<char*>(ws) + ragged_ws_bytes(pl, c.n, c.nf, true) - 256 -
-                                                    al256((size_t)c.nf * pl.n_rows * sizeof(float)))
-                         : reinterpret_cast<float*>(L.out0.p);
-        if ((rc = run_ragged_chunk(ctx, pl, reinterpret_cast<const float*>(L.in.p), ct, c.n, c.nf, feat, c.nf, ws, p->frame_length,
-                                   L.stream)))
-            return rc;
+        if ((rc = L.ws.ensure(tbl_bytes + feat_ws(pl, c.n, c.nf, true, ag).bytes))) return rc;
+        rc = stage_tables(L, tbl_bytes, L.ws.p, L.stream, [&](void* h) { ragged_tbl_fill(ragged_tbl(h, c.n, ag), 0, units, foff, c); });
+        if (rc) return rc;
+        const RaggedTbl ct = ragged_tbl(L.ws.p, c.n, ag);
+        const FeatWs w = feat_ws(pl, c.n, c.nf, true, ag, reinterpret_cast<char*>(L.ws.p) + tbl_bytes);
+        float* feat = ag ? w.feat : reinterpret_cast<float*>(L.out0.p);
+        const float* y_dev = reinterpret_cast<const float*>(L.in.p);
+        if ((rc = run_features_chunk(ctx, pl, y_dev, ragged_geom(c.n), &ct, c.nf, c.nf, feat, w, L.stream))) return rc;
         if (ag) {
-            std::string err;
-            ProfScope ps(ctx, L.stream, PROF_OTHER);
-            const int arc = syglaunch::aggregate(feat, c.n, pl.n_rows, c.nf, ct.seg_off, ct.seg_len, 0, agg,
-                                                 reinterpret_cast<double*>(L.out0.p), ctx->sm_count, L.stream, err);
-            if (arc) return fail(arc, "%s", err.c_str());
+            if ((rc = launch_aggregate(ctx, pl, feat, c.n, c.nf, ct.seg_off, ct.seg_len, 0, agg, reinterpret_cast<double*>(L.out0.p), L.stream)))
+                return rc;
             CK(cudaMemcpyAsync(reinterpret_cast<double*>(out_host) + (size_t)c.u0 * pl.n_rows, L.out0.p, out_bytes, cudaMemcpyDeviceToHost,
                                L.stream));
         } else {
@@ -1220,7 +1201,7 @@ void syg_ctx_destroy(syg_ctx* ctx) {
     ctx->ws.release();
     if (ctx->ws_done) cudaEventDestroy(ctx->ws_done);
     for (auto& l : ctx->lanes) {
-        l.in.release(); l.raw.release(); l.out0.release(); l.out1.release(); l.starts.release(); l.valid.release(); l.ws.release(); l.feat.release();
+        l.in.release(); l.raw.release(); l.out0.release(); l.out1.release(); l.units.release(); l.ws.release();
         l.tbl.release();
         if (l.tbl_done) cudaEventDestroy(l.tbl_done);
         if (l.stream) cudaStreamDestroy(l.stream);
@@ -1300,10 +1281,9 @@ int64_t syg_frame_count(int64_t n_samples, int32_t frame_length, int32_t hop_len
     return 1 + (n - frame_length) / hop_length;
 }
 
-int syg_features_f32(syg_ctx* ctx, const float* y_dev, const syg_units* units, const syg_feature_params* p,
-                     float* out_dev, void* stream) {
-    SYG_TRACE();
-    g_last_feature_frames = 0;
+// agg == nullptr: out_dev is float32 [n_units][n_rows][T];  else: float64 [n_units][n_rows] (per-row SYG_AGG_* over the frames)
+static int features_dev_impl(syg_ctx* ctx, const float* y_dev, const syg_units* units, const syg_feature_params* p, const int32_t* agg,
+                             void* out_dev, cudaStream_t st) {
     if (!ctx) return fail(SYG_E_BADARG, "ctx is NULL");
     int rc = check_units(units);
     if (rc) return rc;
@@ -1314,23 +1294,31 @@ int syg_features_f32(syg_ctx* ctx, const float* y_dev, const syg_units* units, c
     if (units->n_units == 0 || pl.T <= 0 || pl.n_rows == 0) return SYG_OK;
     if (!y_dev && units->total_len > 0) return fail(SYG_E_BADARG, "y_dev is NULL");
     if (!out_dev) return fail(SYG_E_BADARG, "out_dev is NULL");
-    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-    long long chunk = std::max<long long>(1, (long long)(ctx->ws_limit / std::max<size_t>(pl.ws_per_unit, 1)));
+    if (agg && (rc = check_agg(pl, agg))) return rc;
+    // aggregated calls keep the frame features of a chunk in the workspace: [chunk][rows][T] never reaches the caller
+    const bool ag = agg != nullptr;
+    const size_t feat_per_unit = ag ? (size_t)pl.n_rows * pl.T * sizeof(float) : 0;
+    long long chunk = std::max<long long>(1, (long long)(ctx->ws_limit / std::max<size_t>(pl.ws_per_unit + feat_per_unit, 1)));
     chunk = std::min<long long>(chunk, units->n_units);
-    // the workspace is shared by every call on this context: order this call's kernels behind the previous user's, whatever
-    // stream that was (calls on ONE stream are ordered anyway; two streams would otherwise overwrite each other's mel energies)
-    if (ctx->ws_done) CK(cudaStreamWaitEvent(st, ctx->ws_done, 0));
-    else CK(cudaEventCreateWithFlags(&ctx->ws_done, cudaEventDisableTiming));
-    if (features_ws_bytes(pl, chunk) > ctx->ws.cap) CK(cudaStreamSynchronize(st));   // growing frees the old block: nothing may still use it
-    if ((rc = ctx->ws.ensure(features_ws_bytes(pl, chunk)))) return rc;
-    struct Done { syg_ctx* c; cudaStream_t s; ~Done() { cudaEventRecord(c->ws_done, s); } } done_{ctx, st};
+    WsClaim ws{ctx, st};
+    if ((rc = ws.claim(feat_ws(pl, chunk, chunk * pl.T, false, ag).bytes))) return rc;
     for (long long u0 = 0; u0 < units->n_units; u0 += chunk) {
         const long long n = std::min(chunk, units->n_units - u0);
-        syg::UnitGeom g = geom_of(units, u0, n);
-        rc = run_features_chunk(ctx, pl, y_dev, g, out_dev + (size_t)u0 * pl.n_rows * pl.T, ctx->ws.p, p->frame_length, st);
-        if (rc) return rc;
+        const FeatWs w = feat_ws(pl, n, n * pl.T, false, ag, ctx->ws.p);
+        float* feat = ag ? w.feat : reinterpret_cast<float*>(out_dev) + (size_t)u0 * pl.n_rows * pl.T;
+        if ((rc = run_features_chunk(ctx, pl, y_dev, geom_of(units, u0, n), nullptr, n * pl.T, 0, feat, w, st))) return rc;
+        if (ag && (rc = launch_aggregate(ctx, pl, feat, n, pl.T, nullptr, nullptr, pl.T, agg,
+                                         reinterpret_cast<double*>(out_dev) + (size_t)u0 * pl.n_rows, st)))
+            return rc;
     }
     return SYG_OK;
+}
+
+int syg_features_f32(syg_ctx* ctx, const float* y_dev, const syg_units* units, const syg_feature_params* p,
+                     float* out_dev, void* stream) {
+    SYG_TRACE();
+    g_last_feature_frames = 0;
+    return features_dev_impl(ctx, y_dev, units, p, nullptr, out_dev, reinterpret_cast<cudaStream_t>(stream));
 }
 
 // agg == nullptr: out_host is float32 [n_units][n_rows][T];  else: float64 [n_units][n_rows] (per-row SYG_AGG_* over the frames)
@@ -1350,33 +1338,23 @@ static int features_host_impl(syg_ctx* ctx, const void* y_host, InFmt inf, const
     if (units->n_units == 0 || pl.T <= 0 || pl.n_rows == 0) return SYG_OK;
     if (!y_host && units->total_len > 0) return fail(SYG_E_BADARG, "y_host is NULL");
     if (!out_host) return fail(SYG_E_BADARG, "out_host is NULL");
-    if (agg) {
-        if (pl.n_rows > 64) return fail(SYG_E_UNSUPPORTED, "aggregation supports at most 64 rows per call");
-        for (int i = 0; i < pl.n_rows; ++i)
-            if (agg[i] < SYG_AGG_MEAN || agg[i] > SYG_AGG_MAX) return fail(SYG_E_BADARG, "unknown aggregation id %d", agg[i]);
-    }
+    if (agg && (rc = check_agg(pl, agg))) return rc;
+    const bool ag = agg != nullptr;
     const size_t feat_per_unit = (size_t)pl.n_rows * pl.T * sizeof(float);
-    const size_t out_per_unit = agg ? (size_t)pl.n_rows * sizeof(double) : feat_per_unit;
-    const int n_fft = p->frame_length;
-    // aggregated calls keep the [n, rows, T] block on the device: bound the chunk by it (it replaces the D2H-sized output buffer)
-    const long long max_chunk = agg ? std::max<long long>(1, (long long)(((size_t)256 << 20) / feat_per_unit)) : (1LL << 40);
-    return host_pipeline(ctx, y_host, inf, units, out_per_unit, out_host, 0, nullptr, features_ws_bytes(pl, 1), max_chunk,
-                         [&](Lane& L, const float* y_dev, const syg_units& cu, long long shift, long long, long long n) -> int {
-                             int r = L.ws.ensure(features_ws_bytes(pl, n));
+    const size_t out_per_unit = ag ? (size_t)pl.n_rows * sizeof(double) : feat_per_unit;
+    // aggregated calls keep the [n, rows, T] block in the lane's workspace: bound the chunk by it (it replaces the D2H-sized output)
+    const long long max_chunk = ag ? std::max<long long>(1, (long long)(((size_t)256 << 20) / feat_per_unit)) : (1LL << 40);
+    return host_pipeline(ctx, y_host, inf, units, out_per_unit, out_host, 0, nullptr, feat_ws(pl, 1, pl.T, false, false).bytes, max_chunk,
+                         [&](Lane& L, const float* y_dev, const syg::UnitGeom& g) -> int {
+                             const long long n = g.n_units;
+                             int r = L.ws.ensure(feat_ws(pl, n, n * pl.T, false, ag).bytes);
                              if (r) return r;
-                             float* feat = reinterpret_cast<float*>(L.out0.p);
-                             if (agg) {
-                                 if ((r = L.feat.ensure(feat_per_unit * n))) return r;
-                                 feat = reinterpret_cast<float*>(L.feat.p);
-                             }
-                             syg::UnitGeom g = chunk_geom(cu, shift);
-                             r = run_features_chunk(ctx, pl, y_dev + shift, g, feat, L.ws.p, n_fft, L.stream);
-                             if (r || !agg) return r;
-                             std::string err;
-                             ProfScope ps(ctx, L.stream, PROF_OTHER);
-                             const int arc = syglaunch::aggregate(feat, n, pl.n_rows, pl.T, nullptr, nullptr, pl.T, agg,
-                                                                  reinterpret_cast<double*>(L.out0.p), ctx->sm_count, L.stream, err);
-                             return arc ? fail(arc, "%s", err.c_str()) : SYG_OK;
+                             const FeatWs w = feat_ws(pl, n, n * pl.T, false, ag, L.ws.p);
+                             float* feat = ag ? w.feat : reinterpret_cast<float*>(L.out0.p);
+                             r = run_features_chunk(ctx, pl, y_dev, g, nullptr, n * pl.T, 0, feat, w, L.stream);
+                             if (r || !ag) return r;
+                             return launch_aggregate(ctx, pl, feat, n, pl.T, nullptr, nullptr, pl.T, agg, reinterpret_cast<double*>(L.out0.p),
+                                                     L.stream);
                          });
 }
 
@@ -1411,43 +1389,8 @@ int syg_segment_vectors_f32(syg_ctx* ctx, const float* y_dev, const syg_units* u
                             const int32_t* agg, double* out_dev, void* stream) {
     SYG_TRACE();
     g_last_feature_frames = 0;
-    if (!ctx) return fail(SYG_E_BADARG, "ctx is NULL");
-    if (!agg) return fail(SYG_E_BADARG, "agg is NULL");
-    int rc = check_units(units);
-    if (rc) return rc;
-    std::lock_guard<std::mutex> lk(ctx->mu);
-    ENTER_DEVICE(ctx);
-    FeaturePlan pl;
-    if ((rc = build_feature_plan(ctx, units, p, pl))) return rc;
-    if (units->n_units == 0 || pl.T <= 0 || pl.n_rows == 0) return SYG_OK;
-    if (!y_dev && units->total_len > 0) return fail(SYG_E_BADARG, "y_dev is NULL");
-    if (!out_dev) return fail(SYG_E_BADARG, "out_dev is NULL");
-    if (pl.n_rows > 64) return fail(SYG_E_UNSUPPORTED, "aggregation supports at most 64 rows per call");
-    for (int i = 0; i < pl.n_rows; ++i)
-        if (agg[i] < SYG_AGG_MEAN || agg[i] > SYG_AGG_MAX) return fail(SYG_E_BADARG, "unknown aggregation id %d", agg[i]);
-    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-    // the frame features of a chunk live in a library-owned block behind the workspace: [chunk][rows][T] never reaches the caller
-    const size_t feat_per_unit = (size_t)pl.n_rows * pl.T * sizeof(float);
-    long long chunk = std::max<long long>(1, (long long)(ctx->ws_limit / std::max<size_t>(pl.ws_per_unit + feat_per_unit, 1)));
-    chunk = std::min<long long>(chunk, units->n_units);
-    const size_t ws_bytes = (features_ws_bytes(pl, chunk) + 255) / 256 * 256;
-    if (ctx->ws_done) CK(cudaStreamWaitEvent(st, ctx->ws_done, 0));
-    else CK(cudaEventCreateWithFlags(&ctx->ws_done, cudaEventDisableTiming));
-    if (ws_bytes + feat_per_unit * chunk > ctx->ws.cap) CK(cudaStreamSynchronize(st));
-    if ((rc = ctx->ws.ensure(ws_bytes + feat_per_unit * chunk))) return rc;
-    struct Done { syg_ctx* c; cudaStream_t s; ~Done() { cudaEventRecord(c->ws_done, s); } } done_{ctx, st};
-    float* feat = reinterpret_cast<float*>(reinterpret_cast<char*>(ctx->ws.p) + ws_bytes);
-    for (long long u0 = 0; u0 < units->n_units; u0 += chunk) {
-        const long long n = std::min(chunk, units->n_units - u0);
-        syg::UnitGeom g = geom_of(units, u0, n);
-        if ((rc = run_features_chunk(ctx, pl, y_dev, g, feat, ctx->ws.p, p->frame_length, st))) return rc;
-        std::string err;
-        ProfScope ps(ctx, st, PROF_OTHER);
-        const int arc = syglaunch::aggregate(feat, n, pl.n_rows, pl.T, nullptr, nullptr, pl.T, agg, out_dev + (size_t)u0 * pl.n_rows,
-                                             ctx->sm_count, st, err);
-        if (arc) return fail(arc, "%s", err.c_str());
-    }
-    return SYG_OK;
+    if (ctx && !agg) return fail(SYG_E_BADARG, "agg is NULL");           // a NULL ctx is reported first
+    return features_dev_impl(ctx, y_dev, units, p, agg, out_dev, reinterpret_cast<cudaStream_t>(stream));
 }
 
 int64_t syg_ragged_frame_offsets(const syg_ragged_units* units, int32_t frame_length, int32_t hop_length, int32_t center,
@@ -1498,9 +1441,8 @@ int syg_ingest_pcm(syg_ctx* ctx, const void* raw_dev, int32_t sample_format, int
     if (sample_format < SYG_PCM_U8 || sample_format > SYG_PCM_F32) return fail(SYG_E_BADARG, "unknown PCM sample format %d", sample_format);
     ENTER_DEVICE(ctx);
     std::string err;
-    const int rc = syglaunch::pcm_to_f32(raw_dev, sample_format, channels, n_frames, mono_dev, ctx->sm_count,
-                                         reinterpret_cast<cudaStream_t>(stream), err);
-    return rc ? fail(rc, "%s", err.c_str()) : SYG_OK;
+    return launch_rc(syglaunch::pcm_to_f32(raw_dev, sample_format, channels, n_frames, mono_dev, ctx->sm_count,
+                                           reinterpret_cast<cudaStream_t>(stream), err), err);
 }
 
 int syg_pcm16_to_f32(syg_ctx* ctx, const int16_t* in_dev, float* out_dev, int64_t n, void* stream) {
@@ -1509,9 +1451,8 @@ int syg_pcm16_to_f32(syg_ctx* ctx, const int16_t* in_dev, float* out_dev, int64_
     if (n < 0 || (n > 0 && (!in_dev || !out_dev))) return fail(SYG_E_BADARG, "bad pcm16 buffer");
     ENTER_DEVICE(ctx);
     std::string err;
-    const int rc = syglaunch::pcm16_to_f32(reinterpret_cast<const short*>(in_dev), out_dev, n, ctx->sm_count,
-                                           reinterpret_cast<cudaStream_t>(stream), err);
-    return rc ? fail(rc, "%s", err.c_str()) : SYG_OK;
+    return launch_rc(syglaunch::pcm16_to_f32(reinterpret_cast<const short*>(in_dev), out_dev, n, ctx->sm_count,
+                                             reinterpret_cast<cudaStream_t>(stream), err), err);
 }
 
 static size_t stft_elem_bytes(int out_kind) { return out_kind == SYG_OUT_COMPLEX ? 2 * sizeof(float) : sizeof(float); }
@@ -1555,11 +1496,11 @@ int syg_stft_host_f32(syg_ctx* ctx, const float* y_host, const syg_units* units,
     const size_t out_per_unit = (size_t)(n_fft / 2 + 1) * a.T * stft_elem_bytes(out_kind);
     const int sm = ctx->sm_count;
     return host_pipeline(ctx, y_host, InFmt{}, units, out_per_unit, out_host, 0, nullptr, 0, 1LL << 40,
-                         [&](Lane& L, const float* y_dev, const syg_units& cu, long long shift, long long, long long n) -> int {
+                         [&](Lane& L, const float* y_dev, const syg::UnitGeom& g) -> int {
                              syg::FrameArgs c = a;
-                             c.y = y_dev + shift;
-                             c.g = chunk_geom(cu, shift);
-                             c.n_frames = n * (long long)a.T;
+                             c.y = y_dev;
+                             c.g = g;
+                             c.n_frames = g.n_units * (long long)a.T;
                              c.stft_out = L.out0.p;
                              return launch_stft(n_fft, c, sm, L.stream);
                          });
@@ -1603,10 +1544,10 @@ int syg_psd_welch_host_f32(syg_ctx* ctx, const float* y_host, const syg_units* u
     const size_t st_per_unit = stats_host ? 3 * sizeof(float) : 0;
     const int sm = ctx->sm_count;
     return host_pipeline(ctx, y_host, InFmt{}, units, psd_per_unit, psd_host, st_per_unit, stats_host, 0, 1LL << 40,
-                         [&](Lane& L, const float* y_dev, const syg_units& cu, long long shift, long long, long long) -> int {
+                         [&](Lane& L, const float* y_dev, const syg::UnitGeom& g) -> int {
                              syg::WelchArgs c = pl.wa;
-                             c.y = y_dev + shift;
-                             c.g = chunk_geom(cu, shift);
+                             c.y = y_dev;
+                             c.g = g;
                              c.psd = reinterpret_cast<float*>(L.out0.p);
                              c.stats = st_per_unit ? reinterpret_cast<float*>(L.out1.p) : nullptr;
                              return launch_welch(pl.nfft, c, sm, L.stream);
@@ -1625,9 +1566,8 @@ int syg_aggregate_f32(syg_ctx* ctx, const float* feats_dev, int64_t n_seg, int32
         if (agg[i] < SYG_AGG_MEAN || agg[i] > SYG_AGG_MAX) return fail(SYG_E_BADARG, "unknown aggregation id %d", agg[i]);
     ENTER_DEVICE(ctx);
     std::string err;
-    const int rc = syglaunch::aggregate(feats_dev, n_seg, n_rows, row_stride, reinterpret_cast<const long long*>(seg_off_dev), seg_len_dev,
-                                        fixed_len, agg, out_dev, ctx->sm_count, reinterpret_cast<cudaStream_t>(stream), err);
-    return rc ? fail(rc, "%s", err.c_str()) : SYG_OK;
+    return launch_rc(syglaunch::aggregate(feats_dev, n_seg, n_rows, row_stride, reinterpret_cast<const long long*>(seg_off_dev), seg_len_dev,
+                                          fixed_len, agg, out_dev, ctx->sm_count, reinterpret_cast<cudaStream_t>(stream), err), err);
 }
 
 int64_t syg_segment_count(int64_t total_samples, double sr, double segment_length_sec, double overlap_ratio,
@@ -1670,8 +1610,8 @@ int syg_mfcc_from_logmel_f64(syg_ctx* ctx, const double* S_dev, int64_t n_units,
     int rc = upload_table(ctx, dk, dct, &d_dct);
     if (rc) return rc;
     std::string err;
-    rc = syglaunch::dct_matrix(S_dev, d_dct, n_units, n_mels, T, C, out_dev, ctx->sm_count, reinterpret_cast<cudaStream_t>(stream), err);
-    return rc ? fail(rc, "%s", err.c_str()) : SYG_OK;
+    return launch_rc(syglaunch::dct_matrix(S_dev, d_dct, n_units, n_mels, T, C, out_dev, ctx->sm_count, reinterpret_cast<cudaStream_t>(stream),
+                                           err), err);
 }
 
 int syg_spectral_contrast_from_mag_f32(syg_ctx* ctx, const float* S_dev, int32_t n_bins, int64_t T, double sr, int32_t n_bands,
@@ -1690,26 +1630,20 @@ int syg_spectral_contrast_from_mag_f32(syg_ctx* ctx, const float* S_dev, int32_t
     for (int i = 0; i < b.nb; ++i) nq[i] = std::max(1, std::min(b.nq[i], std::max(b.cnt[i], 1)));
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
     // workspace: unit maxima (one "unit" = the whole matrix: power_to_db clamps 80 dB below the array maximum) + linear peaks / valleys
-    const size_t need = 256 + (size_t)T * 2 * b.nb * sizeof(float);
-    if (ctx->ws_done) CK(cudaStreamWaitEvent(st, ctx->ws_done, 0));
-    else CK(cudaEventCreateWithFlags(&ctx->ws_done, cudaEventDisableTiming));
-    if (need > ctx->ws.cap) CK(cudaStreamSynchronize(st));
-    int rc = ctx->ws.ensure(need);
+    WsClaim ws{ctx, st};
+    int rc = ws.claim(256 + (size_t)T * 2 * b.nb * sizeof(float));
     if (rc) return rc;
-    struct Done { syg_ctx* c; cudaStream_t s; ~Done() { cudaEventRecord(c->ws_done, s); } } done_{ctx, st};
     unsigned* um = reinterpret_cast<unsigned*>(ctx->ws.p);
     float* cws = reinterpret_cast<float*>(reinterpret_cast<char*>(ctx->ws.p) + 256);
     CK(cudaMemsetAsync(um, 0, 4 * sizeof(unsigned), st));
-    rc = syglaunch::contrast_spectrum(S_dev, n_bins, T, b.nb, b.lo, b.cnt, nq, cws, um, ctx->sm_count, st, err);
-    if (rc) return fail(rc, "%s", err.c_str());
+    if ((rc = launch_rc(syglaunch::contrast_spectrum(S_dev, n_bins, T, b.nb, b.lo, b.cnt, nq, cws, um, ctx->sm_count, st, err), err))) return rc;
     syg::FinalizeArgs f;
     std::memset(&f, 0, sizeof(f));
     f.n_units = 1; f.T = (int)T; f.n_rows = b.nb; f.row_mfcc = -1; f.nb = b.nb; f.row_contrast = 0; f.amin = 1e-10f; f.top_db = 80.0f;
     f.cws = cws; f.unit_max = um; f.out = out_dev;
     if (T > 0x7fffffffLL) return fail(SYG_E_UNSUPPORTED, "too many frames");
     const long long n_tiles = (T + sygdev::kFinTT - 1) / sygdev::kFinTT;
-    rc = syglaunch::finalize(f, sygdev::kFinTT, (unsigned)std::min<long long>(n_tiles, 0x7fffffffLL), 1u, 256, st, err);
-    return rc ? fail(rc, "%s", err.c_str()) : SYG_OK;
+    return launch_rc(syglaunch::finalize(f, sygdev::kFinTT, (unsigned)std::min<long long>(n_tiles, 0x7fffffffLL), 1u, 256, st, err), err);
 }
 
 int syg_debug_last_stft_path(void) { return syglaunch::g_last.stft_path; }
