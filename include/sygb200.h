@@ -124,7 +124,9 @@ int syg_ctx_set_workspace_limit(syg_ctx* ctx, size_t bytes);
 int syg_ctx_sm_count(const syg_ctx* ctx);
 /* optional per-kernel timing for bench.py: CUDA events around every kernel launch on the launching stream.
  * read: ms[4] / launches[4] = {frame kernel (FFT + features or STFT), finalize kernel, welch kernel, other (ingest +
- * aggregation)}, summed since the last reset; synchronises on the recorded events. */
+ * aggregation)}, summed since the last reset; synchronises on the recorded events.  Not timed: the STFT and Welch launches of
+ * syg_stft_host_f32 and syg_psd_welch_host_f32.  syg_psd_welch_host_pcm_channels times its ingest and Welch launches, one of
+ * each per chunk. */
 int syg_ctx_profile_enable(syg_ctx* ctx, int on);
 int syg_ctx_profile_read(syg_ctx* ctx, double* ms, int64_t* launches, int reset);
 
@@ -160,6 +162,27 @@ int syg_ingest_pcm(syg_ctx* ctx, const void* raw_dev, int32_t sample_format, int
  * FRAMES of the payload (one frame = `channels` samples = one mono sample after the mix-down). */
 int syg_features_host_pcm(syg_ctx* ctx, const void* raw_host, int32_t sample_format, int32_t channels, const syg_units* units,
                           const syg_feature_params* p, float* out_host);
+
+/* Per-channel forms: load_audio(file, sr=None, mono=False) (sygnals/core/audio/io.py:38-102 -> librosa.load, (channels, n)) for
+ * the payload of a WAV 'data' chunk, with the normalisation of syg_ingest_pcm and no mix-down.  channels in [1, 64].
+ * syg_ingest_pcm_channels: interleaved payload in HBM -> float32 planes out_dev[c * pitch + i], i < n_frames, with pitch = n_frames
+ * rounded up to a multiple of 4 (every plane starts 16-byte aligned); the pad words between planes are not written.  raw_dev may
+ * have any byte alignment.
+ * syg_psd_welch_host_pcm_channels: syg_psd_welch_host_f32 per (unit, channel) of a host PCM payload; `units` count frames and apply
+ * to every channel.  psd_host [n_units][channels][1 + nfft/2], stats_host (optional) [n_units][channels][3].
+ * syg_segment_vectors_host_pcm_channels: syg_segment_vectors_host_pcm without the mix-down: out_host [n_units][channels][n_rows].
+ * Each (unit, channel) result equals, bit for bit, the float32 host form on that channel's samples.  The raw bytes cross PCIe; one
+ * ingest launch and one Welch (or feature) launch serve every channel of a chunk.  Errors: SYG_E_BADARG for channels outside
+ * [1, 64], an unknown format, a NULL pointer or a unit outside the payload (nothing is written); plan errors as the float32 forms;
+ * n_units = 0: nothing to do. */
+int syg_ingest_pcm_channels(syg_ctx* ctx, const void* raw_dev, int32_t sample_format, int32_t channels, int64_t n_frames,
+                            float* out_dev, void* stream);
+int syg_psd_welch_host_pcm_channels(syg_ctx* ctx, const void* raw_host, int32_t sample_format, int32_t channels,
+                                    const syg_units* units, double fs, int32_t window, int32_t nperseg, int32_t noverlap,
+                                    int32_t nfft, int32_t detrend_constant, int32_t scaling, float* psd_host, float* stats_host);
+int syg_segment_vectors_host_pcm_channels(syg_ctx* ctx, const void* raw_host, int32_t sample_format, int32_t channels,
+                                          const syg_units* units, const syg_feature_params* p, const int32_t* agg,
+                                          double* out_host);
 
 /* Segment vectors: extract_features() per unit followed by format_feature_vectors_per_segment() (sygnals/core/ml_utils/
  * formatters.py:51-163, the consumer in `sygnals save dataset`, sygnals/cli/save_cmd.py:140-190) with every unit as one segment:

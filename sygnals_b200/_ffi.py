@@ -108,6 +108,9 @@ class Library:
             "syg_pcm16_to_f32": (C.c_int, [vp, vp, vp, i64, vp]),
             "syg_ingest_pcm": (C.c_int, [vp, vp, i32, i32, i64, vp, vp]),
             "syg_features_host_pcm": (C.c_int, [vp, vp, i32, i32, PU, PP, vp]),
+            "syg_ingest_pcm_channels": (C.c_int, [vp, vp, i32, i32, i64, vp, vp]),
+            "syg_psd_welch_host_pcm_channels": (C.c_int, [vp, vp, i32, i32, PU, f64, i32, i32, i32, i32, i32, i32, vp, vp]),
+            "syg_segment_vectors_host_pcm_channels": (C.c_int, [vp, vp, i32, i32, PU, PP, vp, vp]),
             "syg_segment_vectors_f32": (C.c_int, [vp, vp, PU, PP, vp, vp, vp]),
             "syg_segment_vectors_host_f32": (C.c_int, [vp, vp, PU, PP, vp, vp]),
             "syg_segment_vectors_host_pcm": (C.c_int, [vp, vp, i32, i32, PU, PP, vp, vp]),
@@ -289,6 +292,17 @@ def make_params(lib: Library, sr: int, features: Sequence[str], frame_length: in
     return p
 
 
+def plane_pitch(n_frames: int) -> int:
+    """Floats between the planes of ``syg_ingest_pcm_channels``: ``n_frames`` rounded up to a multiple of 4."""
+    return (int(n_frames) + 3) // 4 * 4
+
+
+def _check_out(a, shape, dtype, what: str) -> None:
+    """A caller's preallocated result must be exactly what the library writes: the D2H copies trust its size and layout."""
+    if not isinstance(a, np.ndarray) or a.dtype != dtype or a.shape != tuple(shape) or not a.flags.c_contiguous or not a.flags.writeable:
+        raise ValueError(f"{what} must be a writeable C-contiguous {np.dtype(dtype).name} array of shape {tuple(shape)}")
+
+
 def _f32c(a) -> np.ndarray:
     return np.ascontiguousarray(a, dtype=np.float32)
 
@@ -442,6 +456,46 @@ class Engine:
     def ingest_pcm_dev(self, raw_ptr: int, fmt: int, channels: int, n_frames: int, out_ptr: int, stream: int = 0) -> None:
         """Interleaved PCM in HBM -> mono float32 in HBM (load_audio(mono=True) arithmetic)."""
         self.lib.check(self.lib.dll.syg_ingest_pcm(self._h, raw_ptr, int(fmt), int(channels), int(n_frames), out_ptr, stream or None))
+
+    def ingest_pcm_channels_dev(self, raw_ptr: int, fmt: int, channels: int, n_frames: int, out_ptr: int, stream: int = 0) -> None:
+        """Interleaved PCM in HBM -> float32 planes ``out[c * plane_pitch(n_frames) + i]`` in HBM (load_audio(mono=False))."""
+        self.lib.check(self.lib.dll.syg_ingest_pcm_channels(self._h, raw_ptr, int(fmt), int(channels), int(n_frames), out_ptr,
+                                                            stream or None))
+
+    def psd_welch_host_pcm_channels(self, raw_ptr: int, fmt: int, channels: int, units: SygUnits, fs: float, window: int, nperseg: int,
+                                    noverlap: int, nfft: int, detrend: bool = True, scaling: int = 0, stats: bool = False,
+                                    out: Optional[tuple] = None):
+        """Welch PSD per (unit, channel) of an interleaved PCM payload in host memory (``units`` count frames): psd
+        ``[n_units, channels, 1 + nfft/2]`` float32 and, with ``stats``, ``[n_units, channels, 3]`` (rms, crest, peak).  ``out``:
+        optional preallocated (psd, stats) arrays of those shapes (e.g. ``pinned_empty``)."""
+        nfft_eff = nfft if nfft and nfft > 0 else nperseg
+        n, ch = int(units.n_units), int(channels)
+        if out is None:
+            out = (np.empty((n, ch, nfft_eff // 2 + 1), dtype=np.float32), np.empty((n, ch, 3), dtype=np.float32) if stats else None)
+        psd, st = out
+        _check_out(psd, (n, ch, nfft_eff // 2 + 1), np.float32, "out[0]")
+        if stats:
+            _check_out(st, (n, ch, 3), np.float32, "out[1]")
+        else:
+            st = None
+        self.lib.check(self.lib.dll.syg_psd_welch_host_pcm_channels(
+            self._h, raw_ptr, int(fmt), ch, C.byref(units), float(fs), int(window), int(nperseg), int(noverlap), int(nfft_eff),
+            int(bool(detrend)), int(scaling), psd.ctypes.data, st.ctypes.data if st is not None else None))
+        return (psd, st) if stats else psd
+
+    def segment_vectors_host_pcm_channels(self, raw_ptr: int, fmt: int, channels: int, units: SygUnits, p: SygFeatureParams,
+                                          agg_ids: Sequence[int], out: Optional[np.ndarray] = None) -> np.ndarray:
+        """float64 ``[n_units, channels, n_rows]``: ``segment_vectors_host`` per channel of an interleaved PCM payload, no mix-down."""
+        rows = self.rows(p)
+        if len(agg_ids) != rows:
+            raise ValueError("one aggregation id per feature row")
+        if out is None:
+            out = np.empty((int(units.n_units), int(channels), rows), dtype=np.float64)
+        _check_out(out, (int(units.n_units), int(channels), rows), np.float64, "out")
+        agg = (C.c_int32 * max(1, rows))(*[int(a) for a in agg_ids])
+        self.lib.check(self.lib.dll.syg_segment_vectors_host_pcm_channels(self._h, raw_ptr, int(fmt), int(channels), C.byref(units),
+                                                                          C.byref(p), C.addressof(agg), out.ctypes.data))
+        return out
 
     def stft_host(self, y: np.ndarray, units: SygUnits, n_fft: int, hop: int, win_length: int, window: int = 0,
                   center: bool = True, pad_mode: int = 0, out_kind: int = OUT_COMPLEX, out: Optional[np.ndarray] = None) -> np.ndarray:

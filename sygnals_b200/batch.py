@@ -7,6 +7,10 @@
                                   -- clips of different lengths (a folder of files, variable-length segments) in one launch,
                                      each clip framed on its own: no padding to the longest
 * :func:`stft_batch`, :func:`psd_welch_batch`
+* :func:`channel_psd`, :func:`channel_vectors`
+                                  -- per-channel Welch PSDs / segment vectors of a multi-channel PCM recording (a WAV file or
+                                     a :class:`Payload`, BASELINE cfg5 shape): the interleaved bytes cross PCIe as they are and
+                                     are de-interleaved on the device
 
 Inputs may be numpy arrays (host path: chunked H2D / kernels / D2H inside the library) or CUDA ``torch`` tensors (device
 path: asynchronous on the current torch stream, result stays in HBM).  Row naming follows manager.py:337-343,365-369.
@@ -264,3 +268,69 @@ def psd_welch_batch(windows, fs: float, nperseg: int = 1024, noverlap: Optional[
         return (psd, st) if stats else psd
     return eng.psd_welch_host(np.ascontiguousarray(windows, dtype=np.float32).reshape(-1), units, fs, wid, nperseg, noverlap, nfft,
                               detrend, sid, stats=stats)
+
+
+class Payload(NamedTuple):
+    """An interleaved PCM payload in host memory: ``raw`` the bytes (a numpy array or any buffer), ``fmt`` one of ``_ffi.PCM_*``,
+    ``channels`` samples per frame, ``sample_rate`` in Hz."""
+    raw: object
+    fmt: int
+    channels: int
+    sample_rate: int
+
+
+def _pcm_source(source):
+    """(uint8 array, fmt, channels, frames, sample_rate) of a WAV path (memory-mapped payload) or a :class:`Payload`."""
+    if isinstance(source, Payload):
+        if _is_torch(source.raw):
+            raise ValueError("Payload.raw must be host memory (numpy array or buffer)")
+        raw = source.raw if isinstance(source.raw, np.ndarray) else np.frombuffer(source.raw, dtype=np.uint8)
+        raw = np.ascontiguousarray(raw).view(np.uint8).reshape(-1)
+        fmt, ch, sr = int(source.fmt), int(source.channels), int(source.sample_rate)
+        if fmt not in _ffi.PCM_BYTES:
+            raise ValueError(f"unknown PCM sample format {fmt}")
+        if not 1 <= ch <= 64:
+            raise ValueError(f"channels={ch}: supported range is [1, 64]")
+        return raw, fmt, ch, raw.size // (ch * _ffi.PCM_BYTES[fmt]), sr
+    from .core.audio import io as sio
+    info = sio.wav_info(source)
+    raw, frames = sio.wav_payload(info)
+    return raw, info.fmt, info.channels, frames, info.sample_rate
+
+
+def channel_psd(source, window_sec: float = 1.0, overlap_ratio: float = 0.0, pad: bool = True, nperseg: int = 1024,
+                noverlap: Optional[int] = None, nfft: Optional[int] = None, window: str = "hann", detrend: bool = True,
+                scaling: str = "density", stats: bool = True, device: Optional[int] = None) -> Dict[str, object]:
+    """Welch PSD per (window, channel) of a multi-channel PCM recording (BASELINE cfg5: a machinery monitor's WAV / DAQ payload).
+    ``source``: a WAV path (memory-mapped) or a :class:`Payload` in host memory.  Windows follow ``segment_fixed_length``
+    (segmentation.py:62-114) over the frames; each (window, channel) is ``compute_psd_welch`` of that channel's samples.
+    Returns {'freqs', 'psd' float32 ``[n_windows, channels, 1 + nfft/2]``, 'stats' float32 ``[n_windows, channels, 3]`` (rms, crest
+    factor, peak; None without ``stats``), 'starts', 'valid', 'sample_rate'}."""
+    raw, fmt, ch, frames, sr = _pcm_source(source)
+    eng = _ffi.engine(device)
+    seg_len, _, starts, valid = eng.lib.segment_table(frames, sr, window_sec, overlap_ratio, pad)
+    nfft = nperseg if nfft is None else nfft
+    noverlap = nperseg // 2 if noverlap is None else noverlap
+    if window.lower() not in _ffi.WINDOW_IDS:
+        raise NotImplementedError(f"window={window!r}")
+    units = eng.units_table(starts.ctypes.data, valid.ctypes.data, len(starts), seg_len, frames)
+    res = eng.psd_welch_host_pcm_channels(raw.ctypes.data, fmt, ch, units, sr, _ffi.WINDOW_IDS[window.lower()], nperseg, noverlap,
+                                          nfft, detrend, _ffi.SCALING_IDS[scaling], stats=stats)
+    psd, st = res if stats else (res, None)
+    return {"freqs": np.fft.rfftfreq(nfft, d=1.0 / sr), "psd": psd, "stats": st, "starts": starts, "valid": valid, "sample_rate": sr}
+
+
+def channel_vectors(source, segment_length_sec: float, features: Sequence[str], aggregation="mean", overlap_ratio: float = 0.0,
+                    pad: bool = True, frame_length: int = 2048, hop_length: int = 512, center: bool = True, window: str = "hann",
+                    feature_params: Optional[dict] = None, device: Optional[int] = None):
+    """One vector per (segment, channel) of a multi-channel PCM recording: ``extract_features`` per segment of each channel followed
+    by ``format_feature_vectors_per_segment`` (``aggregation`` a name or a per-row dict, formatters.py:39-45).  ``source`` as in
+    :func:`channel_psd`.  Returns (row names, float64 ``[n_segments, channels, rows]``)."""
+    raw, fmt, ch, frames, sr = _pcm_source(source)
+    eng = _ffi.engine(device)
+    seg_len, _, starts, valid = eng.lib.segment_table(frames, sr, segment_length_sec, overlap_ratio, pad)
+    p = _ffi.make_params(eng.lib, sr, list(features), frame_length, hop_length, center, window, feature_params)
+    names = feature_row_names(features, feature_params)
+    from .core.ml_utils.formatters import _agg_ids
+    units = eng.units_table(starts.ctypes.data, valid.ctypes.data, len(starts), seg_len, frames)
+    return names, eng.segment_vectors_host_pcm_channels(raw.ctypes.data, fmt, ch, units, p, _agg_ids(names, aggregation))

@@ -3,8 +3,9 @@
 Mirror of ``sygnals/core/audio/io.py:38-102`` (``load_audio`` -> ``librosa.load`` -> ``soundfile.read(dtype='float32')`` +
 ``librosa.to_mono``) for RIFF/WAVE files.  The header is parsed here on the host; the payload (the bytes of the ``data`` chunk)
 goes to the GPU as it lies in the file and ``libsygb200`` de-interleaves, normalises and mixes it down there
-(``syg_ingest_pcm`` / ``syg_features_host_pcm`` / ``syg_segment_vectors_host_pcm``), so a 16-bit recording crosses PCIe at
-2 bytes per sample instead of the reference's 8 (float64).
+(``syg_ingest_pcm`` / ``syg_features_host_pcm`` / ``syg_segment_vectors_host_pcm``), or keeps one plane per channel
+(``syg_ingest_pcm_channels`` for ``mono=False``), so a 16-bit recording crosses PCIe at 2 bytes per sample instead of the
+reference's 8 (float64).
 
 Not served here (they stay on the reference path): compressed formats, and resampling (``sr`` different from the file's rate).
 """
@@ -106,13 +107,8 @@ def load_audio(file_path: Union[str, os.PathLike], sr: Optional[int] = None, mon
         raise NotImplementedError(f"sr={sr}: resampling (native rate {info.sample_rate}) stays on the reference path")
     raw, frames = wav_payload(info, offset, duration)
     if not mono and info.channels > 1:
-        # (n_channels, n_samples) like librosa: every channel is an independent mono ingest of a strided view
-        out = np.empty((info.channels, frames), dtype=np.float64)
-        inter = raw.reshape(frames, info.frame_bytes)
-        bps = _ffi.PCM_BYTES[info.fmt]
-        for c in range(info.channels):
-            out[c] = pcm_to_mono(np.ascontiguousarray(inter[:, c * bps:(c + 1) * bps]).reshape(-1), info.fmt, 1, device)
-        return out, info.sample_rate
+        # (n_channels, n_samples) like librosa
+        return pcm_to_planes(raw, info.fmt, info.channels, device).astype(np.float64), info.sample_rate
     return pcm_to_mono(raw, info.fmt, info.channels, device).astype(np.float64), info.sample_rate
 
 
@@ -130,3 +126,21 @@ def pcm_to_mono(raw: np.ndarray, fmt: int, channels: int, device: Optional[int] 
     d_out = torch.empty(frames, dtype=torch.float32, device=dev)
     eng.ingest_pcm_dev(d_raw.data_ptr(), fmt, channels, frames, d_out.data_ptr(), torch.cuda.current_stream(dev).cuda_stream)
     return d_out.cpu().numpy()
+
+
+def pcm_to_planes(raw: np.ndarray, fmt: int, channels: int, device: Optional[int] = None) -> np.ndarray:
+    """Interleaved PCM bytes (uint8 array) -> float32 ``(channels, frames)`` on the GPU: one H2D copy of the payload, one
+    ``syg_ingest_pcm_channels`` launch, one D2H copy of the planes."""
+    import torch
+    raw = np.ascontiguousarray(raw).view(np.uint8).reshape(-1)
+    fb = channels * _ffi.PCM_BYTES[fmt]
+    frames = raw.size // fb
+    if frames == 0:
+        return np.zeros((channels, 0), dtype=np.float32)
+    eng = _ffi.engine(device)
+    dev = torch.device("cuda", eng.device)
+    pitch = _ffi.plane_pitch(frames)
+    d_raw = torch.from_numpy(raw[: frames * fb]).to(dev)
+    d_out = torch.empty(channels * pitch, dtype=torch.float32, device=dev)
+    eng.ingest_pcm_channels_dev(d_raw.data_ptr(), fmt, channels, frames, d_out.data_ptr(), torch.cuda.current_stream(dev).cuda_stream)
+    return d_out.cpu().numpy().reshape(channels, pitch)[:, :frames]

@@ -109,9 +109,13 @@ struct Lane {                      // one in-flight chunk of a *_host_* call
     bool tbl_used = false;
 };
 
-// what a *_host_* call is handed: float32 mono samples (fmt < 0) or an interleaved PCM payload (SYG_PCM_*, `channels` per frame)
+// what a *_host_* call is handed: float32 mono samples (fmt < 0) or an interleaved PCM payload (SYG_PCM_*, `channels` per frame).
+// planes: the payload's channels are kept apart, one float32 plane per channel, and every unit of the call is computed once per
+// channel (device unit w * channels + c); otherwise a PCM payload is mixed down to mono.
 struct InFmt {
     int fmt = -1, channels = 1;
+    bool planes = false;
+    long long units_per_unit() const { return planes ? channels : 1; }
     size_t frame_bytes() const {
         if (fmt < 0) return sizeof(float);
         const size_t bps = fmt == SYG_PCM_U8 ? 1 : (fmt == SYG_PCM_S16 ? 2 : (fmt == SYG_PCM_S24 ? 3 : 4));
@@ -143,8 +147,8 @@ namespace {
 enum { PROF_FRAME = 0, PROF_FINALIZE = 1, PROF_WELCH = 2, PROF_OTHER = 3 };   // other = ingest + aggregation
 struct ProfScope {
     syg_ctx* c; cudaStream_t st; int kind; cudaEvent_t a = nullptr, b = nullptr;
-    ProfScope(syg_ctx* c_, cudaStream_t st_, int kind_) : c(c_), st(st_), kind(kind_) {
-        if (c->prof_on && cudaEventCreate(&a) == cudaSuccess && cudaEventCreate(&b) == cudaSuccess) cudaEventRecord(a, st);
+    ProfScope(syg_ctx* c_, cudaStream_t st_, int kind_) : c(c_), st(st_), kind(kind_) {   // kind < 0: not timed
+        if (kind >= 0 && c->prof_on && cudaEventCreate(&a) == cudaSuccess && cudaEventCreate(&b) == cudaSuccess) cudaEventRecord(a, st);
         else a = b = nullptr;
     }
     ~ProfScope() {
@@ -751,6 +755,13 @@ long long table_valid(const syg_units* u, long long i) {
     return std::min<long long>(std::max<long long>(v, 0), u->unit_len);
 }
 
+// start and valid length of unit i, analytic or from the table (the kernels' arithmetic: valid clamped to [0, unit_len])
+void unit_span(const syg_units* u, long long i, long long* start, long long* valid) {
+    if (u->unit_starts) { *start = u->unit_starts[i]; *valid = table_valid(u, i); return; }
+    *start = i * u->unit_stride;
+    *valid = std::min<long long>(std::max<long long>(u->total_len - *start, 0), u->unit_len);
+}
+
 // sample range needed by units [u0, u0 + n)
 void chunk_range(const syg_units* u, long long u0, long long n, long long* begin, long long* end) {
     if (!u->unit_starts) {
@@ -789,12 +800,17 @@ int open_lanes(syg_ctx* ctx) {
     return SYG_OK;
 }
 
-// H2D of samples [b, e) of a host payload to L.in as float32 mono.  A PCM payload crosses PCIe as it is (fewer bytes) and is
-// de-interleaved, averaged and widened on the device.  The lane's previous chunk has left its device buffers when this chunk's work
-// reaches them (same stream => ordered).
+// a plane of n samples: rounded up to 4 floats, so that every plane of a lane's input starts 16-byte aligned
+long long plane_pitch(long long n) { return (n + 3) / 4 * 4; }
+
+// H2D of samples [b, e) of a host payload to L.in as float32 mono, or with inf.planes as one float32 plane per channel,
+// L.in[c * plane_pitch(e - b) + i].  A PCM payload crosses PCIe as it is (fewer bytes) and is de-interleaved, averaged (mono) and
+// widened on the device.  The lane's previous chunk has left its device buffers when this chunk's work reaches them (same stream =>
+// ordered).
 int upload_samples(syg_ctx* ctx, Lane& L, const void* y_host, InFmt inf, long long b, long long e) {
     const size_t fb = inf.frame_bytes();
-    if (int rc = L.in.ensure(std::max<size_t>((size_t)(e - b) * sizeof(float), 256))) return rc;
+    const size_t in_floats = inf.planes ? (size_t)inf.channels * plane_pitch(e - b) : (size_t)(e - b);
+    if (int rc = L.in.ensure(std::max<size_t>(in_floats * sizeof(float), 256))) return rc;
     if (e <= b) return SYG_OK;
     const unsigned char* src = reinterpret_cast<const unsigned char*>(y_host) + (size_t)b * fb;
     if (inf.fmt < 0) {
@@ -805,8 +821,11 @@ int upload_samples(syg_ctx* ctx, Lane& L, const void* y_host, InFmt inf, long lo
     CK(cudaMemcpyAsync(L.raw.p, src, (size_t)(e - b) * fb, cudaMemcpyHostToDevice, L.stream));
     std::string err;
     ProfScope ps(ctx, L.stream, PROF_OTHER);
-    return launch_rc(syglaunch::pcm_to_f32(L.raw.p, inf.fmt, inf.channels, e - b, reinterpret_cast<float*>(L.in.p), ctx->sm_count,
-                                           L.stream, err), err);
+    float* in = reinterpret_cast<float*>(L.in.p);
+    if (inf.planes)
+        return launch_rc(syglaunch::pcm_to_planes(L.raw.p, inf.fmt, inf.channels, e - b, plane_pitch(e - b), in, ctx->sm_count, L.stream,
+                                                  err), err);
+    return launch_rc(syglaunch::pcm_to_f32(L.raw.p, inf.fmt, inf.channels, e - b, in, ctx->sm_count, L.stream, err), err);
 }
 
 // Unit tables of `bytes` to dev on st through the lane's pinned staging block, after `fill` has written their host image there.  The
@@ -825,18 +844,23 @@ int stage_tables(Lane& L, size_t bytes, void* dev, cudaStream_t st, Fill fill) {
 }
 
 // Generic chunked host pipeline: H2D of the chunk's samples, `run(lane, y, g)` on the lane's stream with the chunk's samples on the
-// device and its geometry there, D2H of up to two outputs.  ws_per_unit bounds the chunk by the workspace limit; `run` sizes the
-// lane's workspace.
+// device and its geometry there, D2H of up to two outputs.  The sizes per unit and max_chunk_units count device units; with
+// inf.planes every unit of u is C = inf.channels device units (one per channel), a chunk is a range of units across all channels and
+// its budgets are multiplied by C.  ws_per_unit bounds the chunk by the workspace limit; `run` sizes the lane's workspace.
 template <class Run>
 int host_pipeline(syg_ctx* ctx, const void* y_host, InFmt inf, const syg_units* u, size_t out0_per_unit, void* out0_host,
                   size_t out1_per_unit, void* out1_host, size_t ws_per_unit, long long max_chunk_units, Run run) {
     if (u->n_units == 0) return SYG_OK;
+    const long long C = inf.units_per_unit();
+    out0_per_unit *= C;
+    out1_per_unit *= C;
+    ws_per_unit *= C;
     const size_t in_target = (size_t)128 << 20, out_target = (size_t)256 << 20;
     long long span = u->unit_starts ? u->unit_len : std::max<long long>(1, std::min(u->unit_stride, u->unit_len));
-    long long chunk = std::max<long long>(1, (long long)(in_target / (std::max<long long>(span, 1) * sizeof(float))));
+    long long chunk = std::max<long long>(1, (long long)(in_target / (std::max<long long>(span, 1) * sizeof(float) * C)));
     if (out0_per_unit + out1_per_unit) chunk = std::min<long long>(chunk, std::max<long long>(1, (long long)(out_target / (out0_per_unit + out1_per_unit))));
     if (ws_per_unit) chunk = std::min<long long>(chunk, std::max<long long>(1, (long long)(ctx->ws_limit / ws_per_unit)));
-    chunk = std::min(chunk, max_chunk_units);
+    chunk = std::min(chunk, std::max<long long>(1, max_chunk_units / C));
     if (u->n_units > 1) chunk = std::min<long long>(chunk, (u->n_units + 1) / 2);           // keep both lanes busy
     chunk = std::max<long long>(chunk, 1);
     int rc = open_lanes(ctx);
@@ -851,30 +875,35 @@ int host_pipeline(syg_ctx* ctx, const void* y_host, InFmt inf, const syg_units* 
         if ((rc = L.out0.ensure(std::max<size_t>(out0_per_unit * n, 256)))) return rc;
         if (out1_per_unit && (rc = L.out1.ensure(out1_per_unit * n))) return rc;
         syg::UnitGeom g{};
-        g.n_units = n;
+        g.n_units = n * C;
         g.unit_len = u->unit_len;
         long long shift = 0;
-        if (!u->unit_starts) {
+        if (!u->unit_starts && !inf.planes) {
             // analytic starts continue inside the chunk: the kernel computes start = u * stride (unit0 = 0), so the base pointer moves
             // to the chunk's first unit, shift >= 0 samples past b
             shift = u0 * u->unit_stride - b;
             g.unit_stride = u->unit_stride;
             g.total_len = e - b - shift;
         } else {
-            // the chunk's own table, starts relative to b: int64 starts, then int32 valid lengths at a 16-byte boundary
-            const size_t off_valid = ((size_t)n * sizeof(long long) + 15) / 16 * 16, bytes = off_valid + (size_t)n * sizeof(int);
+            // the chunk's own table, starts relative to b: int64 starts, then int32 valid lengths at a 16-byte boundary.  Device unit
+            // i * C + c is channel c of unit u0 + i, whose plane starts at c * pitch (C = 1: the mono buffer, pitch unused).
+            const long long m = n * C, pitch = plane_pitch(e - b);
+            const size_t off_valid = ((size_t)m * sizeof(long long) + 15) / 16 * 16, bytes = off_valid + (size_t)m * sizeof(int);
             if ((rc = L.units.ensure(bytes))) return rc;
             rc = stage_tables(L, bytes, L.units.p, L.stream, [&](void* h) {
                 long long* rel = reinterpret_cast<long long*>(h);
                 int* val = reinterpret_cast<int*>(reinterpret_cast<char*>(h) + off_valid);
                 for (long long i = 0; i < n; ++i) {
-                    const long long v = table_valid(u, u0 + i);
-                    rel[i] = v > 0 ? u->unit_starts[u0 + i] - b : 0;
-                    val[i] = (int)v;
+                    long long s, v;
+                    unit_span(u, u0 + i, &s, &v);
+                    for (long long c = 0; c < C; ++c) {
+                        rel[i * C + c] = v > 0 ? c * pitch + s - b : 0;
+                        val[i * C + c] = (int)v;
+                    }
                 }
             });
             if (rc) return rc;
-            g.total_len = e - b;
+            g.total_len = (C - 1) * pitch + (e - b);
             g.unit_starts = reinterpret_cast<const long long*>(L.units.p);
             g.unit_valid = reinterpret_cast<const int*>(reinterpret_cast<char*>(L.units.p) + off_valid);
         }
@@ -1321,14 +1350,16 @@ int syg_features_f32(syg_ctx* ctx, const float* y_dev, const syg_units* units, c
     return features_dev_impl(ctx, y_dev, units, p, nullptr, out_dev, reinterpret_cast<cudaStream_t>(stream));
 }
 
-// agg == nullptr: out_host is float32 [n_units][n_rows][T];  else: float64 [n_units][n_rows] (per-row SYG_AGG_* over the frames)
+static bool pcm_layout_ok(InFmt inf) { return inf.fmt >= SYG_PCM_U8 && inf.fmt <= SYG_PCM_F32 && inf.channels >= 1 && inf.channels <= 64; }
+
+// agg == nullptr: out_host is float32 [n_units][n_rows][T];  else: float64 [n_units][n_rows] (per-row SYG_AGG_* over the frames).
+// inf.planes: [n_units][channels][...], one result per unit and channel.
 static int features_host_impl(syg_ctx* ctx, const void* y_host, InFmt inf, const syg_units* units, const syg_feature_params* p,
                               const int32_t* agg, void* out_host) {
     NvtxRange nvtx_range_(agg ? "syg_segment_vectors_host" : "syg_features_host");
     g_last_feature_frames = 0;
     if (!ctx) return fail(SYG_E_BADARG, "ctx is NULL");
-    if (inf.fmt >= 0 && (inf.fmt > SYG_PCM_F32 || inf.channels < 1 || inf.channels > 64))
-        return fail(SYG_E_BADARG, "bad PCM layout (format %d, %d channels)", inf.fmt, inf.channels);
+    if ((inf.fmt >= 0 || inf.planes) && !pcm_layout_ok(inf)) return fail(SYG_E_BADARG, "bad PCM layout (format %d, %d channels)", inf.fmt, inf.channels);
     int rc = check_host_units(units);
     if (rc) return rc;
     std::lock_guard<std::mutex> lk(ctx->mu);
@@ -1383,6 +1414,12 @@ int syg_segment_vectors_host_pcm(syg_ctx* ctx, const void* raw_host, int32_t sam
                                  const syg_units* units, const syg_feature_params* p, const int32_t* agg, double* out_host) {
     if (!agg) return fail(SYG_E_BADARG, "agg is NULL");
     return features_host_impl(ctx, raw_host, InFmt{sample_format, channels}, units, p, agg, out_host);
+}
+
+int syg_segment_vectors_host_pcm_channels(syg_ctx* ctx, const void* raw_host, int32_t sample_format, int32_t channels,
+                                          const syg_units* units, const syg_feature_params* p, const int32_t* agg, double* out_host) {
+    if (!agg) return fail(SYG_E_BADARG, "agg is NULL");
+    return features_host_impl(ctx, raw_host, InFmt{sample_format, channels, true}, units, p, agg, out_host);
 }
 
 int syg_segment_vectors_f32(syg_ctx* ctx, const float* y_dev, const syg_units* units, const syg_feature_params* p,
@@ -1443,6 +1480,20 @@ int syg_ingest_pcm(syg_ctx* ctx, const void* raw_dev, int32_t sample_format, int
     std::string err;
     return launch_rc(syglaunch::pcm_to_f32(raw_dev, sample_format, channels, n_frames, mono_dev, ctx->sm_count,
                                            reinterpret_cast<cudaStream_t>(stream), err), err);
+}
+
+int syg_ingest_pcm_channels(syg_ctx* ctx, const void* raw_dev, int32_t sample_format, int32_t channels, int64_t n_frames,
+                            float* out_dev, void* stream) {
+    SYG_TRACE();
+    if (!ctx) return fail(SYG_E_BADARG, "ctx is NULL");
+    if (n_frames < 0 || (n_frames > 0 && (!raw_dev || !out_dev))) return fail(SYG_E_BADARG, "bad PCM buffer");
+    if (!pcm_layout_ok(InFmt{sample_format, channels})) return fail(SYG_E_BADARG, "bad PCM layout (format %d, %d channels)", sample_format, channels);
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    ENTER_DEVICE(ctx);
+    std::string err;
+    ProfScope ps(ctx, reinterpret_cast<cudaStream_t>(stream), PROF_OTHER);
+    return launch_rc(syglaunch::pcm_to_planes(raw_dev, sample_format, channels, n_frames, plane_pitch(n_frames), out_dev, ctx->sm_count,
+                                              reinterpret_cast<cudaStream_t>(stream), err), err);
 }
 
 int syg_pcm16_to_f32(syg_ctx* ctx, const int16_t* in_dev, float* out_dev, int64_t n, void* stream) {
@@ -1527,11 +1578,12 @@ int syg_psd_welch_f32(syg_ctx* ctx, const float* y_dev, const syg_units* units, 
     return launch_welch(pl.nfft, pl.wa, ctx->sm_count, reinterpret_cast<cudaStream_t>(stream));
 }
 
-int syg_psd_welch_host_f32(syg_ctx* ctx, const float* y_host, const syg_units* units, double fs, int32_t window,
+// inf.planes: psd_host [n_units][channels][1 + nfft/2], stats_host [n_units][channels][3]
+static int welch_host_impl(syg_ctx* ctx, const void* y_host, InFmt inf, const syg_units* units, double fs, int32_t window,
                            int32_t nperseg, int32_t noverlap, int32_t nfft, int32_t detrend_constant,
                            int32_t scaling, float* psd_host, float* stats_host) {
-    SYG_TRACE();
     if (!ctx) return fail(SYG_E_BADARG, "ctx is NULL");
+    if (inf.planes && !pcm_layout_ok(inf)) return fail(SYG_E_BADARG, "bad PCM layout (format %d, %d channels)", inf.fmt, inf.channels);
     int rc = check_host_units(units);
     if (rc) return rc;
     std::lock_guard<std::mutex> lk(ctx->mu);
@@ -1543,15 +1595,34 @@ int syg_psd_welch_host_f32(syg_ctx* ctx, const float* y_host, const syg_units* u
     const size_t psd_per_unit = (size_t)(pl.nfft / 2 + 1) * sizeof(float);
     const size_t st_per_unit = stats_host ? 3 * sizeof(float) : 0;
     const int sm = ctx->sm_count;
-    return host_pipeline(ctx, y_host, InFmt{}, units, psd_per_unit, psd_host, st_per_unit, stats_host, 0, 1LL << 40,
+    return host_pipeline(ctx, y_host, inf, units, psd_per_unit, psd_host, st_per_unit, stats_host, 0, 1LL << 40,
                          [&](Lane& L, const float* y_dev, const syg::UnitGeom& g) -> int {
                              syg::WelchArgs c = pl.wa;
                              c.y = y_dev;
                              c.g = g;
                              c.psd = reinterpret_cast<float*>(L.out0.p);
                              c.stats = st_per_unit ? reinterpret_cast<float*>(L.out1.p) : nullptr;
+                             // the channel form times its launch (one per chunk, whatever the channel count); the float32 form's
+                             // launches stay untimed, as they were
+                             ProfScope ps(ctx, L.stream, inf.planes ? PROF_WELCH : -1);
                              return launch_welch(pl.nfft, c, sm, L.stream);
                          });
+}
+
+int syg_psd_welch_host_f32(syg_ctx* ctx, const float* y_host, const syg_units* units, double fs, int32_t window,
+                           int32_t nperseg, int32_t noverlap, int32_t nfft, int32_t detrend_constant,
+                           int32_t scaling, float* psd_host, float* stats_host) {
+    SYG_TRACE();
+    return welch_host_impl(ctx, y_host, InFmt{}, units, fs, window, nperseg, noverlap, nfft, detrend_constant, scaling, psd_host,
+                           stats_host);
+}
+
+int syg_psd_welch_host_pcm_channels(syg_ctx* ctx, const void* raw_host, int32_t sample_format, int32_t channels,
+                                    const syg_units* units, double fs, int32_t window, int32_t nperseg, int32_t noverlap,
+                                    int32_t nfft, int32_t detrend_constant, int32_t scaling, float* psd_host, float* stats_host) {
+    SYG_TRACE();
+    return welch_host_impl(ctx, raw_host, InFmt{sample_format, channels, true}, units, fs, window, nperseg, noverlap, nfft,
+                           detrend_constant, scaling, psd_host, stats_host);
 }
 
 int syg_aggregate_f32(syg_ctx* ctx, const float* feats_dev, int64_t n_seg, int32_t n_rows, int64_t row_stride,

@@ -40,6 +40,9 @@ int aggregate(const float* feats, long long n_seg, int n_rows, long long row_str
 int time_extra(const syg::FrameArgs& a, int frame_length, int entropy_bins, int sm_count, cudaStream_t st, std::string& err);
 int pcm_to_f32(const void* raw, int fmt, int channels, long long n_frames, float* out, int sm_count, cudaStream_t st, std::string& err);
 int pcm16_to_f32(const short* in, float* out, long long n, int sm_count, cudaStream_t st, std::string& err);
+// interleaved PCM -> float32 planes out[c * pitch + i] (i < n_frames), one per channel; channels == 1 takes pcm_to_f32
+int pcm_to_planes(const void* raw, int fmt, int channels, long long n_frames, long long pitch, float* out, int sm_count, cudaStream_t st,
+                  std::string& err);
 int dct_matrix(const double* S, const double* D, long long n_units, int N, long long T, int C, double* out, int sm_count, cudaStream_t st,
                std::string& err);
 int contrast_spectrum(const float* S, int B, long long T, int nb, const int* lo, const int* cnt, const int* nq, float* cws, unsigned* unit_max,
