@@ -39,6 +39,33 @@ def power_close(P, Pref):
     assert not bad.any(), f"{bad.sum()} power bins out of tolerance, worst excess {(np.abs(P - Pref) - tol).max():.3e}"
 
 
+def row_tol(n, r, bin_hz=None, nyq=None):
+    """The absolute bar of the table above for row ``n`` against reference values ``r``: everywhere for the continuous rows, the
+    one-bin limit for rolloff / dominant frequency and the 2e-2 dB limit for contrast.  None for zero_crossing_rate (exact)."""
+    r = np.abs(np.asarray(r, dtype=np.float64))
+    if n.startswith("mfcc_"):
+        return np.full_like(r, 1e-3)
+    if n.startswith("contrast_"):
+        return np.full_like(r, 2e-2)
+    if n == "spectral_centroid":
+        return 1e-5 * r + 1e-6 * (24000.0 if nyq is None else nyq)
+    if n in ("rms_energy", "crest_factor", "peak_amplitude", "mean_amplitude", "std_dev_amplitude"):
+        return 1e-5 * r + 1e-9
+    if n in ("spectral_rolloff", "dominant_frequency"):
+        return np.full_like(r, (1.0 + 1e-6) * bin_hz)
+    if n in ("skewness", "kurtosis"):
+        return 2e-5 * r + 2e-6
+    if n == "signal_entropy":
+        return np.full_like(r, 1e-6)
+    if n == "spectral_bandwidth":
+        return 1e-4 * r + 1e-2
+    if n == "spectral_flatness":
+        return 1e-4 * r + 1e-7
+    if n == "zero_crossing_rate":
+        return None
+    raise AssertionError(f"no tolerance defined for {n}")
+
+
 def check_rows(names, got, ref, bin_hz=None, nyq=None, contrast_ok=None):
     """got/ref: [rows, T] (or [units, rows, T]) in the order of ``names``."""
     if nyq is None and bin_hz is not None:
@@ -53,7 +80,7 @@ def check_rows(names, got, ref, bin_hz=None, nyq=None, contrast_ok=None):
         g, r = got[:, i], ref[:, i]
         d = np.abs(g - r)
         if n.startswith("mfcc_"):
-            assert d.max() <= 1e-3, f"{n}: max abs err {d.max():.3e}"
+            assert (d <= row_tol(n, r)).all(), f"{n}: max abs err {d.max():.3e}"
         elif n.startswith("contrast_"):
             assert np.isfinite(g).all()
             if contrast_ok is not None:
@@ -63,9 +90,9 @@ def check_rows(names, got, ref, bin_hz=None, nyq=None, contrast_ok=None):
             contrast_d.append(d.ravel())
         elif n == "spectral_centroid":
             assert bin_hz is not None
-            assert (d <= 1e-5 * np.abs(r) + 1e-6 * nyq).all(), f"{n}: worst {d.max():.3e}"
+            assert (d <= row_tol(n, r, nyq=nyq)).all(), f"{n}: worst {d.max():.3e}"
         elif n in ("rms_energy", "crest_factor", "peak_amplitude", "mean_amplitude", "std_dev_amplitude"):
-            assert (d <= 1e-5 * np.abs(r) + 1e-9).all(), f"{n}: worst rel {(d / (np.abs(r) + 1e-30)).max():.3e}"
+            assert (d <= row_tol(n, r)).all(), f"{n}: worst rel {(d / (np.abs(r) + 1e-30)).max():.3e}"
         elif n in ("spectral_rolloff", "dominant_frequency"):
             assert bin_hz is not None
             off = d / bin_hz
@@ -73,16 +100,8 @@ def check_rows(names, got, ref, bin_hz=None, nyq=None, contrast_ok=None):
             assert (off > 0.5).mean() <= 1e-3, f"{n}: {(off > 0.5).sum()} of {off.size} frames differ"
         elif n == "zero_crossing_rate":
             assert np.array_equal(g, r.astype(np.float32)), f"{n}: differs on {(g != r.astype(np.float32)).sum()} frames"   # counts / frame_length
-        elif n in ("skewness", "kurtosis"):
-            assert (d <= 2e-5 * np.abs(r) + 2e-6).all(), f"{n}: worst {d.max():.3e}"
-        elif n == "signal_entropy":
-            assert (d <= 1e-6).all(), f"{n}: worst {d.max():.3e}"
-        elif n == "spectral_bandwidth":
-            assert (d <= 1e-4 * np.abs(r) + 1e-2).all(), f"{n}: worst {d.max():.3e}"
-        elif n == "spectral_flatness":
-            assert (d <= 1e-4 * np.abs(r) + 1e-7).all(), f"{n}: worst {d.max():.3e}"
         else:
-            raise AssertionError(f"no tolerance defined for {n}")
+            assert (d <= row_tol(n, r)).all(), f"{n}: worst {d.max():.3e}"
     if contrast_d and sum(c.size for c in contrast_d):
         allc = np.concatenate(contrast_d)
         assert (allc > 1e-3).mean() <= 0.01, f"{(allc > 1e-3).sum()} of {allc.size} contrast entries above 1e-3 dB"
