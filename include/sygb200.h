@@ -187,7 +187,8 @@ int syg_segment_vectors_host_pcm_channels(syg_ctx* ctx, const void* raw_host, in
 /* Segment vectors: extract_features() per unit followed by format_feature_vectors_per_segment() (sygnals/core/ml_utils/
  * formatters.py:51-163, the consumer in `sygnals save dataset`, sygnals/cli/save_cmd.py:140-190) with every unit as one segment:
  * out [n_units][n_rows] float64, agg[r] in SYG_AGG_* per feature row (host array).  The frame features [n_units][n_rows][T] stay
- * in a library-owned block on the device: the result that crosses PCIe (host forms) or NVLink (the final gather) is T times smaller. */
+ * in a library-owned block on the device: the result that crosses PCIe (host forms) or NVLink (the final gather) is T times smaller.
+ * Units without frames (T = 0) give NaN rows (formatters.py:31-36). */
 int syg_segment_vectors_f32(syg_ctx* ctx, const float* y_dev, const syg_units* units, const syg_feature_params* p,
                             const int32_t* agg, double* out_dev, void* stream);
 int syg_segment_vectors_host_f32(syg_ctx* ctx, const float* y_host, const syg_units* units, const syg_feature_params* p,
@@ -204,7 +205,8 @@ int syg_segment_vectors_host_pcm(syg_ctx* ctx, const void* raw_host, int32_t sam
  * Segment vectors: float64 [n_units][n_rows], agg[r] in SYG_AGG_* over the unit's T_u frames (T_u = 0: a NaN row).
  * The tables are HOST memory for the device and the host forms alike; the call stages them before it returns.
  * Errors: SYG_E_BADARG for a negative start or length, a unit outside the sample buffer or NULL tables (n_units > 0);
- * SYG_E_UNSUPPORTED for lengths[u] or T_u above 2^31-1; plan errors as syg_features_*.  n_units = 0 or F = 0: nothing to do. */
+ * SYG_E_UNSUPPORTED for lengths[u] or T_u above 2^31-1; plan errors as syg_features_*.  n_units = 0: nothing to do; F = 0:
+ * features write nothing, segment vectors are all NaN rows. */
 typedef struct {
     int64_t n_units;
     int64_t total_len;          /* samples in y */
@@ -264,7 +266,7 @@ int64_t syg_segment_table(int64_t total_samples, double sr, double segment_lengt
  * M *= 1 + (lifter/2) sin(pi (1..n_mfcc) / lifter)): S [n_units][n_mels][T] float64 -> out [n_units][min(n_mfcc, n_mels)][T] float64.
  * spectral_contrast(S=|X|) (sygnals/core/features/frequency_domain.py:147-212, librosa defaults: quantile 0.02, dB output, each
  * of peak / valley clamped 80 dB below its own maximum): S [n_bins][T] float32 magnitudes of an n_fft = 2 (n_bins - 1) transform
- * -> out [n_bands + 1][T] float32. */
+ * -> out [n_bands + 1][T] float32.  When band 0 [0, fmin] holds bin 0 only, every entry is NaN, as librosa returns it. */
 int syg_mfcc_from_logmel_f64(syg_ctx* ctx, const double* S_dev, int64_t n_units, int32_t n_mels, int64_t T, int32_t n_mfcc,
                              int32_t dct_type, int32_t dct_ortho, double lifter, double* out_dev, void* stream);
 int syg_spectral_contrast_from_mag_f32(syg_ctx* ctx, const float* S_dev, int32_t n_bins, int64_t T, double sr, int32_t n_bands,

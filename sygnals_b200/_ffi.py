@@ -223,9 +223,9 @@ class Library:
         return out
 
     def debug_contrast_bands(self, sr: int, n_fft: int, n_bands: int = 6, fmin: float = 200.0, quantile: float = 0.02):
-        lo = np.zeros(n_bands + 1, dtype=np.int32)
-        cnt = np.zeros(n_bands + 1, dtype=np.int32)
-        nq = np.zeros(n_bands + 1, dtype=np.int32)
+        lo = np.zeros(max(n_bands + 1, 0), dtype=np.int32)
+        cnt = np.zeros(max(n_bands + 1, 0), dtype=np.int32)
+        nq = np.zeros(max(n_bands + 1, 0), dtype=np.int32)
         self.check(self.dll.syg_debug_contrast_bands(sr, n_fft, n_bands, fmin, quantile, lo.ctypes.data, cnt.ctypes.data,
                                                      nq.ctypes.data))
         return lo, cnt, nq
@@ -247,6 +247,39 @@ def library() -> Library:
         if _lib is None:
             _lib = Library()
         return _lib
+
+
+def mfcc_count(feature_params: Optional[dict] = None) -> int:
+    """MFCC rows of a request: librosa slices the DCT of the n_mels log-mel rows (``dct(S)[:n_mfcc]``), so at most n_mels."""
+    m = (feature_params or {}).get("mfcc", {})
+    return min(int(m.get("n_mfcc", 13)), int(m.get("n_mels", 128)))
+
+
+def failing_features(lib: Library, features: Sequence[str], sr: int, frame_length: int, feature_params: Optional[dict] = None) -> dict:
+    """{feature: reason} for the requested features whose computation raises in the reference (which then leaves them out):
+    * ``spectral_contrast`` when its octave bands cannot be planned: a band edge at or above Nyquist, a band without FFT bins,
+      bad ``n_bands`` / ``fmin`` / ``quantile`` (librosa's ParameterError, or the IndexError of an empty band).  The engine's own
+      band planner decides; more than 11 bands are left to the engine, which refuses them.
+    * ``mfcc`` with a negative lifter, or a positive one and ``n_mfcc > n_mels`` (librosa's lifter has n_mfcc entries, the DCT
+      output only n_mels rows, and the product does not broadcast)."""
+    fp = feature_params or {}
+    out = {}
+    if "spectral_contrast" in features:
+        c = fp.get("spectral_contrast", {})
+        n_bands = int(c.get("n_bands", 6))
+        if n_bands <= 11:
+            try:
+                lib.debug_contrast_bands(int(sr), int(frame_length), n_bands, float(c.get("fmin", 200.0)), float(c.get("quantile", 0.02)))
+            except ValueError as e:
+                out["spectral_contrast"] = str(e)
+    if "mfcc" in features:
+        m = fp.get("mfcc", {})
+        lifter = float(m.get("lifter", 0.0))
+        if lifter < 0:
+            out["mfcc"] = f"MFCC lifter={lifter} must be a non-negative number"
+        elif lifter > 0 and int(m.get("n_mfcc", 13)) > int(m.get("n_mels", 128)):
+            out["mfcc"] = "the lifter has n_mfcc entries but the DCT only n_mels rows: operands could not be broadcast together"
+    return out
 
 
 def make_params(lib: Library, sr: int, features: Sequence[str], frame_length: int = 2048, hop_length: int = 512,
@@ -290,6 +323,20 @@ def make_params(lib: Library, sr: int, features: Sequence[str], frame_length: in
     p.roll_percent = float(r.get("roll_percent", 0.85))
     p.entropy_bins = int(fp.get("signal_entropy", {}).get("num_bins", 10))
     return p
+
+
+def reference_params(lib: Library, sr: int, features: Sequence[str], frame_length: int = 2048, hop_length: int = 512,
+                     center: bool = True, window: str = "hann", feature_params: Optional[dict] = None) -> SygFeatureParams:
+    """:func:`make_params` for the entry points that mirror the reference.  A feature the reference would fail on
+    (:func:`failing_features`) raises ValueError (the manager leaves such features out before it gets here), and the parameter block
+    asks for :func:`mfcc_count` coefficients, the rows ``batch.feature_row_names`` names.  ``make_params`` itself passes ``n_mfcc``
+    through, so the C ABI still rejects more coefficients than mel bands."""
+    for name, why in failing_features(lib, features, sr, frame_length, feature_params).items():
+        raise ValueError(f"{name}: {why}")
+    fp = dict(feature_params or {})
+    if "mfcc" in fp:
+        fp["mfcc"] = dict(fp["mfcc"], n_mfcc=mfcc_count(fp))
+    return make_params(lib, sr, features, frame_length, hop_length, center, window, fp)
 
 
 def plane_pitch(n_frames: int) -> int:

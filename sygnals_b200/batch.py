@@ -29,7 +29,7 @@ def feature_row_names(features: Sequence[str], feature_params: Optional[dict] = 
     names: List[str] = []
     for f in features:
         if f == "mfcc":
-            names += [f"mfcc_{i}" for i in range(int(fp.get("mfcc", {}).get("n_mfcc", 13)))]
+            names += [f"mfcc_{i}" for i in range(_ffi.mfcc_count(fp))]
         elif f == "spectral_contrast":
             nb = int(fp.get("spectral_contrast", {}).get("n_bands", 6))
             names += [f"contrast_band_{i}" for i in range(nb)] + ["contrast_delta"]
@@ -72,7 +72,7 @@ def extract_features_batch(clips, sr: int, features: Sequence[str], frame_length
     if clips.ndim != 2:
         raise ValueError("clips must be a 2D array [n_clips, n_samples].")
     eng = _engine_for(clips, device)
-    p = _ffi.make_params(eng.lib, sr, list(features), frame_length, hop_length, center, window, feature_params)
+    p = _ffi.reference_params(eng.lib, sr, list(features), frame_length, hop_length, center, window, feature_params)
     n, L = int(clips.shape[0]), int(clips.shape[1])
     out = _run(clips, eng.units_clips(n, L), n, p, eng)
     return feature_row_names(features, feature_params), out
@@ -90,7 +90,7 @@ def segment_features(y, sr: int, segment_length_sec: float, features: Sequence[s
     eng = _engine_for(y, device)
     total = int(y.shape[0])
     seg_len, seg_hop, starts, valid = eng.lib.segment_table(total, sr, segment_length_sec, overlap_ratio, pad, min_segment_length_sec)
-    p = _ffi.make_params(eng.lib, sr, list(features), frame_length, hop_length, center, window, feature_params)
+    p = _ffi.reference_params(eng.lib, sr, list(features), frame_length, hop_length, center, window, feature_params)
     n = len(starts)
     analytic = n > 0 and min_segment_length_sec is None and bool((starts == np.arange(n, dtype=np.int64) * seg_hop).all())
     if n == 0 or analytic:
@@ -163,7 +163,7 @@ def _ragged_call(clips, sr, features, frame_length, hop_length, center, window, 
     if getattr(y, "ndim", None) != 1:
         raise ValueError("the sample buffer must be 1-D")
     eng = _engine_for(y, device)
-    p = _ffi.make_params(eng.lib, sr, list(features), frame_length, hop_length, center, window, feature_params)
+    p = _ffi.reference_params(eng.lib, sr, list(features), frame_length, hop_length, center, window, feature_params)
     units = eng.ragged_units(starts, lengths, int(y.shape[0]))
     names = feature_row_names(features, feature_params)
     ids = None
@@ -329,7 +329,7 @@ def channel_vectors(source, segment_length_sec: float, features: Sequence[str], 
     raw, fmt, ch, frames, sr = _pcm_source(source)
     eng = _ffi.engine(device)
     seg_len, _, starts, valid = eng.lib.segment_table(frames, sr, segment_length_sec, overlap_ratio, pad)
-    p = _ffi.make_params(eng.lib, sr, list(features), frame_length, hop_length, center, window, feature_params)
+    p = _ffi.reference_params(eng.lib, sr, list(features), frame_length, hop_length, center, window, feature_params)
     names = feature_row_names(features, feature_params)
     from .core.ml_utils.formatters import _agg_ids
     units = eng.units_table(starts.ctypes.data, valid.ctypes.data, len(starts), seg_len, frames)

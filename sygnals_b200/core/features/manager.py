@@ -4,7 +4,9 @@ Same signature, feature-name strings, column order (order of ``features``; ``['a
 (``1 + len(y)//hop`` when centred, manager.py:149-157), time axis (``(i*hop + frame_length//2)/sr``, manager.py:166-169),
 naming (``mfcc_i``, ``contrast_band_i``, ``contrast_delta``, manager.py:337-343,365-369), the injected
 ``spectral_centroid`` column when ``spectral_bandwidth`` is requested first (manager.py:296-301), error types and output
-formats.  The arithmetic is ONE fused kernel family on the GPU (FP32); columns are widened to float64.
+formats.  The arithmetic is ONE fused kernel family on the GPU (FP32); columns are widened to float64.  A feature the reference
+fails on is logged and left out, the others are returned (manager.py:394-397; ``_ffi.failing_features``), and NaN rows of the
+reference (contrast whose band 0 holds bin 0 only) come back as NaN.
 
 Differences, by design: features without a CUDA kernel raise ``NotImplementedError`` instead of running on the CPU, and
 only power-of-two ``frame_length`` in [32, 8192] is supported.
@@ -83,12 +85,17 @@ def extract_features(y, sr: int, features: List[str], frame_length: int = 2048, 
         if f == "spectral_bandwidth" and "spectral_centroid" not in plan:
             plan.append("spectral_centroid")
         plan.append(f)
+    # a feature the reference fails on is logged and left out, the others are returned (manager.py:394-397); the rest still run in
+    # one engine call
+    for f, why in _ffi.failing_features(eng.lib, plan, sr, frame_length, feature_params).items():
+        logger.error(f"Error calculating feature '{f}': {why}")
+        plan.remove(f)
     times = frame_times(num_frames, sr, hop_length, frame_length, center)
     if not plan:
         logger.warning("No features were successfully extracted or passed final checks.")
         return empty() if output_format == "dataframe" else {"time": times}
     try:
-        p = _ffi.make_params(eng.lib, sr, plan, frame_length, hop_length, center, window, feature_params)
+        p = _ffi.reference_params(eng.lib, sr, plan, frame_length, hop_length, center, window, feature_params)
         rows = eng.features_host(y.astype(np.float32, copy=False), eng.units_clips(1, len(y)), p)[0]
     except (ValueError, NotImplementedError):
         raise

@@ -14,6 +14,7 @@
 #include <cstdlib>
 #include <cstdio>
 #include <cstring>
+#include <limits>
 #include <map>
 #include <mutex>
 #include <string>
@@ -409,11 +410,14 @@ int rows_of(const syg_feature_params* p, int32_t* n_rows) {
         if (seen & (1u << f)) return fail(SYG_E_BADARG, "feature id %d requested twice", f);
         seen |= 1u << f;
         if (f == SYG_FEAT_MFCC) {
-            if (p->n_mfcc < 1 || p->n_mfcc > 256) return fail(SYG_E_BADARG, "n_mfcc=%d out of range [1, 256]", p->n_mfcc);
+            // librosa takes any count; the engine's limits (n_mfcc <= n_mels <= 256, kMaxBands) are refusals, not bad arguments
+            if (p->n_mfcc < 1) return fail(SYG_E_BADARG, "n_mfcc=%d must be positive", p->n_mfcc);
+            if (p->n_mfcc > 256) return fail(SYG_E_UNSUPPORTED, "n_mfcc=%d: supported range is [1, 256]", p->n_mfcc);
             rows += p->n_mfcc;
         } else if (f == SYG_FEAT_SPECTRAL_CONTRAST) {
-            if (p->contrast_n_bands < 1 || p->contrast_n_bands > syg::kMaxBands - 1)
-                return fail(SYG_E_BADARG, "n_bands=%d out of range [1, %d]", p->contrast_n_bands, syg::kMaxBands - 1);
+            if (p->contrast_n_bands < 1) return fail(SYG_E_BADARG, "n_bands must be a positive integer");
+            if (p->contrast_n_bands > syg::kMaxBands - 1)
+                return fail(SYG_E_UNSUPPORTED, "n_bands=%d: supported range is [1, %d]", p->contrast_n_bands, syg::kMaxBands - 1);
             rows += p->contrast_n_bands + 1;
         }
         else rows += 1;
@@ -578,6 +582,7 @@ int build_feature_plan(syg_ctx* ctx, const syg_units* u, const syg_feature_param
         // the kernels rely on 1 <= band_n <= band_cnt for non-empty bands (sortedr[:idx] with idx > rows takes every row)
         for (int i = 0; i < b.nb; ++i) { a.band_lo[i] = b.lo[i]; a.band_cnt[i] = b.cnt[i]; a.band_n[i] = std::max(1, std::min(b.nq[i], std::max(b.cnt[i], 1))); }
         pl.fin.nb = b.nb;
+        pl.fin.contrast_nan = b.all_nan ? 1 : 0;          // the frame kernels still select (finite) values; finalize writes NaN
         ws += (size_t)T * 2 * b.nb * sizeof(float);
     }
     pl.n_fft = fl;
@@ -731,6 +736,16 @@ int run_features_chunk(syg_ctx* ctx, const FeaturePlan& pl, const float* y, cons
         f.ragged_stride = out_stride;
     }
     return launch_finalize(ctx, f, nf, st);
+}
+
+// The vectors of an aggregated call in which no unit has a frame: a segment without frames aggregates to NaN (formatters.py:31-36),
+// and the launches that would write the NaN rows do not run.  On the device every byte 0xff: the bits of a (negative, quiet) NaN.
+int nan_vectors(void* out, long long n_vec, int n_rows, bool dev, cudaStream_t st) {
+    if (!out) return fail(SYG_E_BADARG, "out is NULL");
+    const size_t n = (size_t)n_vec * n_rows;
+    if (dev) CK(cudaMemsetAsync(out, 0xff, n * sizeof(double), st));
+    else std::fill_n(static_cast<double*>(out), n, std::numeric_limits<double>::quiet_NaN());
+    return SYG_OK;
 }
 
 int check_agg(const FeaturePlan& pl, const int32_t* agg) {
@@ -1100,10 +1115,11 @@ int ragged_dev_impl(syg_ctx* ctx, const float* y_dev, const syg_ragged_units* un
     syg_units pu{};                                   // the plan's per-unit frame count is not used by ragged launches
     if ((rc = build_feature_plan(ctx, &pu, p, pl))) return rc;
     const long long n_units = units->n_units, F = foff.back();
-    if (n_units == 0 || F == 0 || pl.n_rows == 0) return SYG_OK;
+    if (n_units == 0 || pl.n_rows == 0) return SYG_OK;
+    if (agg && (rc = check_agg(pl, agg))) return rc;
+    if (F == 0) return agg ? nan_vectors(out_dev, n_units, pl.n_rows, true, st) : SYG_OK;
     if (!y_dev && units->total_len > 0) return fail(SYG_E_BADARG, "y_dev is NULL");
     if (!out_dev) return fail(SYG_E_BADARG, "out_dev is NULL");
-    if (agg && (rc = check_agg(pl, agg))) return rc;
     const bool ag = agg != nullptr;
     std::vector<RaggedChunk> chunks;
     ragged_chunks(units, foff, pl, ag, ctx->ws_limit, 0x7fffffffLL, 1LL << 62, chunks);     // starts < 2^31 in the frame table
@@ -1145,10 +1161,11 @@ int ragged_host_impl(syg_ctx* ctx, const float* y_host, const syg_ragged_units* 
     syg_units pu{};
     if ((rc = build_feature_plan(ctx, &pu, p, pl))) return rc;
     const long long n_units = units->n_units, F = foff.back();
-    if (n_units == 0 || F == 0 || pl.n_rows == 0) return SYG_OK;
+    if (n_units == 0 || pl.n_rows == 0) return SYG_OK;
+    if (agg && (rc = check_agg(pl, agg))) return rc;
+    if (F == 0) return agg ? nan_vectors(out_host, n_units, pl.n_rows, false, nullptr) : SYG_OK;
     if (!y_host && units->total_len > 0) return fail(SYG_E_BADARG, "y_host is NULL");
     if (!out_host) return fail(SYG_E_BADARG, "out_host is NULL");
-    if (agg && (rc = check_agg(pl, agg))) return rc;
     const bool ag = agg != nullptr;
     // 128 MiB of samples and 256 MiB of frame features per chunk (host_pipeline's targets); at least two chunks keep both lanes busy
     long long max_frames = std::max<long long>(1, (long long)(((size_t)256 << 20) / ((size_t)pl.n_rows * sizeof(float))));
@@ -1320,10 +1337,11 @@ static int features_dev_impl(syg_ctx* ctx, const float* y_dev, const syg_units* 
     ENTER_DEVICE(ctx);
     FeaturePlan pl;
     if ((rc = build_feature_plan(ctx, units, p, pl))) return rc;
-    if (units->n_units == 0 || pl.T <= 0 || pl.n_rows == 0) return SYG_OK;
+    if (units->n_units == 0 || pl.n_rows == 0) return SYG_OK;
+    if (agg && (rc = check_agg(pl, agg))) return rc;
+    if (pl.T <= 0) return agg ? nan_vectors(out_dev, units->n_units, pl.n_rows, true, st) : SYG_OK;
     if (!y_dev && units->total_len > 0) return fail(SYG_E_BADARG, "y_dev is NULL");
     if (!out_dev) return fail(SYG_E_BADARG, "out_dev is NULL");
-    if (agg && (rc = check_agg(pl, agg))) return rc;
     // aggregated calls keep the frame features of a chunk in the workspace: [chunk][rows][T] never reaches the caller
     const bool ag = agg != nullptr;
     const size_t feat_per_unit = ag ? (size_t)pl.n_rows * pl.T * sizeof(float) : 0;
@@ -1366,10 +1384,11 @@ static int features_host_impl(syg_ctx* ctx, const void* y_host, InFmt inf, const
     ENTER_DEVICE(ctx);
     FeaturePlan pl;
     if ((rc = build_feature_plan(ctx, units, p, pl))) return rc;
-    if (units->n_units == 0 || pl.T <= 0 || pl.n_rows == 0) return SYG_OK;
+    if (units->n_units == 0 || pl.n_rows == 0) return SYG_OK;
+    if (agg && (rc = check_agg(pl, agg))) return rc;
+    if (pl.T <= 0) return agg ? nan_vectors(out_host, units->n_units * (inf.planes ? inf.channels : 1), pl.n_rows, false, nullptr) : SYG_OK;
     if (!y_host && units->total_len > 0) return fail(SYG_E_BADARG, "y_host is NULL");
     if (!out_host) return fail(SYG_E_BADARG, "out_host is NULL");
-    if (agg && (rc = check_agg(pl, agg))) return rc;
     const bool ag = agg != nullptr;
     const size_t feat_per_unit = (size_t)pl.n_rows * pl.T * sizeof(float);
     const size_t out_per_unit = ag ? (size_t)pl.n_rows * sizeof(double) : feat_per_unit;
@@ -1711,6 +1730,7 @@ int syg_spectral_contrast_from_mag_f32(syg_ctx* ctx, const float* S_dev, int32_t
     syg::FinalizeArgs f;
     std::memset(&f, 0, sizeof(f));
     f.n_units = 1; f.T = (int)T; f.n_rows = b.nb; f.row_mfcc = -1; f.nb = b.nb; f.row_contrast = 0; f.amin = 1e-10f; f.top_db = 80.0f;
+    f.contrast_nan = b.all_nan ? 1 : 0;
     f.cws = cws; f.unit_max = um; f.out = out_dev;
     if (T > 0x7fffffffLL) return fail(SYG_E_UNSUPPORTED, "too many frames");
     const long long n_tiles = (T + sygdev::kFinTT - 1) / sygdev::kFinTT;

@@ -150,7 +150,8 @@ __global__ void __launch_bounds__(kThreads) finalize_kernel_t(const syg::Finaliz
                     const float* c = a.cws + (gf0 + tt) * (2 * a.nb);
                     const float pdb = fmaxf(db10(fmaxf(a.amin, c[bd])), s_pfloor[tt]);
                     const float vdb = fmaxf(db10(fmaxf(a.amin, c[a.nb + bd])), s_vfloor[tt]);
-                    a.out[s_out[tt] + (long long)(a.row_contrast + bd) * (RAG ? a.ragged_stride : a.T)] = pdb - vdb;
+                    a.out[s_out[tt] + (long long)(a.row_contrast + bd) * (RAG ? a.ragged_stride : a.T)] =
+                        a.contrast_nan ? __uint_as_float(0x7fc00000u) : pdb - vdb;
                 }
             }
         }

@@ -145,6 +145,7 @@ struct FinalizeArgs {
     const double* dct;                  // [n_mfcc][n_mels] float64 (lifter folded in)
     int dct_fold;                       // 1: DCT-II, row k is (-1)^k symmetric about the centre -> half-length sums
     int nb, row_contrast;               // nb == 0: no contrast
+    int contrast_nan;                   // 1: every contrast entry is NaN (sygplan::Bands::all_nan)
     float amin, top_db;
     const float* melws;
     const float* cws;

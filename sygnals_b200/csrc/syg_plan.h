@@ -330,7 +330,10 @@ inline bool build_dct(int n_out, int N, int type, bool ortho, double lifter, int
     return true;
 }
 
-struct Bands { int nb = 0; int lo[16]; int cnt[16]; int nq[16]; };
+// all_nan: band 0 ([0, fmin]) holds bin 0 only, so its sub-band (the band minus its last row) is empty.  librosa then averages an
+// empty slice for that band's peak and valley (NaN), and power_to_db's top_db clamp against the maximum of the whole array spreads
+// the NaN to every band of every frame: the reference returns NaN for all contrast rows of the call.
+struct Bands { int nb = 0; int lo[16]; int cnt[16]; int nq[16]; bool all_nan = false; };
 
 inline bool build_bands(double sr, int n_fft, int n_bands, double fmin, double quantile, Bands& b, std::string& err) {
     if (n_bands < 1 || n_bands + 1 > 12) { err = "n_bands must be in [1, 11]"; return false; }
@@ -343,6 +346,7 @@ inline bool build_bands(double sr, int n_fft, int n_bands, double fmin, double q
     for (int i = 0; i < n_bands + 1; ++i)
         if (octa[i] >= 0.5 * sr) { err = "Frequency band exceeds Nyquist. Reduce either fmin or n_bands."; return false; }
     b.nb = n_bands + 1;
+    b.all_nan = false;
     for (int k = 0; k <= n_bands; ++k) {
         const double lo = octa[k], hi = octa[k + 1];
         int first = -1, last = -1;
@@ -358,6 +362,7 @@ inline bool build_bands(double sr, int n_fft, int n_bands, double fmin, double q
         double q = std::nearbyint(quantile * (double)total);      // np.rint (half to even)
         int nq = (int)(q < 1.0 ? 1.0 : q);
         b.lo[k] = first; b.cnt[k] = rows; b.nq[k] = nq;
+        if (rows == 0) b.all_nan = true;                          // band 0 only: a later band always takes its predecessor's last bin
     }
     return true;
 }

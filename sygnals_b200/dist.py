@@ -109,7 +109,7 @@ def run_shard(y_local, plan: ShardPlan, sr: int, features: Sequence[str], frame_
     if _is_torch(y_local) and y_local.is_cuda:
         import torch
         eng = engine or _ffi.engine(y_local.device.index or 0)
-        p = _ffi.make_params(eng.lib, sr, list(features), frame_length, hop_length, center, window, feature_params)
+        p = _ffi.reference_params(eng.lib, sr, list(features), frame_length, hop_length, center, window, feature_params)
         rows, T = eng.rows(p), eng.frame_count(plan.seg_len, frame_length, hop_length, center)
         shape = (plan.n_local, rows) if ids is not None else (plan.n_local, rows, T)
         if out is None:
@@ -127,7 +127,7 @@ def run_shard(y_local, plan: ShardPlan, sr: int, features: Sequence[str], frame_
             del keep
         return out
     eng = engine or _ffi.engine()
-    p = _ffi.make_params(eng.lib, sr, list(features), frame_length, hop_length, center, window, feature_params)
+    p = _ffi.reference_params(eng.lib, sr, list(features), frame_length, hop_length, center, window, feature_params)
     y32 = np.ascontiguousarray(y_local, dtype=np.float32)
     units, keep = _shard_units(eng, plan, n_have, None)
     if ids is not None:

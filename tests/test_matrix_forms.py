@@ -67,6 +67,21 @@ def test_spectral_contrast_from_magnitudes(eng, sr, n_fft, T, n_bands, fmin, q):
     assert np.abs(got - ref).max() <= 1e-3, np.abs(got - ref).max()
 
 
+@pytest.mark.parametrize("sr,n_fft,T,n_bands,fmin", [(44100, 128, 9, 6, 200.0), (16000, 64, 40, 6, 200.0), (48000, 512, 3, 4, 50.0)])
+def test_spectral_contrast_from_magnitudes_single_bin_band0(eng, sr, n_fft, T, n_bands, fmin):
+    """Bin spacing above fmin: band 0 [0, fmin] holds bin 0 only, librosa averages an empty slice for it and power_to_db's top_db
+    clamp against the array maximum spreads the NaN: every entry is NaN."""
+    rng = np.random.default_rng(n_fft + T)
+    B = 1 + n_fft // 2
+    S = (rng.random((B, T)) * 10.0 ** rng.uniform(-5, 1, (B, T))).astype(np.float32)
+    ref = shim.feature.spectral_contrast(S=S.astype(np.float64), sr=sr, n_fft=n_fft, n_bands=n_bands, fmin=fmin)
+    assert ref.shape == (n_bands + 1, T) and np.isnan(ref).all()
+    out = np.zeros((n_bands + 1, T), dtype=np.float32)
+    hold, (ps, po) = _dev(eng, S, out)
+    eng.spectral_contrast_from_mag_dev(ps, B, T, sr, n_bands, fmin, 0.02, po)
+    assert np.isnan(_host(hold[1])).all()
+
+
 def test_matrix_forms_argument_errors(eng):
     out = np.zeros(8, dtype=np.float64)
     with pytest.raises(ValueError):
@@ -96,3 +111,7 @@ def test_python_mirrors_on_the_gpu():
         frequency_domain.spectral_contrast(mag[0], 44100)
     with pytest.raises(NotImplementedError):
         frequency_domain.spectral_contrast(mag, 44100, linear=True)
+    small = rng.random((65, 12))                                                 # n_fft 128 at 44.1 kHz: band 0 = bin 0 only
+    assert np.isnan(shim.feature.spectral_contrast(S=small, sr=44100)).all()
+    c = frequency_domain.spectral_contrast(small, 44100)
+    assert c.dtype == np.float64 and c.shape == (7, 12) and np.isnan(c).all()

@@ -332,15 +332,18 @@ TIME_ROWS = {"rms_energy", "crest_factor", "peak_amplitude", "mean_amplitude", "
 
 def _mels(n_fft):
     n_mels = 10 if n_fft <= 64 else 20 if n_fft <= 256 else 40
-    return {"mfcc": {"n_mels": n_mels, "n_mfcc": min(13, n_mels)}}
+    fp = {"mfcc": {"n_mels": n_mels, "n_mfcc": min(13, n_mels)}}
+    if n_fft == 64:       # 22.05 kHz / 64 = 344.5 Hz bins: with fmin 200 band 0 holds bin 0 only and the reference's contrast is NaN
+        fp["spectral_contrast"] = {"fmin": 400.0, "n_bands": 5}
+    return fp
 
 
 # (name, sr, n_fft, hop, features, feature_params, expected syg_debug_last_feature_kernel, resident min groups or None)
 # The plan-specialised n_fft 2048 kernels serve requests without bandwidth / flatness / dominant frequency / mean / std only, and the
 # resident kernel requests without contrast either: there the floor probes are centroid, rolloff, contrast and the MFCCs.
 FEATURE_ARMS = [
-    *[(f"warp{n}", 22050, n, n // 4, [f for f in ALL16 if n > 32 or f != "spectral_contrast"], _mels(n), _ffi.FK_WARP, None)
-      for n in (32, 64, 128, 256, 512, 1024)],
+    *[(f"warp{n}" + ("_fmin400" if n == 64 else ""), 22050, n, n // 4, [f for f in ALL16 if n > 32 or f != "spectral_contrast"],
+       _mels(n), _ffi.FK_WARP, None) for n in (32, 64, 128, 256, 512, 1024)],
     ("warpwide2048", 44100, 2048, 512, ALL16, None, _ffi.FK_WARP_WIDE, None),
     ("spec44kl2048", 44100, 2048, 512, CFG4, None, _ffi.FK_SPEC44KL, None),
     ("spec44k2048", 44100, 2048, 512, CFG4_REORDERED, None, _ffi.FK_SPEC44K, None),
