@@ -236,7 +236,7 @@ int syg_stft_host_f32(syg_ctx* ctx, const float* y_host, const syg_units* units,
 
 /* compute_psd_welch() per unit: psd [n_units][1 + nfft/2]; stats (optional) [n_units][3] = rms, crest, peak of
  * the unit.  noverlap < 0: nperseg/2; nfft <= 0: nperseg (a power of two in 32..8192, or
- * any length >= 8 with prime factors <= 13 up to 28 800: the mixed-radix kernels). */
+ * any length >= 8 with prime factors <= 13 up to 29 040 if even, 14 175 if odd: the mixed-radix kernels). */
 int syg_psd_welch_f32(syg_ctx* ctx, const float* y_dev, const syg_units* units, double fs, int32_t window,
                       int32_t nperseg, int32_t noverlap, int32_t nfft, int32_t detrend_constant, int32_t scaling,
                       float* psd_dev, float* stats_dev, void* stream);
@@ -296,6 +296,8 @@ void syg_debug_last_finalize(int32_t* tile_frames, int64_t* ctas, int64_t* tiles
 /* kernel of the last syg_psd_welch_* call */
 enum { SYG_WELCH_WARP = 1, SYG_WELCH_BLOCK = 2, SYG_WELCH_MIXED = 3 };
 int syg_debug_last_welch_path(void);
+/* threads per CTA (64 / 128 / 256, by transform size) of the last mixed-radix launch: features, STFT or Welch */
+int syg_debug_last_mixed_threads(void);
 /* 1 when the last feature launch kept its (short) units on chip: mel tile + dB + DCT inside the frame kernel, no finalize launch */
 int syg_debug_last_features_resident(void);
 /* frames the feature kernels processed in the last syg_features_* / syg_segment_vectors_* call, all chunks (n_units * T for the

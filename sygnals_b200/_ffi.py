@@ -135,6 +135,7 @@ class Library:
             "syg_debug_last_feature_kernel": (C.c_int, []),
             "syg_debug_last_finalize": (None, [C.POINTER(i32), C.POINTER(i64), C.POINTER(i64)]),
             "syg_debug_last_welch_path": (C.c_int, []),
+            "syg_debug_last_mixed_threads": (C.c_int, []),
             "syg_debug_set_resident_min_groups": (None, [C.c_int]),
             "syg_debug_window": (C.c_int, [i32, i32, i32, vp]),
             "syg_debug_mel_basis": (C.c_int, [i32, i32, i32, f64, f64, vp]),

@@ -1745,6 +1745,7 @@ void syg_debug_last_finalize(int32_t* tile_frames, int64_t* ctas, int64_t* tiles
     if (tiles) *tiles = syglaunch::g_last.fin_tiles;
 }
 int syg_debug_last_welch_path(void) { return syglaunch::g_last.welch_path; }
+int syg_debug_last_mixed_threads(void) { return syglaunch::g_last.mixed_threads; }
 int syg_debug_last_features_resident(void) { return g_last_features_resident; }
 int64_t syg_debug_last_feature_frames(void) { return g_last_feature_frames; }
 int syg_debug_last_mel_form(void) { return g_last_mel_form; }

@@ -12,6 +12,7 @@ struct LastLaunch {
     int feature_kernel = 0;        // SYG_FK_*
     int stft_path = 0;             // syg_debug_last_stft_path
     int welch_path = 0;            // SYG_WELCH_*
+    int mixed_threads = 0;         // threads per CTA of the last mixed-radix launch
     int fin_tt = 0;                // finalize: frames per tile, CTAs, tiles
     long long fin_ctas = 0, fin_tiles = 0;
 };

@@ -17,6 +17,7 @@ static int frame_mixed_t(const syg::FrameArgs& a, const syg::MixedPlan& mp, int 
     if (a.n_frames <= 0) return 0;
     const int grid = (int)std::min<long long>(a.n_frames, (long long)sm_count * blocks_per_sm);
     if constexpr (MODE != sygdev::MODE_STFT) g_last.feature_kernel = SYG_FK_MIXED;
+    g_last.mixed_threads = NT;
     SYG_LAUNCH(kfn, grid, NT, smem, st, a, mp);
     LCK(cudaGetLastError());
     return 0;
@@ -47,6 +48,7 @@ static int welch_mixed_t(const syg::WelchArgs& a, const syg::MixedPlan& mp, int 
     if (a.g.n_units <= 0) return 0;
     const int grid = (int)std::min<long long>(a.g.n_units, (long long)sm_count * blocks_per_sm);
     g_last.welch_path = SYG_WELCH_MIXED;
+    g_last.mixed_threads = NT;
     SYG_LAUNCH(kfn, grid, NT, smem, st, a, mp);
     LCK(cudaGetLastError());
     return 0;

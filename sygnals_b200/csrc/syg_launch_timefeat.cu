@@ -79,13 +79,14 @@ SYG_DEVICE SYG_INLINE void time_extra_body(const syg::FrameArgs& a, const int fl
             m2 += d2; m3 += d2 * d; m4 += d2 * d2;
             if (hist) {
                 // numpy.histogram, uniform bins (lib/_histograms_impl.py): index from the scaled offset, then one step of
-                // correction against the linspace edges
+                // correction against the linspace edges.  linspace rounds idx * step, then adds first: a fused multiply-add
+                // moves an edge by an ulp, and the samples lying on it (the zeros of a padded frame) into the next bin
                 int idx = (int)(((x - first) / (last - first)) * (double)nb);
                 if (idx == nb) idx = nb - 1;
-                const double e_lo = (idx == nb) ? last : first + (double)idx * step;
+                const double e_lo = (idx == nb) ? last : SYG_DADD_RN(first, SYG_DMUL_RN((double)idx, step));
                 if (x < e_lo) idx -= 1;
                 else {
-                    const double e_hi = (idx + 1 == nb) ? last : first + (double)(idx + 1) * step;
+                    const double e_hi = (idx + 1 == nb) ? last : SYG_DADD_RN(first, SYG_DMUL_RN((double)(idx + 1), step));
                     if (x >= e_hi && idx != nb - 1) idx += 1;
                 }
                 const unsigned long long inc = 1ull << (16 * (idx & 3));

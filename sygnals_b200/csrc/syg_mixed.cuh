@@ -5,7 +5,7 @@
 //
 //   frame_mixed_kernel<MODE>   MODE_FEATURES: the feature rows of frame_kernel (syg_kernels.cuh) for any smooth frame_length
 //                              MODE_STFT:     complex / magnitude / power spectrogram (dsp.py:167-229)
-//   welch_mixed_kernel         scipy.signal.welch / periodogram (dsp.py:434-560) for any smooth nfft up to 28 800
+//   welch_mixed_kernel         scipy.signal.welch / periodogram (dsp.py:434-560) for any smooth nfft up to 29 040
 //
 // Even lengths are transformed as L = n/2 packed complex points + real split (the layout of every other kernel of the engine);
 // odd lengths as L = n complex points with zero imaginary parts.  The pass structure follows the autosort formulation: with Ns

@@ -26,7 +26,10 @@ inline size_t fin_smem_bytes(int tt, int n_mels, bool fold) {
     return (size_t)(fold ? 2 : 1) * tt * fin_pitch_d(H) * sizeof(double);
 }
 
-// shared-memory layout (float words) of the mixed-radix kernels for L complex points, B bins and nt threads per CTA
+// shared-memory layout (float words) of the mixed-radix kernels for L complex points, B bins and nt threads per CTA.  Every kernel
+// has the two transform buffers and nt/32 doubles of reduction scratch (dsc); the feature epilogue adds the padded power row, the
+// contrast candidates, the per-unit maxima and nt doubles of inclusive-scan results (dinc, the rolloff scan).  The STFT and Welch
+// kernels never touch those, so they do not pay for them: that keeps even lengths up to 29 040 within 227 KiB.
 struct MixedLayout {
     int off_a, off_b, off_pw, off_cand, off_smax, off_dsc_f, total_f;
     size_t bytes;
@@ -42,7 +45,7 @@ inline MixedLayout mixed_layout(int L, int B, bool features, int nt = kThreads) 
     m.off_cand = m.off_pw + (features ? (B + (B >> 5) + 1) : 0);
     m.off_smax = m.off_cand + (features ? (nt / 32) * 32 : 0);
     m.off_dsc_f = ((m.off_smax + 4 + 1) / 2) * 2;
-    m.total_f = m.off_dsc_f + 2 * (nt / 32 + nt);
+    m.total_f = m.off_dsc_f + 2 * (nt / 32 + (features ? nt : 0));
     m.bytes = (size_t)m.total_f * 4;
     return m;
 }

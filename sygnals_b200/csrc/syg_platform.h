@@ -21,6 +21,9 @@
 #define SYG_INLINE inline
 #define SYG_NOINLINE static inline
 #define SYG_UNROLL
+// separately rounded double multiply / add (never fused into one FMA); x86-64 g++ without -mfma has no FMA to fuse into
+#define SYG_DMUL_RN(a, b) ((a) * (b))
+#define SYG_DADD_RN(a, b) ((a) + (b))
 #else
 #include <cuda_runtime.h>
 #define SYG_LAUNCH(kernel, grid, block, smem, stream, ...) \
@@ -31,4 +34,6 @@
 #define SYG_INLINE __forceinline__
 #define SYG_NOINLINE static __noinline__
 #define SYG_UNROLL _Pragma("unroll")
+#define SYG_DMUL_RN(a, b) __dmul_rn((a), (b))
+#define SYG_DADD_RN(a, b) __dadd_rn((a), (b))
 #endif
