@@ -123,9 +123,9 @@ void syg_ctx_destroy(syg_ctx* ctx);
 int syg_ctx_set_workspace_limit(syg_ctx* ctx, size_t bytes);
 int syg_ctx_sm_count(const syg_ctx* ctx);
 /* optional per-kernel timing for bench.py: CUDA events around every kernel launch on the launching stream.
- * read: ms[4] / launches[4] = {frame kernel (FFT + features or STFT), finalize kernel, welch kernel, other (ingest +
- * aggregation)}, summed since the last reset; synchronises on the recorded events.  Not timed: the STFT and Welch launches of
- * syg_stft_host_f32 and syg_psd_welch_host_f32.  syg_psd_welch_host_pcm_channels times its ingest and Welch launches, one of
+ * read: ms[4] / launches[4] = {frame kernel (FFT + features or STFT), finalize kernel (mel_store kernel of the mel spectrogram
+ * calls), welch kernel, other (ingest + aggregation)}, summed since the last reset; synchronises on the recorded events.  Not
+ * timed: the STFT and Welch launches of syg_stft_host_f32 and syg_psd_welch_host_f32.  syg_psd_welch_host_pcm_channels times its ingest and Welch launches, one of
  * each per chunk. */
 int syg_ctx_profile_enable(syg_ctx* ctx, int on);
 int syg_ctx_profile_read(syg_ctx* ctx, double* ms, int64_t* launches, int reset);
@@ -225,6 +225,24 @@ int syg_segment_vectors_ragged_f32(syg_ctx* ctx, const float* y_dev, const syg_r
                                    const int32_t* agg, double* out_dev, void* stream);
 int syg_segment_vectors_ragged_host_f32(syg_ctx* ctx, const float* y_host, const syg_ragged_units* units,
                                         const syg_feature_params* p, const int32_t* agg, double* out_host);
+
+/* Mel spectrograms: the matrix extract_features() builds for its MFCCs (manager.py:213-223), per unit, without the DCT.
+ *   db = 0: S_mel = melspectrogram(S=|STFT|**power, sr, n_mels, fmin, fmax, n_fft=frame_length)        (manager.py:219-222)
+ *   db = 1: S_db = power_to_db(S_mel, ref=np.max), amin 1e-10, top_db 80, the unit's own maximum as reference (manager.py:223):
+ *           the feature calls' dB arithmetic, with each unit's maximum at exactly 0 dB (their DCT input differs from these rows by
+ *           at most a few 1e-6 dB, where a fused multiply-add rounds the reference subtraction).
+ * p: syg_feature_params with n_features = 0 (any other value is SYG_E_BADARG); the calls read sr, frame_length, hop_length, center,
+ * window, n_mels, fmin, fmax and power.  T = syg_frame_count(unit_len, ...).
+ *   uniform: out float32 [n_units][n_mels][T];  ragged: out float32 [n_mels][F], band m of frame t of unit u at out[m * F + F_u + t].
+ * Refusals (SYG_E_UNSUPPORTED) and argument errors as the feature calls; n_units = 0 or units without frames write nothing. */
+int syg_mel_spectrogram_f32(syg_ctx* ctx, const float* y_dev, const syg_units* units, const syg_feature_params* p, int32_t db,
+                            float* out_dev, void* stream);
+int syg_mel_spectrogram_host_f32(syg_ctx* ctx, const float* y_host, const syg_units* units, const syg_feature_params* p, int32_t db,
+                                 float* out_host);
+int syg_mel_spectrogram_ragged_f32(syg_ctx* ctx, const float* y_dev, const syg_ragged_units* units, const syg_feature_params* p,
+                                   int32_t db, float* out_dev, void* stream);
+int syg_mel_spectrogram_ragged_host_f32(syg_ctx* ctx, const float* y_host, const syg_ragged_units* units, const syg_feature_params* p,
+                                        int32_t db, float* out_host);
 
 /* compute_stft(): out [n_units][1 + n_fft/2][T]; complex64 (interleaved) / float32 magnitude / float32 power */
 int syg_stft_f32(syg_ctx* ctx, const float* y_dev, const syg_units* units, int32_t n_fft, int32_t hop_length,

@@ -119,6 +119,10 @@ class Library:
             "syg_features_ragged_host_f32": (C.c_int, [vp, vp, PR, PP, vp]),
             "syg_segment_vectors_ragged_f32": (C.c_int, [vp, vp, PR, PP, vp, vp, vp]),
             "syg_segment_vectors_ragged_host_f32": (C.c_int, [vp, vp, PR, PP, vp, vp]),
+            "syg_mel_spectrogram_f32": (C.c_int, [vp, vp, PU, PP, i32, vp, vp]),
+            "syg_mel_spectrogram_host_f32": (C.c_int, [vp, vp, PU, PP, i32, vp]),
+            "syg_mel_spectrogram_ragged_f32": (C.c_int, [vp, vp, PR, PP, i32, vp, vp]),
+            "syg_mel_spectrogram_ragged_host_f32": (C.c_int, [vp, vp, PR, PP, i32, vp]),
             "syg_stft_f32": (C.c_int, [vp, vp, PU, i32, i32, i32, i32, i32, i32, i32, vp, vp]),
             "syg_stft_host_f32": (C.c_int, [vp, vp, PU, i32, i32, i32, i32, i32, i32, i32, vp]),
             "syg_psd_welch_f32": (C.c_int, [vp, vp, PU, f64, i32, i32, i32, i32, i32, i32, vp, vp, vp]),
@@ -595,7 +599,42 @@ class Engine:
                                                                         C.addressof(agg), out.ctypes.data))
         return out
 
+    def mel_spectrogram_host(self, y: np.ndarray, units: SygUnits, p: SygFeatureParams, db: bool = True,
+                             out: Optional[np.ndarray] = None) -> np.ndarray:
+        """float32 ``[n_units, n_mels, T]``: S_db (``db``) or S_mel of the units of ``y`` (1-D float32 host buffer); ``p`` without
+        features (``n_features = 0``)."""
+        y = _f32c(y)
+        T = self.frame_count(units.unit_len, p.frame_length, p.hop_length, p.center)
+        if out is None:
+            out = np.empty((int(units.n_units), max(int(p.n_mels), 0), T), dtype=np.float32)
+        self.lib.check(self.lib.dll.syg_mel_spectrogram_host_f32(self._h, y.ctypes.data, C.byref(units), C.byref(p), int(bool(db)),
+                                                                 out.ctypes.data))
+        return out
+
+    def mel_spectrogram_ragged_host(self, y: np.ndarray, units: SygRaggedUnits, p: SygFeatureParams, db: bool = True,
+                                    out: Optional[np.ndarray] = None) -> np.ndarray:
+        """float32 ``[n_mels, F]`` for ragged units of the 1-D float32 host buffer ``y`` (band m of frame t of unit u at column
+        F_u + t)."""
+        y = _f32c(y)
+        F = int(self.lib.ragged_frame_offsets(units, p.frame_length, p.hop_length, p.center)[-1])
+        if out is None:
+            out = np.empty((max(int(p.n_mels), 0), F), dtype=np.float32)
+        self.lib.check(self.lib.dll.syg_mel_spectrogram_ragged_host_f32(self._h, y.ctypes.data, C.byref(units), C.byref(p),
+                                                                        int(bool(db)), out.ctypes.data))
+        return out
+
     # ------------------------------------------------------------------ device-pointer entry points (async)
+    def mel_spectrogram_dev(self, y_ptr: int, units: SygUnits, p: SygFeatureParams, db: bool, out_ptr: int, stream: int = 0) -> None:
+        """Device form of ``mel_spectrogram_host``: float32 ``[n_units, n_mels, T]`` in HBM, asynchronous on ``stream``."""
+        self.lib.check(self.lib.dll.syg_mel_spectrogram_f32(self._h, y_ptr, C.byref(units), C.byref(p), int(bool(db)), out_ptr,
+                                                            stream or None))
+
+    def mel_spectrogram_ragged_dev(self, y_ptr: int, units: SygRaggedUnits, p: SygFeatureParams, db: bool, out_ptr: int,
+                                   stream: int = 0) -> None:
+        """Device form of ``mel_spectrogram_ragged_host``: float32 ``[n_mels, F]`` in HBM, asynchronous on ``stream``."""
+        self.lib.check(self.lib.dll.syg_mel_spectrogram_ragged_f32(self._h, y_ptr, C.byref(units), C.byref(p), int(bool(db)), out_ptr,
+                                                                   stream or None))
+
     def features_dev(self, y_ptr: int, units: SygUnits, p: SygFeatureParams, out_ptr: int, stream: int = 0) -> None:
         self.lib.check(self.lib.dll.syg_features_f32(self._h, y_ptr, C.byref(units), C.byref(p), out_ptr, stream or None))
 

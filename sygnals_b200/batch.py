@@ -6,6 +6,9 @@
 * :func:`extract_features_ragged`, :func:`clip_vectors`
                                   -- clips of different lengths (a folder of files, variable-length segments) in one launch,
                                      each clip framed on its own: no padding to the longest
+* :func:`mel_spectrogram_batch`, :func:`segment_mel_spectrogram`, :func:`mel_spectrogram_ragged`
+                                  -- the (log-)mel spectrogram ``extract_features`` computes for its MFCCs, per clip or segment,
+                                     for the same three input shapes
 * :func:`stft_batch`, :func:`psd_welch_batch`
 * :func:`channel_psd`, :func:`channel_vectors`
                                   -- per-channel Welch PSDs / segment vectors of a multi-channel PCM recording (a WAV file or
@@ -88,9 +91,29 @@ def segment_features(y, sr: int, segment_length_sec: float, features: Sequence[s
     if y.ndim != 1:
         raise ValueError("Input signal y must be 1D.")
     eng = _engine_for(y, device)
+    seg = _segments(eng, y, sr, segment_length_sec, overlap_ratio, pad, min_segment_length_sec)
+    p = _ffi.reference_params(eng.lib, sr, list(features), frame_length, hop_length, center, window, feature_params)
+    out = _run(y, seg.units, len(seg.starts), p, eng)
+    return {"names": feature_row_names(features, feature_params), "features": out, "starts": seg.starts, "valid": seg.valid,
+            "seg_len": seg.seg_len, "seg_hop": seg.seg_hop}
+
+
+class _Segments(NamedTuple):
+    units: object                   # _ffi.SygUnits
+    keep: object                    # the tables `units` points at
+    starts: np.ndarray
+    valid: np.ndarray
+    seg_len: int
+    seg_hop: int
+
+
+def _segments(eng, y, sr, segment_length_sec, overlap_ratio, pad, min_segment_length_sec) -> _Segments:
+    """The units of ``segment_fixed_length`` over the 1-D recording ``y``: analytic starts when they are multiples of the hop, else
+    the segment table (on ``y``'s device for a CUDA tensor).  The tables may be dropped without a host synchronisation once the
+    call is queued: the kernels run on the current torch stream, and the caching allocator reuses a freed block only for work queued
+    later on that stream."""
     total = int(y.shape[0])
     seg_len, seg_hop, starts, valid = eng.lib.segment_table(total, sr, segment_length_sec, overlap_ratio, pad, min_segment_length_sec)
-    p = _ffi.reference_params(eng.lib, sr, list(features), frame_length, hop_length, center, window, feature_params)
     n = len(starts)
     analytic = n > 0 and min_segment_length_sec is None and bool((starts == np.arange(n, dtype=np.int64) * seg_hop).all())
     if n == 0 or analytic:
@@ -105,12 +128,7 @@ def segment_features(y, sr: int, segment_length_sec: float, features: Sequence[s
     else:
         units = eng.units_table(starts.ctypes.data, valid.ctypes.data, n, seg_len, total)
         keep = (starts, valid)
-    out = _run(y, units, n, p, eng)
-    # `keep` (device tables) may be dropped without a host synchronisation: the kernels are queued on the current torch stream and
-    # the caching allocator reuses a freed block only for work queued later on that stream
-    del keep
-    return {"names": feature_row_names(features, feature_params), "features": out, "starts": starts, "valid": valid,
-            "seg_len": seg_len, "seg_hop": seg_hop}
+    return _Segments(units, keep, starts, valid, seg_len, seg_hop)
 
 
 class Windows(NamedTuple):
@@ -210,6 +228,90 @@ def clip_vectors(clips, sr: int, features: Sequence[str], aggregation="mean", fr
     Returns (row names, float64 ``[n_clips, rows]``); a clip without frames gives a NaN row."""
     names, out, _ = _ragged_call(clips, sr, features, frame_length, hop_length, center, window, feature_params, device, agg=aggregation)
     return names, out
+
+
+def _mel_params(lib, sr, frame_length, hop_length, center, window, n_mels, fmin, fmax, power):
+    """The mel stage's arguments (manager.py:213-217) as a parameter block without features.  Invalid values raise ValueError;
+    what the kernels do not serve (n_mels above 256, transform lengths, windows) raises NotImplementedError from the library."""
+    if int(hop_length) < 1:
+        raise ValueError(f"hop_length={hop_length} must be >= 1")
+    if int(n_mels) < 1:
+        raise ValueError(f"n_mels={n_mels} must be positive")
+    if not float(power) > 0:
+        raise ValueError(f"power={power} must be positive")
+    top = sr / 2.0 if fmax is None else float(fmax)
+    if not top > float(fmin):
+        raise ValueError(f"fmax={top} must be above fmin={fmin}")
+    mel = {"n_mels": int(n_mels), "fmin": float(fmin), "fmax": fmax, "power": float(power)}
+    return _ffi.make_params(lib, sr, [], frame_length, hop_length, center, window, {"mfcc": mel})
+
+
+def _run_mel(y, units, p, db, eng):
+    T = eng.frame_count(units.unit_len, p.frame_length, p.hop_length, p.center)
+    if _is_torch(y):
+        import torch
+        if not y.is_cuda:
+            raise ValueError("torch inputs must live on a CUDA device (use numpy arrays for host data)")
+        if y.dtype != torch.float32 or not y.is_contiguous():
+            y = y.contiguous().float()
+        out = torch.empty((int(units.n_units), int(p.n_mels), T), dtype=torch.float32, device=y.device)
+        eng.mel_spectrogram_dev(y.data_ptr(), units, p, db, out.data_ptr(), torch.cuda.current_stream(y.device).cuda_stream)
+        return out
+    return eng.mel_spectrogram_host(np.ascontiguousarray(y, dtype=np.float32).reshape(-1), units, p, db)
+
+
+def mel_spectrogram_batch(clips, sr: int, frame_length: int = 2048, hop_length: int = 512, center: bool = True, window: str = "hann",
+                          n_mels: int = 128, fmin: float = 0.0, fmax: Optional[float] = None, power: float = 2.0, db: bool = True,
+                          device: Optional[int] = None):
+    """``clips``: ``[n_clips, L]`` float32 (numpy: host path; CUDA torch: asynchronous on the current stream).  Returns float32
+    ``[n_clips, n_mels, T]``: per clip the mel spectrogram ``extract_features`` builds for its MFCCs (manager.py:213-223),
+    ``power_to_db(S_mel, ref=np.max)`` (clip's own maximum, top_db 80) with ``db``, ``S_mel`` without."""
+    if clips.ndim != 2:
+        raise ValueError("clips must be a 2D array [n_clips, n_samples].")
+    eng = _engine_for(clips, device)
+    p = _mel_params(eng.lib, sr, frame_length, hop_length, center, window, n_mels, fmin, fmax, power)
+    return _run_mel(clips, eng.units_clips(int(clips.shape[0]), int(clips.shape[1])), p, db, eng)
+
+
+def segment_mel_spectrogram(y, sr: int, segment_length_sec: float, overlap_ratio: float = 0.0, pad: bool = True,
+                            min_segment_length_sec: Optional[float] = None, frame_length: int = 2048, hop_length: int = 512,
+                            center: bool = True, window: str = "hann", n_mels: int = 128, fmin: float = 0.0, fmax: Optional[float] = None,
+                            power: float = 2.0, db: bool = True, device: Optional[int] = None) -> Dict[str, object]:
+    """:func:`mel_spectrogram_batch` of every segment of one recording, segmented as :func:`segment_features` does (one launch over
+    the un-segmented recording).  Returns {'mel' ``[n_seg, n_mels, T]``, 'starts', 'valid', 'seg_len', 'seg_hop'}."""
+    if y.ndim != 1:
+        raise ValueError("Input signal y must be 1D.")
+    eng = _engine_for(y, device)
+    seg = _segments(eng, y, sr, segment_length_sec, overlap_ratio, pad, min_segment_length_sec)
+    p = _mel_params(eng.lib, sr, frame_length, hop_length, center, window, n_mels, fmin, fmax, power)
+    out = _run_mel(y, seg.units, p, db, eng)
+    return {"mel": out, "starts": seg.starts, "valid": seg.valid, "seg_len": seg.seg_len, "seg_hop": seg.seg_hop}
+
+
+def mel_spectrogram_ragged(clips, sr: int, frame_length: int = 2048, hop_length: int = 512, center: bool = True, window: str = "hann",
+                           n_mels: int = 128, fmin: float = 0.0, fmax: Optional[float] = None, power: float = 2.0, db: bool = True,
+                           device: Optional[int] = None) -> Dict[str, object]:
+    """Mel spectrograms of clips of different lengths in one launch; ``clips`` as in :func:`extract_features_ragged`.  Returns
+    {'mel': float32 ``[n_mels, F]``, 'frame_offsets': int64 ``[n_clips + 1]``}: columns ``frame_offsets[c] ..
+    frame_offsets[c + 1] - 1`` are :func:`mel_spectrogram_batch` of clip c alone."""
+    y, starts, lengths = _ragged_input(clips)
+    if getattr(y, "ndim", None) != 1:
+        raise ValueError("the sample buffer must be 1-D")
+    eng = _engine_for(y, device)
+    p = _mel_params(eng.lib, sr, frame_length, hop_length, center, window, n_mels, fmin, fmax, power)
+    units = eng.ragged_units(starts, lengths, int(y.shape[0]))
+    foff = eng.lib.ragged_frame_offsets(units, frame_length, hop_length, center)
+    if _is_torch(y):
+        import torch
+        if not y.is_cuda:
+            raise ValueError("torch inputs must live on a CUDA device (use numpy arrays for host data)")
+        if y.dtype != torch.float32 or not y.is_contiguous():
+            y = y.contiguous().float()
+        out = torch.empty((int(n_mels), int(foff[-1])), dtype=torch.float32, device=y.device)
+        eng.mel_spectrogram_ragged_dev(y.data_ptr(), units, p, db, out.data_ptr(), torch.cuda.current_stream(y.device).cuda_stream)
+    else:
+        out = eng.mel_spectrogram_ragged_host(np.ascontiguousarray(y, dtype=np.float32), units, p, db)
+    return {"mel": out, "frame_offsets": foff}
 
 
 def stft_batch(clips, n_fft: int = 2048, hop_length: Optional[int] = None, win_length: Optional[int] = None, window: str = "hann",

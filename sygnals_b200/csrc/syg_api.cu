@@ -397,6 +397,7 @@ struct FeaturePlan {
     size_t ws_per_unit = 0;        // bytes of melws + cws per unit
     int n_fft = 0;
     int entropy_bins = 10;
+    int mel_db = -1;               // >= 0: a mel spectrogram call, n_mels rows of S_mel (0) or S_db (1) written by mel_store_kernel
 };
 
 int rows_of(const syg_feature_params* p, int32_t* n_rows) {
@@ -426,7 +427,8 @@ int rows_of(const syg_feature_params* p, int32_t* n_rows) {
     return SYG_OK;
 }
 
-int build_feature_plan(syg_ctx* ctx, const syg_units* u, const syg_feature_params* p, FeaturePlan& pl) {
+// mel_db >= 0: the plan of a mel spectrogram call (p->n_features == 0): the MFCC frame stage alone, no DCT table, n_mels rows
+int build_feature_plan(syg_ctx* ctx, const syg_units* u, const syg_feature_params* p, FeaturePlan& pl, int mel_db = -1) {
     if (!p) return fail(SYG_E_BADARG, "params is NULL");
     if (p->sr <= 0) return fail(SYG_E_BADARG, "sr must be positive");
     const int fl = p->frame_length;
@@ -439,6 +441,9 @@ int build_feature_plan(syg_ctx* ctx, const syg_units* u, const syg_feature_param
     int32_t rows = 0;
     int rc = rows_of(p, &rows);
     if (rc) return rc;
+    const bool mel = mel_db >= 0;
+    if (mel) rows = p->n_mels;
+    pl.mel_db = mel_db;
     std::memset(&pl.fa, 0, sizeof(pl.fa));
     std::memset(&pl.fin, 0, sizeof(pl.fin));
     syg::FrameArgs& a = pl.fa;
@@ -468,6 +473,7 @@ int build_feature_plan(syg_ctx* ctx, const syg_units* u, const syg_feature_param
             case SYG_FEAT_SIGNAL_ENTROPY: mask |= syg::FB_ENTROPY; a.row_entropy = row++; break;
         }
     }
+    if (mel) mask = syg::FB_MFCC;
     a.mask = mask;
     a.n_rows = rows;
     pl.n_rows = rows;
@@ -488,7 +494,7 @@ int build_feature_plan(syg_ctx* ctx, const syg_units* u, const syg_feature_param
     size_t ws = 0;
     if (mask & syg::FB_MFCC) {
         if (p->n_mels < 1 || p->n_mels > 256) return fail(SYG_E_UNSUPPORTED, "n_mels=%d: supported range is [1, 256]", p->n_mels);
-        if (p->n_mfcc < 1 || p->n_mfcc > p->n_mels) return fail(SYG_E_BADARG, "n_mfcc must be in [1, n_mels]");
+        if (!mel && (p->n_mfcc < 1 || p->n_mfcc > p->n_mels)) return fail(SYG_E_BADARG, "n_mfcc must be in [1, n_mels]");
         if (!(p->power > 0.0)) return fail(SYG_E_BADARG, "power must be positive");
         const double fmax = p->fmax > 0 ? (double)p->fmax : 0.5 * (double)p->sr;
         std::string key = keyf("mel:%d:%d:%d:%.9g:%.9g", p->sr, fl, p->n_mels, (double)p->fmin, fmax);
@@ -559,6 +565,11 @@ int build_feature_plan(syg_ctx* ctx, const syg_units* u, const syg_feature_param
         a.n_mels = p->n_mels;
         a.mel_power_is_2 = (p->power == 2.0);
         a.mel_half_power = (float)(0.5 * p->power);
+        pl.fin.n_mels = p->n_mels;
+        pl.fin.mel_db = mel_db > 0 ? 1 : 0;
+        ws += (size_t)T * p->n_mels * sizeof(float);
+    }
+    if ((mask & syg::FB_MFCC) && !mel) {
         std::string dk = keyf("dct64:%d:%d:%d:%d:%.9g", p->n_mfcc, p->n_mels, p->dct_type, p->dct_ortho, (double)p->lifter);
         std::vector<double> dct;
         if (!ctx->tables.count(dk)) {
@@ -567,10 +578,8 @@ int build_feature_plan(syg_ctx* ctx, const syg_units* u, const syg_feature_param
                 return fail(SYG_E_BADARG, "%s", err.c_str());
         }
         if ((rc = upload_table(ctx, dk, dct, &pl.fin.dct))) return rc;
-        pl.fin.n_mels = p->n_mels;
         pl.fin.n_mfcc = p->n_mfcc;
         pl.fin.dct_fold = (p->dct_type == 2) ? 1 : 0;
-        ws += (size_t)T * p->n_mels * sizeof(float);
     }
     if (mask & syg::FB_CONTRAST) {
         sygplan::Bands b;
@@ -678,13 +687,13 @@ int run_features_chunk(syg_ctx* ctx, const FeaturePlan& pl, const float* y, cons
     }
     // Short units with an MFCC-only epilogue stay on chip (frame_warp_kernel STAGE 5): no mel workspace, no finalize launch.  Needs
     // enough unit groups to fill the GPU; SYGB200_NO_RES=1 keeps the two-kernel path (A/B measurements).  The epilogue sizes its
-    // tile by units x T: uniform chunks only.
+    // tile by units x T: uniform chunks only.  Mel spectrogram calls never take it: it writes DCT rows and keeps no mel tile in HBM.
     {
         static int no_res = -1;
         if (no_res < 0) { const char* e = std::getenv("SYGB200_NO_RES"); no_res = e ? std::atoi(e) : 0; }
         constexpr unsigned other = syg::FB_CONTRAST | syg::FB_BANDWIDTH | syg::FB_FLATNESS | syg::FB_DOMINANT | syg::FB_MEAN_AMP | syg::FB_STD_AMP;
         a.res_units = 0;
-        if (!rt && !no_res && (a.mask & syg::FB_MFCC) && !(a.mask & other) && native_pow2(n_fft) && n_fft <= 1024) {
+        if (!rt && !no_res && pl.mel_db < 0 && (a.mask & syg::FB_MFCC) && !(a.mask & other) && native_pow2(n_fft) && n_fft <= 1024) {
             const int ku = syglaunch::frame_warp_res_units(n_fft, a);
             const long long min_groups = g_resident_min_groups >= 0 ? g_resident_min_groups : 4LL * ctx->sm_count;
             if (ku > 0 && (g.n_units + ku - 1) / ku >= min_groups) {
@@ -735,6 +744,7 @@ int run_features_chunk(syg_ctx* ctx, const FeaturePlan& pl, const float* y, cons
         f.n_frames = nf;
         f.ragged_stride = out_stride;
     }
+    if (pl.mel_db >= 0) return launch_rc(syglaunch::mel_store(f, ctx->sm_count, st, err), err);
     return launch_finalize(ctx, f, nf, st);
 }
 
@@ -1103,7 +1113,7 @@ void ragged_chunks(const syg_ragged_units* u, const std::vector<long long>& foff
 
 // agg == nullptr: out is float32 [n_rows][F]; else float64 [n_units][n_rows]
 int ragged_dev_impl(syg_ctx* ctx, const float* y_dev, const syg_ragged_units* units, const syg_feature_params* p, const int32_t* agg,
-                    void* out_dev, cudaStream_t st) {
+                    void* out_dev, cudaStream_t st, int mel_db = -1) {
     if (!ctx) return fail(SYG_E_BADARG, "ctx is NULL");
     if (!p) return fail(SYG_E_BADARG, "params is NULL");
     std::vector<long long> foff;
@@ -1113,7 +1123,7 @@ int ragged_dev_impl(syg_ctx* ctx, const float* y_dev, const syg_ragged_units* un
     ENTER_DEVICE(ctx);
     FeaturePlan pl;
     syg_units pu{};                                   // the plan's per-unit frame count is not used by ragged launches
-    if ((rc = build_feature_plan(ctx, &pu, p, pl))) return rc;
+    if ((rc = build_feature_plan(ctx, &pu, p, pl, mel_db))) return rc;
     const long long n_units = units->n_units, F = foff.back();
     if (n_units == 0 || pl.n_rows == 0) return SYG_OK;
     if (agg && (rc = check_agg(pl, agg))) return rc;
@@ -1149,7 +1159,7 @@ int ragged_dev_impl(syg_ctx* ctx, const float* y_dev, const syg_ragged_units* un
 
 // host forms: chunks alternate between the two lanes (H2D of the chunk's samples and tables, kernels, D2H overlapped)
 int ragged_host_impl(syg_ctx* ctx, const float* y_host, const syg_ragged_units* units, const syg_feature_params* p, const int32_t* agg,
-                     void* out_host) {
+                     void* out_host, int mel_db = -1) {
     if (!ctx) return fail(SYG_E_BADARG, "ctx is NULL");
     if (!p) return fail(SYG_E_BADARG, "params is NULL");
     std::vector<long long> foff;
@@ -1159,7 +1169,7 @@ int ragged_host_impl(syg_ctx* ctx, const float* y_host, const syg_ragged_units* 
     ENTER_DEVICE(ctx);
     FeaturePlan pl;
     syg_units pu{};
-    if ((rc = build_feature_plan(ctx, &pu, p, pl))) return rc;
+    if ((rc = build_feature_plan(ctx, &pu, p, pl, mel_db))) return rc;
     const long long n_units = units->n_units, F = foff.back();
     if (n_units == 0 || pl.n_rows == 0) return SYG_OK;
     if (agg && (rc = check_agg(pl, agg))) return rc;
@@ -1329,14 +1339,14 @@ int64_t syg_frame_count(int64_t n_samples, int32_t frame_length, int32_t hop_len
 
 // agg == nullptr: out_dev is float32 [n_units][n_rows][T];  else: float64 [n_units][n_rows] (per-row SYG_AGG_* over the frames)
 static int features_dev_impl(syg_ctx* ctx, const float* y_dev, const syg_units* units, const syg_feature_params* p, const int32_t* agg,
-                             void* out_dev, cudaStream_t st) {
+                             void* out_dev, cudaStream_t st, int mel_db = -1) {
     if (!ctx) return fail(SYG_E_BADARG, "ctx is NULL");
     int rc = check_units(units);
     if (rc) return rc;
     std::lock_guard<std::mutex> lk(ctx->mu);
     ENTER_DEVICE(ctx);
     FeaturePlan pl;
-    if ((rc = build_feature_plan(ctx, units, p, pl))) return rc;
+    if ((rc = build_feature_plan(ctx, units, p, pl, mel_db))) return rc;
     if (units->n_units == 0 || pl.n_rows == 0) return SYG_OK;
     if (agg && (rc = check_agg(pl, agg))) return rc;
     if (pl.T <= 0) return agg ? nan_vectors(out_dev, units->n_units, pl.n_rows, true, st) : SYG_OK;
@@ -1373,8 +1383,8 @@ static bool pcm_layout_ok(InFmt inf) { return inf.fmt >= SYG_PCM_U8 && inf.fmt <
 // agg == nullptr: out_host is float32 [n_units][n_rows][T];  else: float64 [n_units][n_rows] (per-row SYG_AGG_* over the frames).
 // inf.planes: [n_units][channels][...], one result per unit and channel.
 static int features_host_impl(syg_ctx* ctx, const void* y_host, InFmt inf, const syg_units* units, const syg_feature_params* p,
-                              const int32_t* agg, void* out_host) {
-    NvtxRange nvtx_range_(agg ? "syg_segment_vectors_host" : "syg_features_host");
+                              const int32_t* agg, void* out_host, int mel_db = -1) {
+    NvtxRange nvtx_range_(mel_db >= 0 ? "syg_mel_spectrogram_host" : agg ? "syg_segment_vectors_host" : "syg_features_host");
     g_last_feature_frames = 0;
     if (!ctx) return fail(SYG_E_BADARG, "ctx is NULL");
     if ((inf.fmt >= 0 || inf.planes) && !pcm_layout_ok(inf)) return fail(SYG_E_BADARG, "bad PCM layout (format %d, %d channels)", inf.fmt, inf.channels);
@@ -1383,7 +1393,7 @@ static int features_host_impl(syg_ctx* ctx, const void* y_host, InFmt inf, const
     std::lock_guard<std::mutex> lk(ctx->mu);
     ENTER_DEVICE(ctx);
     FeaturePlan pl;
-    if ((rc = build_feature_plan(ctx, units, p, pl))) return rc;
+    if ((rc = build_feature_plan(ctx, units, p, pl, mel_db))) return rc;
     if (units->n_units == 0 || pl.n_rows == 0) return SYG_OK;
     if (agg && (rc = check_agg(pl, agg))) return rc;
     if (pl.T <= 0) return agg ? nan_vectors(out_host, units->n_units * (inf.planes ? inf.channels : 1), pl.n_rows, false, nullptr) : SYG_OK;
@@ -1487,6 +1497,46 @@ int syg_segment_vectors_ragged_host_f32(syg_ctx* ctx, const float* y_host, const
     g_last_feature_frames = 0;
     if (!agg) return fail(SYG_E_BADARG, "agg is NULL");
     return ragged_host_impl(ctx, y_host, units, p, agg, out_host);
+}
+
+// The mel spectrogram calls take the feature parameter block without a feature list: other values of n_features are reserved.
+static int check_mel(syg_ctx* ctx, const syg_feature_params* p, int32_t db) {
+    if (!ctx) return fail(SYG_E_BADARG, "ctx is NULL");
+    if (!p) return fail(SYG_E_BADARG, "params is NULL");
+    if (p->n_features != 0) return fail(SYG_E_BADARG, "n_features=%d: the mel spectrogram calls take no feature list", p->n_features);
+    if (db != 0 && db != 1) return fail(SYG_E_BADARG, "db=%d must be 0 or 1", db);
+    return SYG_OK;
+}
+
+int syg_mel_spectrogram_f32(syg_ctx* ctx, const float* y_dev, const syg_units* units, const syg_feature_params* p, int32_t db,
+                            float* out_dev, void* stream) {
+    SYG_TRACE();
+    g_last_feature_frames = 0;
+    if (int rc = check_mel(ctx, p, db)) return rc;
+    return features_dev_impl(ctx, y_dev, units, p, nullptr, out_dev, reinterpret_cast<cudaStream_t>(stream), db);
+}
+
+int syg_mel_spectrogram_host_f32(syg_ctx* ctx, const float* y_host, const syg_units* units, const syg_feature_params* p, int32_t db,
+                                 float* out_host) {
+    g_last_feature_frames = 0;
+    if (int rc = check_mel(ctx, p, db)) return rc;
+    return features_host_impl(ctx, y_host, InFmt{}, units, p, nullptr, out_host, db);
+}
+
+int syg_mel_spectrogram_ragged_f32(syg_ctx* ctx, const float* y_dev, const syg_ragged_units* units, const syg_feature_params* p,
+                                   int32_t db, float* out_dev, void* stream) {
+    SYG_TRACE();
+    g_last_feature_frames = 0;
+    if (int rc = check_mel(ctx, p, db)) return rc;
+    return ragged_dev_impl(ctx, y_dev, units, p, nullptr, out_dev, reinterpret_cast<cudaStream_t>(stream), db);
+}
+
+int syg_mel_spectrogram_ragged_host_f32(syg_ctx* ctx, const float* y_host, const syg_ragged_units* units, const syg_feature_params* p,
+                                        int32_t db, float* out_host) {
+    SYG_TRACE();
+    g_last_feature_frames = 0;
+    if (int rc = check_mel(ctx, p, db)) return rc;
+    return ragged_host_impl(ctx, y_host, units, p, nullptr, out_host, db);
 }
 
 int syg_ingest_pcm(syg_ctx* ctx, const void* raw_dev, int32_t sample_format, int32_t channels, int64_t n_frames, float* mono_dev,

@@ -1,4 +1,4 @@
-// sygnals_b200/csrc/syg_finalize.cuh -- per-unit epilogue (included by exactly one translation unit)
+// sygnals_b200/csrc/syg_finalize.cuh -- per-unit epilogues, finalize and mel_store (included by exactly one translation unit)
 #pragma once
 
 #include "syg_device.cuh"
@@ -14,6 +14,26 @@ namespace sygdev {
 //   contrast: power_to_db(peak) - power_to_db(valley), each clamped to its own unit-wide max - top_db
 //         (librosa.feature.spectral_contrast, frequency_domain.py:200-207).
 // --------------------------------------------------------------------------------------------------------
+
+// One slot of a tile (finalize and mel_store): frame gf's place in `out` -- (unit, row 0, frame t) of a uniform launch, gf of a ragged
+// one -- its unit's maxima, and the unit's reference level and floor of power_to_db(ref=np.max): the maximum of S_db over the unit is
+// attained at the maximum energy -> 0 dB.
+struct FinSlot {
+    long long out;
+    const unsigned* um;
+    float ref_db, floor_db;
+};
+template <bool RAG>
+SYG_DEVICE SYG_INLINE FinSlot fin_slot(const syg::FinalizeArgs& a, long long gf) {
+    const long long u = RAG ? (long long)__ldg(a.ragged_ut + gf).x : gf / a.T;
+    const int t = RAG ? 0 : (int)(gf - u * a.T);
+    FinSlot s;
+    s.um = a.unit_max + u * 4;
+    s.out = RAG ? gf : u * (long long)a.n_rows * a.T + t;
+    s.ref_db = db10(fmaxf(a.amin, __uint_as_float(s.um[0])));
+    s.floor_db = -a.top_db;
+    return s;
+}
 
 // Persistent: the chunk's frames are one flat sequence cut into tiles of kFinTT consecutive frames (a tile may straddle units:
 // every slot carries its own unit, reference level and clamps), CTAs stride over the tiles.  Short units (T = 101 in the
@@ -47,17 +67,12 @@ __global__ void __launch_bounds__(kThreads) finalize_kernel_t(const syg::Finaliz
         const long long gf0 = tile * kFinTT;
         const int nt = (int)min((long long)kFinTT, total - gf0);
         if (tid < nt) {
-            const long long gf = gf0 + tid;
-            const long long u = RAG ? (long long)__ldg(a.ragged_ut + gf).x : gf / a.T;
-            const int t = RAG ? 0 : (int)(gf - u * a.T);
-            const unsigned* um = a.unit_max + u * 4;
-            s_out[tid] = RAG ? gf : u * (long long)a.n_rows * a.T + t;
-            // power_to_db(ref=np.max): the maximum of S_db over the unit is attained at the maximum energy -> 0 dB
-            const float ref_db = db10(fmaxf(a.amin, __uint_as_float(um[0])));
-            s_ref[tid] = ref_db;
-            s_floor[tid] = -a.top_db;
-            s_pfloor[tid] = db10(fmaxf(a.amin, __uint_as_float(um[1]))) - a.top_db;
-            s_vfloor[tid] = db10(fmaxf(a.amin, __uint_as_float(um[2]))) - a.top_db;
+            const FinSlot sl = fin_slot<RAG>(a, gf0 + tid);
+            s_out[tid] = sl.out;
+            s_ref[tid] = sl.ref_db;
+            s_floor[tid] = sl.floor_db;
+            s_pfloor[tid] = db10(fmaxf(a.amin, __uint_as_float(sl.um[1]))) - a.top_db;
+            s_vfloor[tid] = db10(fmaxf(a.amin, __uint_as_float(sl.um[2]))) - a.top_db;
         }
         __syncthreads();
         if (a.row_mfcc >= 0) {
@@ -154,6 +169,101 @@ __global__ void __launch_bounds__(kThreads) finalize_kernel_t(const syg::Finaliz
                         a.contrast_nan ? __uint_as_float(0x7fc00000u) : pdb - vdb;
                 }
             }
+        }
+        __syncthreads();                                                // the tile buffers are reused
+    }
+}
+
+// --------------------------------------------------------------------------------------------------------
+// mel_store: the epilogue of the mel spectrogram calls, in place of finalize.  The frame kernels left the chunk's mel energies
+// frame-major in melws ([frame][n_mels]) and each unit's maximum in unit_max[0]; this kernel writes them frequency-major, as
+// S_mel (a.mel_db == 0) or as S_db with finalize's reference level and floor (a.mel_db == 1, store_db): uniform launches
+// out[u][m][t] (= s_out + m * T), ragged ones out[m * ragged_stride + gf].  Tiles and slots are finalize's (fin_slot).
+//
+// A tile's block of nt * N floats is contiguous: it is read in order (16-byte loads when N % 4 == 0) and transposed through
+// shared memory tile[m][tt] with a pitch of TT + 1 words (1 mod 32).  A warp's store reads 32 consecutive frames of one band, 32
+// distinct banks, and writes one contiguous run of `out`.  On the load side lane L holds bands 4L' .. 4L' + 3 of a frame; writing
+// component j in every lane at once would touch 8 banks, so lane L writes its components in the order (j + L / 8) % 4 and each
+// write step covers 32 banks wherever a warp's 128 floats lie in one frame (every warp when N is a multiple of 128).
+// --------------------------------------------------------------------------------------------------------
+// S_db of one mel energy: finalize's power_to_db (db10, amin, the unit's reference level, the -top_db floor) with the subtraction of
+// the reference level rounded on its own.  In finalize the compiler fuses it with db10's product into one FMA, which leaves each
+// unit's maximum a few 1e-8 dB off 0; here the maximum is exactly 0 dB, as power_to_db(ref=np.max) returns it.  The two differ by
+// at most half an ulp of the product (a few 1e-6 dB).
+SYG_DEVICE SYG_INLINE float store_db(float x, float amin, float ref_db, float floor_db) {
+    return fmaxf(__fadd_rn(db10(fmaxf(amin, x)), -ref_db), floor_db);
+}
+
+template <int KT>
+__global__ void __launch_bounds__(kThreads) mel_store_kernel(const syg::FinalizeArgs a) {
+    constexpr int TT = KT & (kFinRagged - 1);
+    constexpr bool RAG = (KT & kFinRagged) != 0;
+    constexpr int P = TT + 1;
+    SYG_DYN_SMEM(smem_raw);
+    float* const tile = reinterpret_cast<float*>(smem_raw);            // [n_mels][P]
+    __shared__ long long s_out[TT];
+    __shared__ float s_ref[TT];
+    const int tid = threadIdx.x;
+    const long long total = RAG ? a.n_frames : a.n_units * (long long)a.T;
+    const long long n_tiles = (total + TT - 1) / TT;
+    const int N = a.n_mels;
+    const long long row_stride = RAG ? a.ragged_stride : a.T;
+    const float floor_db = -a.top_db;
+    const bool db = a.mel_db != 0;
+
+    for (long long ti = blockIdx.x; ti < n_tiles; ti += gridDim.x) {
+        const long long gf0 = ti * TT;
+        const int nt = (int)min((long long)TT, total - gf0);
+        if (tid < nt) {
+            const FinSlot sl = fin_slot<RAG>(a, gf0 + tid);
+            s_out[tid] = sl.out;
+            s_ref[tid] = sl.ref_db;
+        }
+        __syncthreads();
+        const float* const blk = a.melws + gf0 * N;
+        if ((N & 3) == 0) {
+            // 16-byte aligned: melws is, and every tile starts a multiple of 4 floats into it.  Four loads in flight per thread.
+            const int q = N >> 2;                                       // float4 per frame
+            const int n4 = nt * q;
+            const int rot = (tid >> 3) & 3;                             // = lane / 8
+            const float4* const b4 = reinterpret_cast<const float4*>(blk);
+            for (int c0 = tid; c0 < n4; c0 += 4 * kThreads) {
+                float4 v[4];
+#pragma unroll
+                for (int r = 0; r < 4; ++r)
+                    if (c0 + r * kThreads < n4) v[r] = __ldg(b4 + c0 + r * kThreads);
+#pragma unroll
+                for (int r = 0; r < 4; ++r) {
+                    const int c = c0 + r * kThreads;
+                    if (c >= n4) break;
+                    const int tt = c / q, m = (c - tt * q) << 2;
+                    if (db) {
+                        const float ref_db = s_ref[tt];
+                        v[r].x = store_db(v[r].x, a.amin, ref_db, floor_db);
+                        v[r].y = store_db(v[r].y, a.amin, ref_db, floor_db);
+                        v[r].z = store_db(v[r].z, a.amin, ref_db, floor_db);
+                        v[r].w = store_db(v[r].w, a.amin, ref_db, floor_db);
+                    }
+                    float* const col = tile + m * P + tt;
+#pragma unroll
+                    for (int j = 0; j < 4; ++j) {
+                        const int k = (j + rot) & 3;
+                        col[k * P] = k == 0 ? v[r].x : k == 1 ? v[r].y : k == 2 ? v[r].z : v[r].w;
+                    }
+                }
+            }
+        } else {
+            const int n_el = nt * N;
+            for (int i = tid; i < n_el; i += kThreads) {
+                const int tt = i / N, m = i - tt * N;
+                const float x = __ldg(blk + i);
+                tile[m * P + tt] = db ? store_db(x, a.amin, s_ref[tt], floor_db) : x;
+            }
+        }
+        __syncthreads();
+        for (int i = tid; i < N * TT; i += kThreads) {
+            const int m = i / TT, tt = i - m * TT;
+            if (tt < nt) a.out[s_out[tt] + (long long)m * row_stride] = tile[m * P + tt];
         }
         __syncthreads();                                                // the tile buffers are reused
     }

@@ -36,6 +36,8 @@ int ragged_frame_table(const long long* frame_off, const long long* starts, cons
 int frame_warp_ragged(int n_fft, bool extra, const syg::FrameArgs& a, int sm_count, cudaStream_t st, std::string& err);
 int frame_warp_stft(int n_fft, const syg::FrameArgs& a, int sm_count, cudaStream_t st, std::string& err);
 int finalize(const syg::FinalizeArgs& a, int tt, unsigned grid_x, unsigned grid_y, size_t smem, cudaStream_t st, std::string& err);
+// mel spectrogram epilogue (mel_store_kernel): a chunk's mel energies to [unit][n_mels][T] / [n_mels][ragged_stride], S_mel or S_db
+int mel_store(const syg::FinalizeArgs& a, int sm_count, cudaStream_t st, std::string& err);
 int aggregate(const float* feats, long long n_seg, int n_rows, long long row_stride, const long long* seg_off, const int* seg_len,
               int fixed_len, const int* agg_host, double* out, int sm_count, cudaStream_t st, std::string& err);
 int time_extra(const syg::FrameArgs& a, int frame_length, int entropy_bins, int sm_count, cudaStream_t st, std::string& err);

@@ -95,4 +95,27 @@ int finalize(const syg::FinalizeArgs& a, int tt, unsigned grid_x, unsigned grid_
     return tt == 64 ? finalize_t<64, false>(a, grid_x, grid_y, smem, st, err) : finalize_t<32, false>(a, grid_x, grid_y, smem, st, err);
 }
 
+template <int TT, bool RAG>
+static int mel_store_t(const syg::FinalizeArgs& a, int sm_count, cudaStream_t st, std::string& err) {
+    auto kfn = sygdev::mel_store_kernel<RAG ? (TT | sygdev::kFinRagged) : TT>;
+    const size_t smem = (size_t)a.n_mels * (TT + 1) * sizeof(float);
+    static KernelCache kc;
+    int blocks_per_sm = 0;
+    if (int rc = prepare_kernel(kfn, sygdev::kThreads, smem, kc, &blocks_per_sm, err)) return rc;
+    const long long total = RAG ? a.n_frames : a.n_units * (long long)a.T;
+    const long long n_tiles = (total + TT - 1) / TT;
+    if (n_tiles <= 0) return 0;
+    const int grid = (int)std::min<long long>(n_tiles, (long long)sm_count * blocks_per_sm);
+    SYG_LAUNCH(kfn, grid, sygdev::kThreads, smem, st, a);
+    LCK(cudaGetLastError());
+    return 0;
+}
+
+// tiles of 64 frames for bands of 64 mels or fewer (as finalize: twice the bytes per tile in flight), else 32
+int mel_store(const syg::FinalizeArgs& a, int sm_count, cudaStream_t st, std::string& err) {
+    const bool wide = a.n_mels <= 64;
+    if (a.ragged_ut) return wide ? mel_store_t<64, true>(a, sm_count, st, err) : mel_store_t<32, true>(a, sm_count, st, err);
+    return wide ? mel_store_t<64, false>(a, sm_count, st, err) : mel_store_t<32, false>(a, sm_count, st, err);
+}
+
 }  // namespace syglaunch

@@ -157,6 +157,7 @@ struct FinalizeArgs {
     const int4* ragged_ut;              // ragged launches: [n_frames] {unit, frame in unit, ...} (T unused)
     long long n_frames;                 // ragged launches: frames of the chunk
     long long ragged_stride;            // ragged launches: row r of frame gf at out[r * ragged_stride + gf]
+    int mel_db;                         // mel_store_kernel: 1 writes S_db (power_to_db, ref = the unit's maximum), 0 S_mel
 };
 
 struct WelchArgs {
